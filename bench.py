@@ -13,6 +13,7 @@ again: every timed step streams its state from HBM ("inputs larger than L2").
 
   python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
   python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU algorithm (oracle) on host cores
+  python bench.py --steps K --warmup W --dump-outputs DIR  # also write the last timed step's outputs as DIR/*.npy
 """
 import argparse
 import json
@@ -211,6 +212,41 @@ def port_rate(sample_envs=8192, sample_steps=24, threads=None):
     return {"value": sample_envs * sample_steps / dt, "unit": "env-steps/s", "cores": threads, "kind": "port",
             "sample": f"{sample_envs} envs x {sample_steps} steps of the same workload (Philox noise, auto-reset with "
                       f"64-tick history fill, agent reward + DSR), oracle/mdg_oracle.c with OpenMP over envs, {dt:.2f} s"}
+
+
+DUMP_LIMIT = 64 << 20  # bytes written by --dump-outputs
+
+
+def write_outputs(out_dir, arrays, env_offset=0, limit=DUMP_LIMIT):
+    """Write `arrays` (name -> numpy array with the env axis first) as <out_dir>/<name>.npy, floating arrays in their
+    own precision and integer / bool ones as float64 / float32, plus env_index (the global index of each row's env).
+    When they exceed `limit` bytes together, the rows of a fixed seeded sample of envs are written instead."""
+    import numpy as np
+    out = {k: (a if a.dtype.kind == "f" else a.astype(np.float64 if a.dtype.itemsize == 8 else np.float32))
+           for k, a in arrays.items()}
+    n = next(iter(out.values())).shape[0]
+    per_env = sum(a.nbytes for a in out.values()) // n + 8
+    keep = min(n, limit // per_env)
+    idx = np.arange(n) if keep == n else np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+    out = {k: a[idx] for k, a in out.items()}
+    out["env_index"] = (idx + env_offset).astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in out.items():
+        np.save(os.path.join(out_dir, k + ".npy"), np.ascontiguousarray(a))
+
+
+def dump_outputs(out_dir, env, extra=None):
+    """--dump-outputs: what the env's last Env.step call returned (State, reward, done and the BrokerResponse of
+    EnvInfo, all views of live buffers that the next call overwrites), the agent and shaped rewards the same step
+    computed, and `extra` tensors of the timed path; one row per env."""
+    st, br, t = env._state(), env._info.brokerResponse, env.t
+    arrays = {"state_price": st.price, "state_portfolio": st.portfolio, "state_timestamp": st.timestamp,
+              "reward": t["reward"], "done": t["done"], "transaction_price": br.transactionPrice,
+              "transaction_units": br.transactionUnits, "transaction_cost": br.transactionCost,
+              "risk_info": br.riskInfo, "margin_call": br.marginCall, "agent_reward": env.agent_reward,
+              "shaped_reward": t["shaped_reward"].permute(2, 0, 1)}
+    arrays.update(extra or {})
+    write_outputs(out_dir, {k: v.cpu().numpy() for k, v in arrays.items()}, env.env_offset)
 
 
 def kernel_source_hash():
@@ -419,6 +455,8 @@ def run_ours(args):
     clocks = sampler.summary(t_region0, t_region1)
     step_no = counters["step_no"]
     t_issue = counters["t_issue"]
+    if args.dump_outputs and rank == 0:  # the slab of the last timed step, before the regions below step it again
+        dump_outputs(args.dump_outputs, envs[(step_no - 1) % slabs])
 
     # ---- the dominant kernel alone (roofline): the step kernels of the `slabs` slabs back to back on ONE stream
     # between one pair of CUDA events (so that a launch's set-up overlaps its predecessor's execution, as it does in
@@ -682,6 +720,8 @@ def run_workload(args):
     launches = (env.launches - l0) // max(1, args.repeats)
     sampler.stop()
     clocks = sampler.summary(t0, t1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, env, {"window": wout} if norm else None)
     ms_total = sorted(ms_all)[len(ms_all) // 2]
     # the dominant kernel alone: events around the step launch, the reset outside the pair
     KK = min(K, 100)
@@ -787,7 +827,8 @@ def run_reference(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=4000)
+    ap.add_argument("--steps", type=int, default=None,
+                    help="timed steps per repeat (default 4000 for c5 and the reference arm, 200 for the other --config)")
     ap.add_argument("--warmup", type=int, default=100)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--slabs", type=int, default=8)
@@ -800,12 +841,17 @@ def main():
     ap.add_argument("--repeats", type=int, default=5, help="the K timed steps are issued this many times; the median is reported")
     ap.add_argument("--graph", default="auto", choices=["auto", "on", "off"],
                     help="timed region as one CUDA graph launch (auto: when --steps <= 512)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (rank 0's envs; "
+                         "a fixed seeded sample of them above 64 MB)")
     args = ap.parse_args()
+    if args.steps is None:
+        args.steps = 200 if args.impl == "ours" and args.config != "c5" else 4000
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the CUDA path's outputs; the reference arm has none")
     if args.impl == "reference":
         run_reference(args)
     elif args.config != "c5":
-        if args.steps == 4000:  # (the default of the c5 run)
-            args.steps = 200
         run_workload(args)
     else:
         run_ours(args)

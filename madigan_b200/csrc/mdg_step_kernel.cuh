@@ -611,6 +611,11 @@ __device__ __forceinline__ void step_body(const StepArgs& a) {
           : "memory");
   };
   auto bulk_issue = [&](int pp, int stage) {  // one thread
+    // The copies below write the stage through the async proxy; it was last accessed through the generic proxy (read
+    // by this block's threads, ordered by the barrier before the issue).  PTX orders the two proxies only through a
+    // proxy fence.  Without it, runs with slabs on concurrent streams (tests/test_bench_dump.py) differed from run
+    // to run in thousands of envs.
+    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
     if (tma) { tma_issue(pp, stage); return; }
     const uint32_t mb = smem_u32(&full[stage]);
     asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(mb),

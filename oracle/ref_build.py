@@ -5,7 +5,8 @@ The reference's C++ env needs Eigen, HighFive/HDF5 and CMake with hard-coded con
 (environments/cpp/CMakeLists.txt:5-15); none of that exists here and there is no network.  Its env path,
 however, compiles from a handful of its source files with g++ directly once `Eigen/Core` and the HighFive
 headers resolve -- oracle/ref_shim provides a small eager Eigen subset (left-to-right folds) and throwing
-HighFive stubs.  The reference sources are compiled WHERE THEY LIE under /root/reference (never copied).
+HighFive stubs.  The reference sources are compiled WHERE THEY LIE, in the madigan checkout that MADIGAN_REFERENCE
+names (never copied); without it there is nothing to build.
 pybind11 + Python headers are real (the reference headers include them).  Strict IEEE flags instead of the
 reference's -ffast-math -mfma, so that the result is reproducible and comparable bit for bit.
 """
@@ -15,14 +16,15 @@ import sys
 import sysconfig
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF = "/root/reference/madigan/environments/cpp"
+REF = os.path.join(os.environ["MADIGAN_REFERENCE"], "madigan", "environments", "cpp") \
+    if os.environ.get("MADIGAN_REFERENCE") else None
 OUT = os.path.join(HERE, "_ref")
 LIB = os.path.join(OUT, "libmadigan_ref.so")
 SOURCES = ["Portfolio.cpp", "Account.cpp", "Broker.cpp", "DataSource.cpp", "Config.cpp"]
 
 
 def build(verbose=False):
-    if not os.path.isdir(REF):
+    if not REF or not os.path.isdir(REF):
         return None
     import pybind11
     os.makedirs(OUT, exist_ok=True)

@@ -2,7 +2,7 @@
 
 * `prep_state_tensors` (reference: modelling/algorithm/dqn.py:188-199, with `abs_port_norm`,
   modelling/algorithm/utils.py:31-41) is restated below in the reference's words.  CPU test (runs where
-  /root/reference exists, i.e. in the build container): the restatement equals the reference's own functions, cut
+  MADIGAN_REFERENCE names a madigan checkout): the restatement equals the reference's own functions, cut
   out of the reference files with `ast` (the modules themselves import the compiled C++ env), on random States.
 * GPU tests: the restated function consumes the States produced by `madigan_b200.Env` + `StackerDiscrete` --
   batch=False for a single-env view, batch=True for N envs -- and the reference's agent-loop body
@@ -15,7 +15,8 @@ import os
 import numpy as np
 import pytest
 
-REF = "/root/reference/madigan/modelling/algorithm"
+REF = os.path.join(os.environ["MADIGAN_REFERENCE"], "madigan", "modelling", "algorithm") \
+    if os.environ.get("MADIGAN_REFERENCE") else None
 
 
 def abs_port_norm(port):
@@ -50,7 +51,7 @@ def _reference_functions():
     return ns["prep_state_tensors"], ns["abs_port_norm"]
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="the reference tree is not on this machine")
+@pytest.mark.skipif(not REF or not os.path.isdir(REF), reason="needs MADIGAN_REFERENCE (a madigan checkout)")
 def test_restated_prep_state_tensors_equals_the_reference_function():
     import types
     import torch

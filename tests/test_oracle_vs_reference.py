@@ -9,7 +9,8 @@ marginCall -- and the accounting properties must then agree BIT FOR BIT (same co
 This pins what the reference's own tests leave unpinned: OU / OUPair / noisy Synth generators, Env::step's
 reward clamp and done logic, slippage and transaction-cost arithmetic, the risk gates under leverage.
 
-Skipped when the reference build is absent (it can only be produced where /root/reference exists)."""
+Skipped when the reference build is absent: oracle/ref_build.py produces it from the madigan checkout that
+MADIGAN_REFERENCE names."""
 import zlib
 
 import numpy as np
@@ -20,7 +21,7 @@ from madigan_b200.environments.data_source import make_params
 from oracle import ref
 from oracle.oracle import OracleEnv
 
-pytestmark = pytest.mark.skipif(not ref.available(), reason="oracle/_ref not built (needs /root/reference)")
+pytestmark = pytest.mark.skipif(not ref.available(), reason="oracle/_ref not built (needs MADIGAN_REFERENCE)")
 
 
 def bits(a):
