@@ -237,6 +237,9 @@ typedef struct MdgLaunch {
 /* validation: every risk gate of mdg_step takes the exact left-to-right fold path (the cold path that otherwise
  * only decides knife-edge cases); ledgers must be identical with and without it */
 #define MDG_FLAG_FORCE_EXACT_GATE 1
+/* validation: refills (mdg_reset_ws, mdg_step_autoreset) take the generic kernel, also for parameter sets that have a
+ * specialised one (all OU pairs); the results must be identical */
+#define MDG_FLAG_GENERIC_FILL 2
 
 /* derived accounting, Portfolio.cpp:140-235,243-252; any pointer may be NULL */
 typedef struct MdgDerived {
@@ -292,7 +295,9 @@ int mdg_reset(const MdgParams *params, const MdgState *state, const MdgStepIO *i
  * resetting envs are compacted into a list and ONE kernel refills them, a block per listed env (Philox +
  * Box-Muller of the whole history packed over the block into shared memory, then the serial recurrences of the
  * env's generator groups on neighbouring lanes) -- many times faster than mdg_reset when a few percent of the
- * envs reset every step.  workspace == NULL falls back to mdg_reset.  The first 256 bytes of the workspace are a
+ * envs reset every step.  When every asset belongs to an OU pair, there are at least 8 assets and the normals
+ * come from Philox, the refill runs one lane per (env, pair) instead, with bit-identical results
+ * (MDG_FLAG_GENERIC_FILL forces the generic kernel).  workspace == NULL falls back to mdg_reset.  The first 256 bytes of the workspace are a
  * header (list length, exit ticket) that must be ZERO before the first use; every call leaves it zero again. */
 int mdg_reset_ws(const MdgParams *params, const MdgState *state, const MdgStepIO *io,
                  const MdgLaunch *launch, const uint8_t *mask, int fill_ticks, int clear_nstep,

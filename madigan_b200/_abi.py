@@ -7,6 +7,7 @@ import ctypes as C
 
 MDG_ABI_VERSION = 12
 FLAG_FORCE_EXACT_GATE = 1
+FLAG_GENERIC_FILL = 2
 XFORM_NONE, XFORM_PAIR_RATIO, XFORM_RETURNS = 0, 1, 2
 MDG_MAX_ASSETS = 16
 MDG_GEN_NPARAM = 10

@@ -1,6 +1,8 @@
 // extern "C" entry points of the step path + the (rare, non-unrolled) reset / init kernels.
 #include <stdlib.h>
 
+#include <atomic>
+
 #include "mdg_step_kernel.cuh"
 
 namespace mdg {
@@ -319,6 +321,126 @@ __global__ void __launch_bounds__(kFillBlock) reset_fill_kernel(const __grid_con
   }
 }
 
+// The refill of the all-OU-pairs parameter sets (all_ou_pairs(P)) when the normals come from Philox: one lane per
+// (listed env, pair), np = nA/2 lanes per env, 128/np envs per block.  A pair is an independent process whose three
+// normals per tick (slots 3p, 3p+1, 3p+2) are two Philox blocks, so every lane draws its own normals in registers and
+// runs its pair's recurrence without shared memory or a barrier inside the tick loop; the tick loop is unrolled so that
+// the next ticks' Philox overlaps the current tick's dependent chain.  (Pairs 2q and 2q+1 share block 3q+1: measured,
+// swapping its halves between the two lanes beats drawing it twice, profiles/r3_notes.md.)  The draws, the recurrence
+// and the stores are reset_fill_kernel's expression for expression (same translation unit, same -fmad=false), so the
+// two kernels write bit-identical results.
+// -DMDG_FILL_PAIRS_UNROLL / -DMDG_FILL_PAIRS_MINB (profiling builds): tick-loop unroll and the minimum resident blocks
+// per SM the register budget is sized for
+#ifndef MDG_FILL_PAIRS_UNROLL
+#define MDG_FILL_PAIRS_UNROLL 4
+#endif
+#ifndef MDG_FILL_PAIRS_MINB
+#define MDG_FILL_PAIRS_MINB 1
+#endif
+constexpr int kFillPairsUnroll = MDG_FILL_PAIRS_UNROLL;
+__global__ void __launch_bounds__(kFillBlock, MDG_FILL_PAIRS_MINB) reset_fill_pairs_kernel(const __grid_constant__ ResetWsArgs a) {
+  const MdgParams& P = a.P;
+  const int tid = threadIdx.x;
+  const int na = P.n_assets, np = na >> 1, epb = kFillBlock / np;
+  const int slot = tid / np, p = tid - slot * np;  // env of the group, pair of the env
+  const int fill = a.fill_ticks, k = a.L.window;
+  const int64_t N = a.L.n_envs;
+  const int listed = *(volatile int*)a.count;
+  const int count = (int64_t)listed < N ? listed : (int)N;  // a stale header cannot index past the list
+  const double cash = P.init_cash;
+  const double eq = cash + 0. - 0.;              // flat portfolio: equity == cash
+  const bool eq_plain = eq > 0. && eq < 1e300;   // then (0*p)/eq == 0*p exactly
+  const uint32_t k0 = (uint32_t)a.L.seed, k1 = (uint32_t)(a.L.seed >> 32);
+  const int i0 = 2 * p;
+  const MdgAssetGen &g0 = P.gen[i0], &g1 = P.gen[i0 + 1];
+  const double theta0 = g0.p[0], phi0 = g0.p[1], noise = g0.p[2], theta1 = g1.p[0], phi1 = g1.p[1];
+  // slot s = Philox block s>>1, output s&1: pair p reads blocks b and b+1, b = 3p>>1
+  const uint32_t blk = (uint32_t)(3 * p) >> 1;
+  const bool odd = p & 1;
+  for (int d0 = blockIdx.x * epb; d0 < count; d0 += gridDim.x * epb) {
+    const int d = d0 + slot;
+    const bool active = slot < epb && d < count;
+    const int64_t e = active ? a.list[d] : 0;
+    const long long ts0 = active ? a.S.timestamp[e] : 0;
+    __syncthreads();  // every lane of an env has read the old timestamp before its pair-0 lane writes the new one
+    // idle lanes run the tick loop too (without storing): the loop's shuffles take every lane of the warp
+    if (active && p == 0) {  // fresh Broker/Account/Portfolio (Env.h:150-165): per-env scalars
+      if (a.clear_nstep && a.S.nstep_len) a.S.nstep_len[e] = 0;  // offpolicy_q.py:94
+      a.S.cash[e] = cash;
+      if (a.S.folds) {  // flat portfolio: every fold is a sum of zeros
+        a.S.folds[(int64_t)MDG_FOLD_AV * N + e] = 0.;
+        a.S.folds[(int64_t)MDG_FOLD_ML * N + e] = 0.;
+        a.S.folds[(int64_t)MDG_FOLD_BM * N + e] = 0.;
+        a.S.folds[(int64_t)MDG_FOLD_SE * N + e] = 0.;
+        a.S.folds[(int64_t)MDG_FOLD_G * N + e] = fabs(cash);
+      }
+      a.S.timestamp[e] = ts0 + fill;
+      a.S.reset_ts[e] = ts0 + fill;
+      a.IO.obs_port[((int64_t)a.L.head * (na + 1)) * N + e] = (cash - 0.) / eq;  // newest row = current state
+    }
+    for (int c = 0; c < 2 && active; ++c) {  // the empty ledger
+      a.S.ledger[(int64_t)(i0 + c) * N + e] = 0.;
+      a.S.mean_entry[(int64_t)(i0 + c) * N + e] = 0.;
+      a.S.borrowed[(int64_t)(i0 + c) * N + e] = 0.;
+    }
+    // OUPair::reset (gen_reset, DataSource.cpp:1242-1246) draws nothing: the shared mean and both prices restart at 10
+    double m = 10., pr0 = 10., pr1 = 10.;
+    const uint32_t gid = (uint32_t)(a.L.env_offset + e);
+    double2* prow = reinterpret_cast<double2*>(a.IO.pre_price + ((int64_t)e * k + (k - fill)) * na) + p;
+    auto tick = [&](int t, double z_rw, double z_0, double z_1) {  // OUPair::getData (DataSource.cpp:1232-1240)
+      m += m * (z_rw * noise);
+      pr0 += (theta0 * (m - pr0)) + m * (z_0 * phi0);
+      pr1 += (theta1 * (m - pr1)) + m * (z_1 * phi1);
+      if (active) prow[(int64_t)t * np] = make_double2(pr0, pr1);  // a warp's tick: 128 contiguous bytes per env
+    };
+    int t = 0;
+    if ((np & 1) == 0) {
+      // pairs 2q and 2q+1 sit on neighbouring lanes of one warp and share Philox block 3q+1: of two ticks, the even
+      // lane draws it for the first and the odd lane for the second, and each hands the other the half it needs
+      const uint32_t b_own = odd ? blk + 1 : blk, b_sh = odd ? blk : blk + 1;
+#pragma unroll kFillPairsUnroll / 2
+      for (; t + 1 < fill; t += 2) {
+        const unsigned long long ta = (unsigned long long)ts0 + (unsigned)t, tb = ta + 1, tsh = odd ? tb : ta;
+        double oa0, oa1, ob0, ob1, s0, s1;
+        normal_block(gid, b_own, (uint32_t)ta, (uint32_t)(ta >> 32), k0, k1, oa0, oa1);
+        normal_block(gid, b_own, (uint32_t)tb, (uint32_t)(tb >> 32), k0, k1, ob0, ob1);
+        normal_block(gid, b_sh, (uint32_t)tsh, (uint32_t)(tsh >> 32), k0, k1, s0, s1);
+        const double recv = __shfl_xor_sync(0xffffffffu, odd ? s0 : s1, 1);
+        const double sa = odd ? recv : s0, sb = odd ? s1 : recv;  // this lane's half of the shared block
+        tick(t, odd ? sa : oa0, odd ? oa0 : oa1, odd ? oa1 : sa);
+        tick(t + 1, odd ? sb : ob0, odd ? ob0 : ob1, odd ? ob1 : sb);
+      }
+    }
+#pragma unroll kFillPairsUnroll
+    for (; t < fill; ++t) {  // an odd number of pairs, or the last of an odd number of ticks: both blocks per lane
+      const unsigned long long tk = (unsigned long long)ts0 + (unsigned)t;
+      double l0, l1, h0, h1;
+      normal_block(gid, blk, (uint32_t)tk, (uint32_t)(tk >> 32), k0, k1, l0, l1);
+      normal_block(gid, blk + 1, (uint32_t)tk, (uint32_t)(tk >> 32), k0, k1, h0, h1);
+      tick(t, odd ? l1 : l0, odd ? h0 : l1, odd ? h1 : h0);
+    }
+    if (!active) continue;
+    a.IO.obs_price[((int64_t)a.L.head * na + i0) * N + e] = pr0;  // newest row = current state, also in the ring
+    a.IO.obs_price[((int64_t)a.L.head * na + i0 + 1) * N + e] = pr1;
+    a.IO.obs_port[((int64_t)a.L.head * (na + 1) + i0 + 1) * N + e] = eq_plain ? 0. * pr0 : (0. * pr0) / eq;
+    a.IO.obs_port[((int64_t)a.L.head * (na + 1) + i0 + 2) * N + e] = eq_plain ? 0. * pr1 : (0. * pr1) / eq;
+    a.S.gstate[(int64_t)g0.gslot * N + e] = m;
+    a.S.price[(int64_t)i0 * N + e] = pr0;
+    a.S.price[(int64_t)(i0 + 1) * N + e] = pr1;
+  }
+  // self-cleaning header: the last block to leave zeroes the count for the next step kernel
+  __syncthreads();
+  if (tid == 0) {
+    __threadfence();
+    const int t = atomicAdd(a.ticket, 1);
+    if (t == (int)gridDim.x - 1) {
+      *a.count = 0;
+      *a.ticket = 0;
+      __threadfence();
+    }
+  }
+}
+
 // constructor state (Env.h:139-165 before the first tick)
 struct InitArgs {
   MdgParams P;
@@ -507,17 +629,48 @@ static int fill_ws_args(ResetWsArgs& a, const MdgParams* P, const MdgState* S, c
   }
   return MDG_OK;
 }
+// SM count of the current device, looked up once per device ordinal
+static int64_t sm_count() {
+  constexpr int kMaxDevices = 64;
+  static std::atomic<int> cached[kMaxDevices];
+  int dev = 0, n = 0;
+  if (cudaGetDevice(&dev) != cudaSuccess || dev < 0) dev = 0;
+  if (dev < kMaxDevices) n = cached[dev].load(std::memory_order_relaxed);
+  if (n == 0) {
+    if (cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || n <= 0) n = 148;
+    if (dev < kMaxDevices) cached[dev].store(n, std::memory_order_relaxed);
+  }
+  return n;
+}
+// all-OU-pairs refill: blocks per SM of its grid (grid-stride over groups of envs beyond that)
+constexpr int kFillPairsBlocksPerSm = 2;
+// ... and the fewest assets it is taken for: a lane runs its pair's 64 ticks in series (~20 us), where the generic kernel
+// spreads an env's draws over a block (~12 us).  With few pairs per env that latency is not paid back: one OU pair per
+// env (C3, 65,536 envs, one stream) measured 20.5 us per step with the generic refill, 34.9 with this one.
+constexpr int kFillPairsMinAssets = 8;
 static int launch_fill(const ResetWsArgs& a, int64_t max_listed) {
   // the count is on the device: size the grid for the most the list can hold, capped at a few blocks per SM
   // (grid-stride; blocks past the end of the list only read the count and take their exit ticket)
-  static const int64_t cap = []() {  // MDG_FILL_GRID: profiling knob
+  static const int64_t knob = []() {  // MDG_FILL_GRID: profiling knob
     const char* v = getenv("MDG_FILL_GRID");
     const long n = v ? atol(v) : 0;
-    return (int64_t)(n > 0 ? n : 148 * 8);
+    return (int64_t)(n > 0 ? n : 0);
   }();
+  cudaStream_t st = (cudaStream_t)a.L.stream;
+  if (!(a.L.flags & MDG_FLAG_GENERIC_FILL) && !a.IO.normals && !a.IO.uniforms && a.P.n_assets >= kFillPairsMinAssets &&
+      all_ou_pairs(a.P) &&
+      (reinterpret_cast<uintptr_t>(a.IO.pre_price) & 15) == 0) {
+    const int64_t epb = kFillBlock / (a.P.n_assets / 2);
+    const int64_t groups = (max_listed + epb - 1) / epb;
+    const int64_t cap = knob ? knob : kFillPairsBlocksPerSm * sm_count();
+    const unsigned grid = (unsigned)(groups < cap ? (groups > 0 ? groups : 1) : cap);
+    reset_fill_pairs_kernel<<<grid, kFillBlock, 0, st>>>(a);
+    return cuda_err(cudaGetLastError(), "reset_fill_pairs launch");
+  }
+  const int64_t cap = knob ? knob : 148 * 8;
   const unsigned grid = (unsigned)(max_listed < cap ? (max_listed > 0 ? max_listed : 1) : cap);
   const size_t smem = sizeof(double) * (size_t)a.chunk * (size_t)(a.P.n_normals > 0 ? a.P.n_normals : 1);
-  reset_fill_kernel<<<grid, kFillBlock, smem, (cudaStream_t)a.L.stream>>>(a);
+  reset_fill_kernel<<<grid, kFillBlock, smem, st>>>(a);
   return cuda_err(cudaGetLastError(), "reset_fill launch");
 }
 }  // namespace mdg

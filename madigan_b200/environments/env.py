@@ -138,7 +138,7 @@ class Env:
         self._version = 0
         self._derived_version = -1
         self.launches = 0  # kernels launched so far (bench.py's gpu_launches)
-        self.flags = 0     # MdgLaunch.flags (validation: A.FLAG_FORCE_EXACT_GATE)
+        self.flags = 0     # MdgLaunch.flags (validation: A.FLAG_FORCE_EXACT_GATE, A.FLAG_GENERIC_FILL)
         with torch.cuda.device(self.device):
             check(self._lib.mdg_init_state(C.byref(self.P), C.byref(self.R), C.byref(self._S), C.byref(self._launch())))
             self.launches += 1
