@@ -28,7 +28,7 @@
 extern "C" {
 #endif
 
-#define MDG_ABI_VERSION 12
+#define MDG_ABI_VERSION 13
 #define MDG_MAX_ASSETS 16
 #define MDG_GEN_NPARAM 10
 #define MDG_MAX_NSTEP 64
@@ -271,8 +271,8 @@ enum MdgNorm {
 
 int mdg_abi_version(void);
 /* sizeof of the ABI structs as compiled: 0 MdgAssetGen 1 MdgParams 2 MdgReward 3 MdgState 4 MdgStepIO
- * 5 MdgLaunch 6 MdgDerived 7 MdgWindow 8 MdgReplay 9 MdgReplayBatch 10 MdgRewardNorm 11 MdgTearsheet; -1 for an unknown
- * index (lets a binding verify its struct mirror) */
+ * 5 MdgLaunch 6 MdgDerived 7 MdgWindow 8 MdgReplay 9 MdgReplayBatch 10 MdgRewardNorm 11 MdgTearsheet
+ * 12 MdgPrioritized; -1 for an unknown index (lets a binding verify its struct mirror) */
 int mdg_sizeof(int which);
 const char *mdg_last_error(void);
 
@@ -408,6 +408,66 @@ typedef struct MdgReplayBatch {
 int mdg_replay_sample(const MdgReplay *rp, int64_t n_envs, int64_t cur_step, const void *obs_price,
                       const double *obs_port, int32_t window_elems, int32_t n_port, int32_t obs_dtype,
                       int64_t batch, uint64_t seed, uint64_t draw, const MdgReplayBatch *out, void *stream);
+
+/* ---------------------------------------------------------------------------------------------------
+ * Proportional prioritized replay over the ring of MdgReplay (Schaul et al. 2016, the segment-tree form of the
+ * reference's PrioritizedReplayBuffer, utils/buffers/prioritized_replay_buffer.py + segment_tree.py).
+ *
+ * A sum tree and a min tree in heap layout over the ring's slots: node 1 is the root, node j has the children 2j and
+ * 2j+1, the leaf of ring slot i is node tree_size + i (tree_size: a power of two >= max(capacity, 1024)).  Every
+ * internal node is left + right (min(left, right)), recomputed from its two children, so a tree is a pure function of
+ * its leaves.  An unfilled leaf is 0 in the sum tree and +inf in the min tree.
+ *   ingest  every record appended since the last ingest takes the leaf max_priority ** alpha (max_priority starts at
+ *           1); a slot the ring overwrites takes the new record's priority.
+ *   sample  total = sum root, seg = total / batch.  Sample b draws u (Philox, below) and descends with the mass
+ *           u * seg + b * seg: at each node, go left if the left child > mass, else subtract it and go right.  A leaf
+ *           that is unfilled, has priority 0, or is stale (its state's observation slot was overwritten, the test of
+ *           mdg_replay_sample) is rejected and redrawn from the whole distribution (mass u * total, a fresh draw);
+ *           after 64 attempts the row is idx = -1, position -1, weight 0, a zero row with done = 1.
+ *           weight = (p_i / total * n) ** -beta / (p_min / total * n) ** -beta, n = filled records,
+ *           p_min = the min root.
+ *   update  applies to the batch of the last sample, in batch order as a sequential loop would: idx = -1 is
+ *           skipped; so is a record the ring overwrote since it was sampled (leaf_pos differs from the sampled
+ *           position); a priority that is not finite or not > 0 is skipped and counted in n_rejected; otherwise the
+ *           leaf becomes priority ** alpha and max_priority = max(max_priority, priority).  Of an index that appears
+ *           twice, the last occurrence wins.
+ * Philox: sample b, attempt a uses the counter (b lo, (b hi) ^ (a << 8) ^ 0x80000000, draw lo, draw hi) with the
+ * key seed, u = (x0 >> 11) 2^-53; bit 31 of the second word keeps these draws apart from mdg_replay_sample's.
+ * Deviation (documented): a stale leaf keeps its mass until the ring overwrites it.  Rejection keeps sampling exactly
+ * proportional over the resident records, but the weights' total and p_min include the stale leaves.
+ * Every call enqueues a fixed number of launches with grids known to the host and never synchronises, so ingest,
+ * sample and update can be captured in a CUDA graph.  Trees are rebuilt per 1024-leaf subtree: the calls that change
+ * leaves list the subtrees they touch, one refresh kernel rebuilds the listed ones and its last block the levels
+ * above them. */
+typedef struct MdgPrioritized {
+  double *sum_tree, *min_tree;   /* [2 * tree_size], node 0 unused */
+  int64_t *leaf_pos;             /* [capacity] cursor position of the record in each slot, -1 = unfilled */
+  int32_t *batch_pos;            /* [capacity] mdg_per_update scratch (last batch position per leaf), -1 between calls */
+  uint32_t *dirty;               /* [tree_size / 1024] subtree marks, 0 between calls */
+  int32_t *dirty_list;           /* [tree_size / 1024] the marked subtrees */
+  uint32_t *ctl;                 /* [4] marked count, refresh exit ticket, ingest exit ticket, unused: zero before the
+                                    first call, left zero by every call */
+  unsigned long long *seen;      /* [1] MdgReplay.cursor as of the last ingest, 0 at first */
+  double *max_priority;          /* [1] 1.0 at first */
+  unsigned long long *n_rejected;/* [1] priorities update skipped as not finite or not > 0 */
+  int64_t capacity;              /* == MdgReplay.capacity */
+  int64_t tree_size;
+  double alpha;
+} MdgPrioritized;
+
+/* After mdg_replay_append on the same stream (PrioritizedReplayBuffer.add): leaves of the records appended since
+ * the last call.  max_new: a bound on their count (n_envs * nstep), sizes the grid. */
+int mdg_per_ingest(const MdgPrioritized *pr, const MdgReplay *rp, int64_t max_new, void *stream);
+/* PrioritizedReplayBuffer.sample: the arguments and the gather of mdg_replay_sample, plus weights [batch] f64 and the
+ * sampled records' cursor positions pos [batch] int64 (what mdg_per_update checks against overwrites). */
+int mdg_per_sample(const MdgPrioritized *pr, const MdgReplay *rp, int64_t n_envs, int64_t cur_step,
+                   const void *obs_price, const double *obs_port, int32_t window_elems, int32_t n_port,
+                   int32_t obs_dtype, int64_t batch, double beta, uint64_t seed, uint64_t draw,
+                   const MdgReplayBatch *out, double *weights, int64_t *pos, void *stream);
+/* PrioritizedReplayBuffer.update_priorities for the batch of the last sample: idx and pos as mdg_per_sample wrote
+ * them, priorities [batch] f64. */
+int mdg_per_update(const MdgPrioritized *pr, int64_t batch, const int64_t *idx, const int64_t *pos,
+                   const double *priorities, void *stream);
 
 /* ---------------------------------------------------------------------------------------------------
  * Streaming reward normalisers (environments/reward_normalization.pyx:14-272): one scalar state machine per env,

@@ -5,7 +5,7 @@ checks the struct sizes against the compiled library (``mdg_sizeof``).
 """
 import ctypes as C
 
-MDG_ABI_VERSION = 12
+MDG_ABI_VERSION = 13
 FLAG_FORCE_EXACT_GATE = 1
 FLAG_GENERIC_FILL = 2
 XFORM_NONE, XFORM_PAIR_RATIO, XFORM_RETURNS = 0, 1, 2
@@ -111,6 +111,12 @@ class MdgReplayBatch(C.Structure):
                                    "reward", "done")]
 
 
+class MdgPrioritized(C.Structure):
+    _fields_ = [(n, _dp) for n in ("sum_tree", "min_tree", "leaf_pos", "batch_pos", "dirty", "dirty_list", "ctl",
+                                   "seen", "max_priority", "n_rejected")] + \
+               [("capacity", C.c_int64), ("tree_size", C.c_int64), ("alpha", C.c_double)]
+
+
 RN_NULL, RN_SHARPE_FIXED, RN_SORTINO_A, RN_SORTINO_B, RN_SORTINO_C, RN_SHARPE_EWMA = range(6)
 
 
@@ -150,6 +156,11 @@ SYMBOLS = {
                                     C.c_void_p, C.c_void_p, C.c_void_p]),
     "mdg_replay_sample": (C.c_int, [_P(MdgReplay), C.c_int64, C.c_int64, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32,
                                     C.c_int32, C.c_int64, C.c_uint64, C.c_uint64, _P(MdgReplayBatch), C.c_void_p]),
+    "mdg_per_ingest": (C.c_int, [_P(MdgPrioritized), _P(MdgReplay), C.c_int64, C.c_void_p]),
+    "mdg_per_sample": (C.c_int, [_P(MdgPrioritized), _P(MdgReplay), C.c_int64, C.c_int64, C.c_void_p, C.c_void_p,
+                                 C.c_int32, C.c_int32, C.c_int32, C.c_int64, C.c_double, C.c_uint64, C.c_uint64,
+                                 _P(MdgReplayBatch), C.c_void_p, C.c_void_p, C.c_void_p]),
+    "mdg_per_update": (C.c_int, [_P(MdgPrioritized), C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "mdg_materialise_time": (C.c_int, [C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p]),
     "mdg_episode_stats": (C.c_int, [_P(MdgParams), _P(MdgState), _P(MdgStepIO), _P(MdgLaunch),
                                     C.c_void_p]),
@@ -171,4 +182,4 @@ def bind(lib):
 
 
 STRUCTS = (MdgAssetGen, MdgParams, MdgReward, MdgState, MdgStepIO, MdgLaunch, MdgDerived, MdgWindow, MdgReplay,
-           MdgReplayBatch, MdgRewardNorm, MdgTearsheet)  # mdg_sizeof order
+           MdgReplayBatch, MdgRewardNorm, MdgTearsheet, MdgPrioritized)  # mdg_sizeof order

@@ -53,7 +53,7 @@ def _deps_hash(src="", defs=()):
 
 def _units():
     return [("mdg_api.o", "mdg_api.cu", []), ("mdg_aux.o", "mdg_aux.cu", []), ("mdg_replay.o", "mdg_replay.cu", []),
-            ("mdg_rewardnorm.o", "mdg_rewardnorm.cu", []), ("mdg_tearsheet.o", "mdg_tearsheet.cu", [])]
+            ("mdg_per.o", "mdg_per.cu", []), ("mdg_rewardnorm.o", "mdg_rewardnorm.cu", []), ("mdg_tearsheet.o", "mdg_tearsheet.cu", [])]
 
 
 def build(force=False, verbose=False, ptxas_info=False):

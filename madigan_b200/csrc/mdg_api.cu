@@ -772,6 +772,7 @@ extern "C" int mdg_sizeof(int which) {
     case 9: return (int)sizeof(MdgReplayBatch);
     case 10: return (int)sizeof(MdgRewardNorm);
     case 11: return (int)sizeof(MdgTearsheet);
+    case 12: return (int)sizeof(MdgPrioritized);
   }
   return -1;
 }

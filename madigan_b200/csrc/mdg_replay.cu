@@ -1,7 +1,7 @@
 // Device-side n-step replay ingest and sampling (include/madigan_b200.h, "Device-side n-step replay ingest").
 #include <stdio.h>
 
-#include "mdg_common.cuh"
+#include "mdg_replay.cuh"
 
 namespace mdg {
 
@@ -59,17 +59,14 @@ __global__ void __launch_bounds__(256) replay_append_kernel(const __grid_constan
 
 struct SampleArgs {
   MdgReplay rp;
-  int64_t N, cur_step, batch;
-  const void* obs_price;
-  const double* obs_port;
-  int welems, n_port, dtype;
+  int64_t cur_step, batch;
   uint64_t seed, draw;
-  MdgReplayBatch out;
+  GatherArgs g;
 };
 
 // one block per sample: thread 0 draws a non-stale transition (ReplayBuffer._sample_idxs, replay_buffer.py:107-108:
 // uniform over the filled part), then the block copies the two windows and the small fields
-__global__ void __launch_bounds__(128) replay_sample_kernel(const __grid_constant__ SampleArgs a) {
+__global__ void __launch_bounds__(kGatherThreads) replay_sample_kernel(const __grid_constant__ SampleArgs a) {
   __shared__ long long s_idx;
   const MdgReplay& r = a.rp;
   const int64_t b = blockIdx.x;
@@ -83,62 +80,14 @@ __global__ void __launch_bounds__(128) replay_sample_kernel(const __grid_constan
                     (uint32_t)a.seed, (uint32_t)(a.seed >> 32), x0, x1);
       const unsigned long long j = (unsigned long long)(((x0 >> 11) * 0x1.0p-53) * (double)filled);
       const long long cand = (long long)(j < filled ? j : filled - 1);
-      // the observation slot of the state must not have been overwritten: it survives `depth` steps
-      const long long sstep = r.t_state_step[cand];  // LLONG_MIN = never written (step -1 is observe_start's slot)
-      if (sstep != (-9223372036854775807LL - 1) && sstep > a.cur_step - r.depth) { pick = cand; break; }
+      if (replay_resident(r, cand, a.cur_step)) { pick = cand; break; }
     }
     s_idx = pick;
   }
   __syncthreads();
   const long long idx = s_idx;
-  if (threadIdx.x == 0) a.out.idx[b] = idx;
-  if (idx < 0) {  // no resident transition found: a zero row, flagged by idx = -1 and masked by done = 1
-    const int64_t o_b = b * a.welems;
-    if (a.dtype == MDG_DTYPE_F32) {
-      float* d0 = (float*)a.out.state_price; float* d1 = (float*)a.out.next_price;
-      for (int i = threadIdx.x; i < a.welems; i += 128) { d0[o_b + i] = 0.f; d1[o_b + i] = 0.f; }
-    } else {
-      double* d0 = (double*)a.out.state_price; double* d1 = (double*)a.out.next_price;
-      for (int i = threadIdx.x; i < a.welems; i += 128) { d0[o_b + i] = 0.; d1[o_b + i] = 0.; }
-    }
-    for (int i = threadIdx.x; i < a.n_port; i += 128) { a.out.state_port[b * a.n_port + i] = 0.; a.out.next_port[b * a.n_port + i] = 0.; }
-    for (int i = threadIdx.x; i < r.n_action; i += 128) a.out.action[b * r.n_action + i] = 0.;
-    for (int i = threadIdx.x; i < r.ra; i += 128) a.out.reward[b * r.ra + i] = 0.;
-    if (threadIdx.x == 0) a.out.done[b] = 1;
-    return;
-  }
-  const int64_t e = r.t_env[idx];
-  const int64_t ss = r.t_state_slot[idx], sn = r.t_next_slot[idx];
-  const int64_t o_s = (ss * a.N + e) * a.welems, o_n = (sn * a.N + e) * a.welems, o_b = b * a.welems;
-  if (a.dtype == MDG_DTYPE_F32) {
-    const float* src = (const float*)a.obs_price;
-    float* d0 = (float*)a.out.state_price;
-    float* d1 = (float*)a.out.next_price;
-    for (int i = threadIdx.x; i < a.welems; i += 128) { d0[o_b + i] = src[o_s + i]; d1[o_b + i] = src[o_n + i]; }
-  } else {
-    const double* src = (const double*)a.obs_price;
-    double* d0 = (double*)a.out.state_price;
-    double* d1 = (double*)a.out.next_price;
-    for (int i = threadIdx.x; i < a.welems; i += 128) { d0[o_b + i] = src[o_s + i]; d1[o_b + i] = src[o_n + i]; }
-  }
-  for (int i = threadIdx.x; i < a.n_port; i += 128) {
-    a.out.state_port[b * a.n_port + i] = a.obs_port[(ss * a.N + e) * a.n_port + i];
-    a.out.next_port[b * a.n_port + i] = a.obs_port[(sn * a.N + e) * a.n_port + i];
-  }
-  for (int i = threadIdx.x; i < r.n_action; i += 128) a.out.action[b * r.n_action + i] = r.t_action[idx * r.n_action + i];
-  for (int i = threadIdx.x; i < r.ra; i += 128) a.out.reward[b * r.ra + i] = r.t_reward[idx * r.ra + i];
-  if (threadIdx.x == 0) a.out.done[b] = r.t_done[idx];
-}
-
-static int check_replay(const MdgReplay* rp) {
-  if (!rp) return set_err(MDG_E_INVALID, "null replay");
-  if (!rp->t_env || !rp->t_state_slot || !rp->t_next_slot || !rp->t_state_step || !rp->t_done || !rp->t_reward ||
-      !rp->t_action || !rp->cursor || !rp->act_ring)
-    return set_err(MDG_E_INVALID, "replay storage pointer is null");
-  if (rp->capacity < 1 || rp->depth < 2 || rp->nstep < 1 || rp->nstep > MDG_MAX_NSTEP || rp->ra < 1 || rp->n_action < 1)
-    return set_err(MDG_E_INVALID, "bad replay dimensions");
-  if (rp->depth <= rp->nstep) return set_err(MDG_E_INVALID, "replay depth must exceed nstep");
-  return MDG_OK;
+  if (threadIdx.x == 0) a.g.out.idx[b] = idx;
+  replay_gather(r, a.g, b, idx);
 }
 
 }  // namespace mdg
@@ -167,16 +116,13 @@ extern "C" int mdg_replay_sample(const MdgReplay* rp, int64_t n_envs, int64_t cu
                                  void* stream) {
   int rc = check_replay(rp);
   if (rc) return rc;
-  if (!obs_price || !obs_port || !out) return set_err(MDG_E_INVALID, "null sample input");
-  if (!out->idx || !out->state_price || !out->next_price || !out->state_port || !out->next_port || !out->action ||
-      !out->reward || !out->done)
-    return set_err(MDG_E_INVALID, "null sample output");
-  if (obs_dtype != MDG_DTYPE_F64 && obs_dtype != MDG_DTYPE_F32) return set_err(MDG_E_INVALID, "bad obs dtype");
-  if (window_elems < 1 || n_port < 1) return set_err(MDG_E_INVALID, "bad window/portfolio size");
+  rc = check_gather(obs_price, obs_port, window_elems, n_port, obs_dtype, out);
+  if (rc) return rc;
   if (batch <= 0) return batch == 0 ? MDG_OK : set_err(MDG_E_INVALID, "batch < 0");
   SampleArgs a;
-  a.rp = *rp; a.N = n_envs; a.cur_step = cur_step; a.batch = batch; a.obs_price = obs_price; a.obs_port = obs_port;
-  a.welems = window_elems; a.n_port = n_port; a.dtype = obs_dtype; a.seed = seed; a.draw = draw; a.out = *out;
-  replay_sample_kernel<<<(unsigned)batch, 128, 0, (cudaStream_t)stream>>>(a);
+  a.rp = *rp; a.cur_step = cur_step; a.batch = batch; a.seed = seed; a.draw = draw;
+  a.g.N = n_envs; a.g.obs_price = obs_price; a.g.obs_port = obs_port; a.g.welems = window_elems; a.g.n_port = n_port;
+  a.g.dtype = obs_dtype; a.g.out = *out;
+  replay_sample_kernel<<<(unsigned)batch, kGatherThreads, 0, (cudaStream_t)stream>>>(a);
   return cuda_err(cudaGetLastError(), "mdg_replay_sample launch");
 }

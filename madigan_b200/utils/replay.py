@@ -87,10 +87,8 @@ class DeviceReplay:
         return min(int(self.t["cursor"].item()), self.capacity)
 
     # ------------------------------------------------------------------ sample
-    def sample(self, n):
-        """``ReplayBuffer.sample`` (replay_buffer.py:94-103): (SARSD of batched tensors, None).  Runs on the env's
-        stream (``Env.bind_stream``).  ``self.last_valid`` flags the rows that hold a real transition (all of them
-        unless the ring is nearly empty or mostly stale)."""
+    def _batch_out(self, n):
+        """Output tensors of a batch of n and the MdgReplayBatch pointing at them."""
         dev = self.env.device
         out = self._out.get(n)
         if out is None:  # output buffers are allocated once per batch size and reused (a sample is consumed by the
@@ -104,17 +102,120 @@ class DeviceReplay:
                 action=torch.empty((n, self.n_action), dtype=torch.float64, device=dev),
                 reward=torch.empty((n, self.ra), dtype=torch.float64, device=dev),
                 done=torch.empty(n, dtype=torch.uint8, device=dev))
-        b = A.MdgReplayBatch(**{k_: v.data_ptr() for k_, v in out.items()})
-        self.draws += 1
-        with torch.cuda.device(dev):
-            check(self._lib.mdg_replay_sample(
-                C.byref(self._rp), self.N, self.step_count, self.obs_price.data_ptr(), self.obs_port.data_ptr(),
-                self.k * self.nF, self.n_port, A.DTYPE_F32 if self.dtype == torch.float32 else A.DTYPE_F64, n,
-                self.seed, self.draws, C.byref(b), self.env._sptr()))
+        return out, A.MdgReplayBatch(**{k_: v.data_ptr() for k_, v in out.items()})
+
+    def _sarsd(self, out):
         self.last_idx = out["idx"]
         # (batch,) bool: False where 64 draws found no resident transition (the row is zero-filled with done = True)
         with self.env._copy_ctx():
             self.last_valid = out["idx"] >= 0
-        sarsd = SARSD(State(out["state_price"], out["state_port"], None), out["action"], out["reward"],
-                      State(out["next_price"], out["next_port"], None), out["done"].bool())
-        return sarsd, None
+        return SARSD(State(out["state_price"], out["state_port"], None), out["action"], out["reward"],
+                     State(out["next_price"], out["next_port"], None), out["done"].bool())
+
+    def sample(self, n):
+        """``ReplayBuffer.sample`` (replay_buffer.py:94-103): (SARSD of batched tensors, None).  Runs on the env's
+        stream (``Env.bind_stream``).  ``self.last_valid`` flags the rows that hold a real transition (all of them
+        unless the ring is nearly empty or mostly stale)."""
+        out, b = self._batch_out(n)
+        self.draws += 1
+        with torch.cuda.device(self.env.device):
+            check(self._lib.mdg_replay_sample(
+                C.byref(self._rp), self.N, self.step_count, self.obs_price.data_ptr(), self.obs_port.data_ptr(),
+                self.k * self.nF, self.n_port, A.DTYPE_F32 if self.dtype == torch.float32 else A.DTYPE_F64, n,
+                self.seed, self.draws, C.byref(b), self.env._sptr()))
+        return self._sarsd(out), None
+
+
+class DevicePrioritizedReplay(DeviceReplay):
+    """Proportional prioritized replay (Schaul et al. 2016; the reference's PrioritizedReplayBuffer over sum/min
+    segment trees, utils/buffers/prioritized_replay_buffer.py + segment_tree.py) on the device ring of DeviceReplay.
+
+    A record enters with priority ``max_priority ** alpha``; ``sample(n, beta)`` draws records with probability
+    proportional to their priority among the resident ones and returns importance weights beside the batch;
+    ``update_priorities`` sets the priorities of the last sample's records (|TD| + eps, made by the caller).  Trees,
+    draws and updates stay on the device and on the env's stream, with no host synchronisation: ``add``, ``sample``
+    and ``update_priorities`` can be captured in a CUDA graph.  Semantics and the one documented deviation (stale
+    records count in the weights' normalisers): include/madigan_b200.h, "Proportional prioritized replay"."""
+
+    def __init__(self, env, alpha=0.6, depth=64, capacity=None, n_action=None, norm_type=None, dtype=torch.float32,
+                 seed=0):
+        super().__init__(env, depth=depth, capacity=capacity, n_action=n_action, norm_type=norm_type, dtype=dtype,
+                         seed=seed)
+        self.alpha = float(alpha)
+        if not self.alpha >= 0:
+            raise ValueError("alpha must be >= 0")
+        cap = self.capacity
+        T = max(1024, 1 << (cap - 1).bit_length())
+        self.tree_size = T
+        dev = env.device
+        S = T // 1024
+        self.per = dict(sum_tree=torch.zeros(2 * T, dtype=torch.float64, device=dev),
+                        min_tree=torch.full((2 * T,), float("inf"), dtype=torch.float64, device=dev),
+                        leaf_pos=torch.full((cap,), -1, dtype=torch.int64, device=dev),
+                        batch_pos=torch.full((cap,), -1, dtype=torch.int32, device=dev),
+                        dirty=torch.zeros(S, dtype=torch.int32, device=dev),
+                        dirty_list=torch.zeros(S, dtype=torch.int32, device=dev),
+                        ctl=torch.zeros(4, dtype=torch.int32, device=dev),
+                        seen=torch.zeros(1, dtype=torch.int64, device=dev),
+                        max_priority=torch.ones(1, dtype=torch.float64, device=dev),
+                        n_rejected=torch.zeros(1, dtype=torch.int64, device=dev))
+        self._pr = A.MdgPrioritized(capacity=cap, tree_size=T, alpha=self.alpha,
+                                    **{k_: v.data_ptr() for k_, v in self.per.items()})
+        self._pout = {}
+
+    def add(self, action):
+        """``DeviceReplay.add``, then the new records' leaves enter the trees at ``max_priority ** alpha``."""
+        super().add(action)
+        with torch.cuda.device(self.env.device):
+            check(self._lib.mdg_per_ingest(C.byref(self._pr), C.byref(self._rp), self.N * self.nstep,
+                                           self.env._sptr()))
+
+    def sample(self, n, beta):
+        """``PrioritizedReplayBuffer.sample``: (SARSD of batched tensors, importance weights (n,) float64, 1 for the
+        record of least priority).  ``last_idx`` / ``last_valid`` as for DeviceReplay; ``last_pos`` holds the
+        sampled records' append positions, which ``update_priorities`` uses to skip records overwritten since."""
+        out, b = self._batch_out(n)
+        pout = self._pout.get(n)
+        if pout is None:
+            dev = self.env.device
+            pout = self._pout[n] = dict(weights=torch.empty(n, dtype=torch.float64, device=dev),
+                                        pos=torch.empty(n, dtype=torch.int64, device=dev))
+        self.draws += 1
+        with torch.cuda.device(self.env.device):
+            check(self._lib.mdg_per_sample(
+                C.byref(self._pr), C.byref(self._rp), self.N, self.step_count, self.obs_price.data_ptr(),
+                self.obs_port.data_ptr(), self.k * self.nF, self.n_port,
+                A.DTYPE_F32 if self.dtype == torch.float32 else A.DTYPE_F64, n, float(beta), self.seed, self.draws,
+                C.byref(b), pout["weights"].data_ptr(), pout["pos"].data_ptr(), self.env._sptr()))
+        self.last_pos = pout["pos"]
+        return self._sarsd(out), pout["weights"]
+
+    def update_priorities(self, priorities):
+        """``PrioritizedReplayBuffer.update_priorities`` for the records of the last ``sample``: ``priorities`` is a
+        float32 or float64 tensor of shape (n,).  Rows with idx -1, records overwritten since the sample, and
+        priorities that are not finite or not > 0 are skipped (the last counted in ``n_rejected``); of an index
+        drawn twice the last row wins."""
+        idx = getattr(self, "last_idx", None)
+        if idx is None:
+            raise RuntimeError("update_priorities needs a sample() first")
+        p = priorities if isinstance(priorities, torch.Tensor) else torch.as_tensor(priorities)
+        if p.dtype not in (torch.float32, torch.float64):
+            raise ValueError("priorities must be float32 or float64")
+        if p.shape != idx.shape:
+            raise ValueError(f"priorities must have shape {tuple(idx.shape)}")
+        with self.env._copy_ctx():
+            p = p.to(device=self.env.device, dtype=torch.float64).contiguous()
+        with torch.cuda.device(self.env.device):
+            check(self._lib.mdg_per_update(C.byref(self._pr), idx.numel(), idx.data_ptr(), self.last_pos.data_ptr(),
+                                           p.data_ptr(), self.env._sptr()))
+
+    @property
+    def n_rejected(self):
+        """(1,) int64 device tensor: priorities ``update_priorities`` skipped as not finite or not > 0 (reading it
+        on the host synchronises; keep it on the device inside a training loop)."""
+        return self.per["n_rejected"]
+
+    @property
+    def max_priority(self):
+        """(1,) float64 device tensor: the largest priority applied so far (1 at first)."""
+        return self.per["max_priority"]
