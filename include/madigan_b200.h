@@ -28,7 +28,7 @@
 extern "C" {
 #endif
 
-#define MDG_ABI_VERSION 13
+#define MDG_ABI_VERSION 14
 #define MDG_MAX_ASSETS 16
 #define MDG_GEN_NPARAM 10
 #define MDG_MAX_NSTEP 64
@@ -272,7 +272,7 @@ enum MdgNorm {
 int mdg_abi_version(void);
 /* sizeof of the ABI structs as compiled: 0 MdgAssetGen 1 MdgParams 2 MdgReward 3 MdgState 4 MdgStepIO
  * 5 MdgLaunch 6 MdgDerived 7 MdgWindow 8 MdgReplay 9 MdgReplayBatch 10 MdgRewardNorm 11 MdgTearsheet
- * 12 MdgPrioritized; -1 for an unknown index (lets a binding verify its struct mirror) */
+ * 12 MdgPrioritized 13 MdgReplayRows; -1 for an unknown index (lets a binding verify its struct mirror) */
 int mdg_sizeof(int which);
 const char *mdg_last_error(void);
 
@@ -468,6 +468,61 @@ int mdg_per_sample(const MdgPrioritized *pr, const MdgReplay *rp, int64_t n_envs
  * them, priorities [batch] f64. */
 int mdg_per_update(const MdgPrioritized *pr, int64_t batch, const int64_t *idx, const int64_t *pos,
                    const double *priorities, void *stream);
+
+/* ---------------------------------------------------------------------------------------------------
+ * Replay row store: the observations of MdgReplay kept as raw price rows instead of materialised windows, and the
+ * windows built and normalised at sample time for the sampled records only.
+ *
+ * Storage (device):
+ *   rows       [N][n_rows][n_feats] f64, env-major: a per-env ring of raw price rows.  Rows are counted from 1:
+ *              env e has appended row_count[e] rows, and row c is at position c % n_rows.
+ *   row_count  [N] int64, rows appended per env (monotonic, 0 at first)
+ *   row_end    [depth][N] int64: for observation slot t % depth, row_count[e] right after step t's ingest (0 = never
+ *              written).  The window of that observation is the rows row_end - k + 1 ... row_end, oldest first.
+ *   last_ts    [N] int64, the env's timestamp at its last ingest
+ * Invariant: the k rows that end at row_end[t % depth][e] are bit for bit the raw (k, F) window mdg_materialise_window
+ * (norm NONE, f64, n_valid = k) writes for env e after step t.
+ * Ingest rule (mdg_replay_rows_ingest), per env, with since = timestamp - reset_ts + 1 and the rows read as
+ * mdg_materialise_window reads them (ring rows for ages < since, prefix rows otherwise):
+ *   - whole_window != 0, since == 1 (the env reset at this observation) or timestamp != last_ts + 1: append the whole
+ *     k-row window (a reset's history fill, or whatever the window holds after a fill shorter than k);
+ *   - otherwise append one row, the newest ring row (at `head`).
+ * Timestamps are monotone across resets (reset_ts = timestamp + fill), so the rule covers auto-reset, explicit resets
+ * between the step and the ingest, and fills shorter than k.  An env-step costs one row; a reset k rows.
+ * Residency: a record is drawn only when the test of mdg_replay_sample holds AND its state's rows are still in the
+ * ring:  row_end >= k  and  row_end - k + 1 > row_count - n_rows  (row_end of the state's slot).  The next state's
+ * rows are newer.  Every reset during a record's life costs k - 1 extra rows, so with
+ * n_rows >= depth + (k - 1)(r + 1) no record of an env that reset at most r times in `depth` steps goes stale through
+ * its rows; n_rows < depth + k - 1 is rejected.  The Philox counters and draw loops are those of mdg_replay_sample and
+ * mdg_per_sample, so when no record is stale through its rows both samplers draw the same indices as with stored
+ * windows, and the batches are bit-identical to theirs (the windows are normalised by the same device code as
+ * mdg_materialise_window's).
+ * Deviation (documented), prioritized: a record stale through its rows keeps its leaf's mass until the ring overwrites
+ * it, like a record whose observation slot was overwritten; the weights' total and p_min include it. */
+typedef struct MdgReplayRows {
+  double *rows;         /* [N][n_rows][n_feats] */
+  int64_t *row_end;     /* [depth][N] */
+  int64_t *row_count;   /* [N] */
+  int64_t *last_ts;     /* [N] */
+  int64_t n_rows;       /* rows kept per env */
+  int32_t n_feats;      /* F, the env's assets */
+  int32_t window;       /* k, the env's window */
+} MdgReplayRows;
+
+/* After a step (or for the first observation, with whole_window = 1): the ingest rule above for every env, reading the
+ * env's observation ring through w (ring = obs_price, prefix = pre_price, timestamp, reset_ts, head, window, n_envs,
+ * n_feats, stream; n_valid must equal window), then row_end[slot] = row_count.  slot in [0, depth). */
+int mdg_replay_rows_ingest(const MdgReplayRows *rows, const MdgWindow *w, int64_t slot, int32_t whole_window);
+/* mdg_replay_sample over the row store: windows normalised with norm_type (MDG_NORM_*) and written as out_dtype
+ * (MDG_DTYPE_*), (batch, k, F); the other outputs as mdg_replay_sample. */
+int mdg_replay_sample_rows(const MdgReplay *rp, const MdgReplayRows *rows, int64_t n_envs, int64_t cur_step,
+                           const double *obs_port, int32_t n_port, int32_t norm_type, int32_t out_dtype,
+                           int64_t batch, uint64_t seed, uint64_t draw, const MdgReplayBatch *out, void *stream);
+/* mdg_per_sample over the row store (windows as mdg_replay_sample_rows). */
+int mdg_per_sample_rows(const MdgPrioritized *pr, const MdgReplay *rp, const MdgReplayRows *rows, int64_t n_envs,
+                        int64_t cur_step, const double *obs_port, int32_t n_port, int32_t norm_type,
+                        int32_t out_dtype, int64_t batch, double beta, uint64_t seed, uint64_t draw,
+                        const MdgReplayBatch *out, double *weights, int64_t *pos, void *stream);
 
 /* ---------------------------------------------------------------------------------------------------
  * Streaming reward normalisers (environments/reward_normalization.pyx:14-272): one scalar state machine per env,

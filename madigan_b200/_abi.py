@@ -5,7 +5,7 @@ checks the struct sizes against the compiled library (``mdg_sizeof``).
 """
 import ctypes as C
 
-MDG_ABI_VERSION = 13
+MDG_ABI_VERSION = 14
 FLAG_FORCE_EXACT_GATE = 1
 FLAG_GENERIC_FILL = 2
 XFORM_NONE, XFORM_PAIR_RATIO, XFORM_RETURNS = 0, 1, 2
@@ -117,6 +117,11 @@ class MdgPrioritized(C.Structure):
                [("capacity", C.c_int64), ("tree_size", C.c_int64), ("alpha", C.c_double)]
 
 
+class MdgReplayRows(C.Structure):
+    _fields_ = [(n, _dp) for n in ("rows", "row_end", "row_count", "last_ts")] + \
+               [("n_rows", C.c_int64), ("n_feats", C.c_int32), ("window", C.c_int32)]
+
+
 RN_NULL, RN_SHARPE_FIXED, RN_SORTINO_A, RN_SORTINO_B, RN_SORTINO_C, RN_SHARPE_EWMA = range(6)
 
 
@@ -161,6 +166,13 @@ SYMBOLS = {
                                  C.c_int32, C.c_int32, C.c_int32, C.c_int64, C.c_double, C.c_uint64, C.c_uint64,
                                  _P(MdgReplayBatch), C.c_void_p, C.c_void_p, C.c_void_p]),
     "mdg_per_update": (C.c_int, [_P(MdgPrioritized), C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "mdg_replay_rows_ingest": (C.c_int, [_P(MdgReplayRows), _P(MdgWindow), C.c_int64, C.c_int32]),
+    "mdg_replay_sample_rows": (C.c_int, [_P(MdgReplay), _P(MdgReplayRows), C.c_int64, C.c_int64, C.c_void_p, C.c_int32,
+                                         C.c_int32, C.c_int32, C.c_int64, C.c_uint64, C.c_uint64, _P(MdgReplayBatch),
+                                         C.c_void_p]),
+    "mdg_per_sample_rows": (C.c_int, [_P(MdgPrioritized), _P(MdgReplay), _P(MdgReplayRows), C.c_int64, C.c_int64,
+                                      C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int64, C.c_double, C.c_uint64,
+                                      C.c_uint64, _P(MdgReplayBatch), C.c_void_p, C.c_void_p, C.c_void_p]),
     "mdg_materialise_time": (C.c_int, [C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p]),
     "mdg_episode_stats": (C.c_int, [_P(MdgParams), _P(MdgState), _P(MdgStepIO), _P(MdgLaunch),
                                     C.c_void_p]),
@@ -182,4 +194,4 @@ def bind(lib):
 
 
 STRUCTS = (MdgAssetGen, MdgParams, MdgReward, MdgState, MdgStepIO, MdgLaunch, MdgDerived, MdgWindow, MdgReplay,
-           MdgReplayBatch, MdgRewardNorm, MdgTearsheet, MdgPrioritized)  # mdg_sizeof order
+           MdgReplayBatch, MdgRewardNorm, MdgTearsheet, MdgPrioritized, MdgReplayRows)  # mdg_sizeof order

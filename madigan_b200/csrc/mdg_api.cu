@@ -773,6 +773,7 @@ extern "C" int mdg_sizeof(int which) {
     case 10: return (int)sizeof(MdgRewardNorm);
     case 11: return (int)sizeof(MdgTearsheet);
     case 12: return (int)sizeof(MdgPrioritized);
+    case 13: return (int)sizeof(MdgReplayRows);
   }
   return -1;
 }

@@ -127,8 +127,10 @@ struct DescentArgs {
   double* weights;
 };
 
-// one thread per sample: the proportional descent with rejection, then the importance weight
-__global__ void __launch_bounds__(128, 8) per_descent_kernel(const __grid_constant__ DescentArgs a) {
+// one thread per sample: the proportional descent with rejection (a leaf `resident` refuses is redrawn too), then the
+// importance weight
+template <class Resident>
+__device__ __forceinline__ void per_descend(const DescentArgs& a, Resident resident) {
   const int64_t b = (int64_t)blockIdx.x * 128 + threadIdx.x;
   if (b >= a.batch) return;
   const MdgPrioritized& p = a.pr;
@@ -156,7 +158,7 @@ __global__ void __launch_bounds__(128, 8) per_descent_kernel(const __grid_consta
     }
     const int64_t leaf = node - T;
     if (leaf >= p.capacity || p.leaf_pos[leaf] < 0 || !(p.sum_tree[node] > 0.)) continue;
-    if (replay_resident(a.rp, leaf, a.cur_step)) { pick = leaf; break; }
+    if (resident(leaf)) { pick = leaf; break; }
   }
   a.idx[b] = pick;
   if (pick < 0) {
@@ -169,6 +171,23 @@ __global__ void __launch_bounds__(128, 8) per_descent_kernel(const __grid_consta
   a.weights[b] = pow(p.sum_tree[T + pick] / total * n, -a.beta) / pow(p.min_tree[1] / total * n, -a.beta);
 }
 
+__global__ void __launch_bounds__(128, 8) per_descent_kernel(const __grid_constant__ DescentArgs a) {
+  per_descend(a, [&](long long leaf) { return replay_resident(a.rp, leaf, a.cur_step); });
+}
+
+struct DescentRowsArgs {
+  DescentArgs d;
+  MdgReplayRows rw;
+  int64_t N;
+};
+
+// per_descent_kernel over the row store: a record whose state rows were overwritten is rejected too
+__global__ void __launch_bounds__(128, 8) per_descent_rows_kernel(const __grid_constant__ DescentRowsArgs a) {
+  per_descend(a.d, [&](long long leaf) {
+    return replay_resident(a.d.rp, leaf, a.d.cur_step) && rows_resident(a.d.rp, a.rw, a.N, leaf);
+  });
+}
+
 struct PerGatherArgs {
   MdgReplay rp;
   GatherArgs g;
@@ -178,6 +197,17 @@ struct PerGatherArgs {
 __global__ void __launch_bounds__(kGatherThreads) per_gather_kernel(const __grid_constant__ PerGatherArgs a) {
   const int64_t b = blockIdx.x;
   replay_gather(a.rp, a.g, b, a.g.out.idx[b]);
+}
+
+struct PerGatherRowsArgs {
+  MdgReplay rp;
+  RowsGatherArgs g;
+};
+
+// one block per sample: the rows gather of mdg_replay_sample_rows for the index the descent chose
+__global__ void __launch_bounds__(kGatherThreads) per_gather_rows_kernel(const __grid_constant__ PerGatherRowsArgs a) {
+  const int64_t b = blockIdx.x;
+  replay_gather_rows(a.rp, a.g, b, a.g.out.idx[b]);
 }
 
 struct UpdateArgs {
@@ -291,6 +321,39 @@ extern "C" int mdg_per_sample(const MdgPrioritized* pr, const MdgReplay* rp, int
   g.g.dtype = obs_dtype; g.g.out = *out;
   per_gather_kernel<<<(unsigned)batch, kGatherThreads, 0, st>>>(g);
   return cuda_err(cudaGetLastError(), "mdg_per_sample gather launch");
+}
+
+extern "C" int mdg_per_sample_rows(const MdgPrioritized* pr, const MdgReplay* rp, const MdgReplayRows* rows,
+                                   int64_t n_envs, int64_t cur_step, const double* obs_port, int32_t n_port,
+                                   int32_t norm_type, int32_t out_dtype, int64_t batch, double beta, uint64_t seed,
+                                   uint64_t draw, const MdgReplayBatch* out, double* weights, int64_t* pos,
+                                   void* stream) {
+  int rc = check_per(pr);
+  if (!rc) rc = check_replay(rp);
+  if (!rc) rc = check_rows_sample(rows, rp, obs_port, n_port, norm_type, out_dtype, out);
+  if (rc) return rc;
+  if (rp->capacity != pr->capacity) return set_err(MDG_E_INVALID, "prioritized replay capacity != replay capacity");
+  if (!weights || !pos) return set_err(MDG_E_INVALID, "null weights/pos output");
+  if (!(beta >= 0.)) return set_err(MDG_E_INVALID, "beta must be >= 0");
+  if (batch <= 0) return batch == 0 ? MDG_OK : set_err(MDG_E_INVALID, "batch < 0");
+  const size_t smem = rows_gather_smem(*rows);
+  static size_t smem_allowed = 48 * 1024;
+  rc = rows_gather_smem_attr(per_gather_rows_kernel, smem, &smem_allowed);
+  if (rc) return rc;
+  const cudaStream_t st = (cudaStream_t)stream;
+  DescentRowsArgs d;
+  d.d.pr = *pr; d.d.rp = *rp; d.d.cur_step = cur_step; d.d.batch = batch; d.d.beta = beta; d.d.seed = seed;
+  d.d.draw = draw; d.d.idx = out->idx; d.d.pos = pos; d.d.weights = weights;
+  d.rw = *rows; d.N = n_envs;
+  per_descent_rows_kernel<<<(unsigned)((batch + 127) / 128), 128, 0, st>>>(d);
+  rc = cuda_err(cudaGetLastError(), "mdg_per_sample_rows descent launch");
+  if (rc) return rc;
+  PerGatherRowsArgs g;
+  g.rp = *rp;
+  g.g.N = n_envs; g.g.rw = *rows; g.g.obs_port = obs_port; g.g.n_port = n_port; g.g.dtype = out_dtype;
+  g.g.norm = norm_type; g.g.out = *out;
+  per_gather_rows_kernel<<<(unsigned)batch, kGatherThreads, smem, st>>>(g);
+  return cuda_err(cudaGetLastError(), "mdg_per_sample_rows gather launch");
 }
 
 extern "C" int mdg_per_update(const MdgPrioritized* pr, int64_t batch, const int64_t* idx, const int64_t* pos,

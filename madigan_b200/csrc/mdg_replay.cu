@@ -57,6 +57,25 @@ __global__ void __launch_bounds__(256) replay_append_kernel(const __grid_constan
   }
 }
 
+// Sample b's draw (ReplayBuffer._sample_idxs, replay_buffer.py:107-108: uniform over the filled part), redrawn until
+// `resident` accepts the record, 64 attempts at most (-1: none found).
+template <class Resident>
+__device__ __forceinline__ long long replay_draw(const MdgReplay& r, int64_t b, uint64_t seed, uint64_t draw,
+                                                 Resident resident) {
+  const unsigned long long cur = *r.cursor;
+  const unsigned long long filled = cur < (unsigned long long)r.capacity ? cur : (unsigned long long)r.capacity;
+  long long pick = -1;
+  for (uint32_t attempt = 0; attempt < 64 && filled > 0; ++attempt) {
+    uint64_t x0, x1;
+    philox4x32_10((uint32_t)b, (uint32_t)(b >> 32) ^ (attempt << 8), (uint32_t)draw, (uint32_t)(draw >> 32),
+                  (uint32_t)seed, (uint32_t)(seed >> 32), x0, x1);
+    const unsigned long long j = (unsigned long long)(((x0 >> 11) * 0x1.0p-53) * (double)filled);
+    const long long cand = (long long)(j < filled ? j : filled - 1);
+    if (resident(cand)) { pick = cand; break; }
+  }
+  return pick;
+}
+
 struct SampleArgs {
   MdgReplay rp;
   int64_t cur_step, batch;
@@ -70,24 +89,119 @@ __global__ void __launch_bounds__(kGatherThreads) replay_sample_kernel(const __g
   __shared__ long long s_idx;
   const MdgReplay& r = a.rp;
   const int64_t b = blockIdx.x;
-  if (threadIdx.x == 0) {
-    const unsigned long long cur = *r.cursor;
-    const unsigned long long filled = cur < (unsigned long long)r.capacity ? cur : (unsigned long long)r.capacity;
-    long long pick = -1;
-    for (uint32_t attempt = 0; attempt < 64 && filled > 0; ++attempt) {
-      uint64_t x0, x1;
-      philox4x32_10((uint32_t)b, (uint32_t)(b >> 32) ^ (attempt << 8), (uint32_t)a.draw, (uint32_t)(a.draw >> 32),
-                    (uint32_t)a.seed, (uint32_t)(a.seed >> 32), x0, x1);
-      const unsigned long long j = (unsigned long long)(((x0 >> 11) * 0x1.0p-53) * (double)filled);
-      const long long cand = (long long)(j < filled ? j : filled - 1);
-      if (replay_resident(r, cand, a.cur_step)) { pick = cand; break; }
-    }
-    s_idx = pick;
-  }
+  if (threadIdx.x == 0)
+    s_idx = replay_draw(r, b, a.seed, a.draw, [&](long long c) { return replay_resident(r, c, a.cur_step); });
   __syncthreads();
   const long long idx = s_idx;
   if (threadIdx.x == 0) a.g.out.idx[b] = idx;
   replay_gather(r, a.g, b, idx);
+}
+
+struct RowsIngestArgs {
+  MdgReplayRows rw;
+  const double* ring;        // [k][F][N] obs_price
+  const double* prefix;      // [N][k][F] pre_price
+  const int64_t* timestamp;  // [N]
+  const int64_t* reset_ts;   // [N]
+  int64_t N, slot;
+  int head, whole;
+};
+
+constexpr int kIngestEnvs = 64;  // envs per block of the rows ingest (256 threads)
+
+// The ingest rule (include/madigan_b200.h, "Replay row store") for kIngestEnvs envs per block: one thread per env
+// decides and counts; the newest ring rows are read coalesced over envs into shared memory and written back as one
+// contiguous run of F doubles per env (per-thread row writes, 32 KB apart at the bench shape, were far slower); each
+// env that appends its whole window is copied by one warp.  The window's rows are read as window_kernel (mdg_aux.cu)
+// reads them: ring rows for ages < since, prefix rows otherwise.
+__global__ void __launch_bounds__(256) replay_rows_ingest_kernel(const __grid_constant__ RowsIngestArgs a) {
+  __shared__ double s_row[kIngestEnvs][65];  // newest ring row per env (F <= 64), padded
+  __shared__ long long s_pos[kIngestEnvs];  // ring position of the first row the env appends
+  __shared__ int s_since[kIngestEnvs], s_whole[kIngestEnvs];
+  const MdgReplayRows& w = a.rw;
+  const int t = threadIdx.x, k = w.window, F = w.n_feats;
+  const int64_t R = w.n_rows, e0 = (int64_t)blockIdx.x * kIngestEnvs;
+  const int ne = (int)(a.N - e0 < kIngestEnvs ? a.N - e0 : kIngestEnvs);
+  if (t < ne) {
+    const int64_t e = e0 + t;
+    const int64_t ts = a.timestamp[e];
+    const long long since = ts - a.reset_ts[e] + 1;  // ring rows written since the last reset
+    const bool whole = a.whole || since == 1 || ts != w.last_ts[e] + 1;
+    const long long cnt = w.row_count[e], added = whole ? k : 1;
+    s_pos[t] = (cnt + 1) % R;
+    s_since[t] = since > k ? k : (int)since;
+    s_whole[t] = whole;
+    w.row_count[e] = cnt + added;
+    w.row_end[a.slot * a.N + e] = cnt + added;
+    w.last_ts[e] = ts;
+  }
+  for (int i = t; i < kIngestEnvs * F; i += 256) {
+    const int el = i % kIngestEnvs, f = i / kIngestEnvs;
+    if (el < ne) s_row[el][f] = a.ring[((int64_t)a.head * F + f) * a.N + e0 + el];
+  }
+  __syncthreads();
+  for (int i = t; i < ne * F; i += 256) {
+    const int el = i / F, f = i - el * F;
+    if (!s_whole[el]) w.rows[((e0 + el) * R + s_pos[el]) * F + f] = s_row[el][f];
+  }
+  // whole windows: U independent loads in flight per lane (one load per iteration left each copy latency-bound)
+  const int lane = t & 31;
+  for (int el = t >> 5; el < ne; el += 256 / 32) {
+    if (!s_whole[el]) continue;
+    const int64_t e = e0 + el, p0 = s_pos[el];
+    const int is = s_since[el];
+    double* dst = w.rows + e * R * F;
+    const double* rb = a.ring + e;
+    const double* pb = a.prefix + (e * k + (k - 2 + is)) * F;  // prefix row of age `age`: (k - 2 + since) - age
+    constexpr int U = 8;
+    for (int i0 = lane; i0 < k * F; i0 += 32 * U) {
+      double v[U];
+      int64_t o[U];
+#pragma unroll
+      for (int u = 0; u < U; ++u) {
+        const int i = i0 + 32 * u;
+        o[u] = -1;
+        v[u] = 0.;
+        if (i < k * F) {
+          const int s = i / F, f = i - s * F;
+          const int age = k - 1 - s;
+          int slot = a.head - age;
+          if (slot < 0) slot += k;
+          v[u] = age < is ? rb[((int64_t)slot * F + f) * a.N] : pb[f - (int64_t)age * F];
+          int64_t p = p0 + s;  // k <= R: one wrap at most
+          if (p >= R) p -= R;
+          o[u] = p * F + f;
+        }
+      }
+#pragma unroll
+      for (int u = 0; u < U; ++u)
+        if (o[u] >= 0) dst[o[u]] = v[u];
+    }
+  }
+}
+
+struct SampleRowsArgs {
+  MdgReplay rp;
+  int64_t cur_step;
+  uint64_t seed, draw;
+  RowsGatherArgs g;
+};
+
+// replay_sample_kernel over the row store: the same draws, with the row store's residency test added
+__global__ void __launch_bounds__(kGatherThreads) replay_sample_rows_kernel(const __grid_constant__ SampleRowsArgs a) {
+  __shared__ long long s_idx;
+  const MdgReplay& r = a.rp;
+  const int64_t b = blockIdx.x;
+  if (threadIdx.x == 0) {
+    const int64_t cur = a.cur_step, N = a.g.N;
+    s_idx = replay_draw(r, b, a.seed, a.draw, [&](long long c) {
+      return replay_resident(r, c, cur) && rows_resident(r, a.g.rw, N, c);
+    });
+  }
+  __syncthreads();
+  const long long idx = s_idx;
+  if (threadIdx.x == 0) a.g.out.idx[b] = idx;
+  replay_gather_rows(r, a.g, b, idx);
 }
 
 }  // namespace mdg
@@ -125,4 +239,43 @@ extern "C" int mdg_replay_sample(const MdgReplay* rp, int64_t n_envs, int64_t cu
   a.g.dtype = obs_dtype; a.g.out = *out;
   replay_sample_kernel<<<(unsigned)batch, kGatherThreads, 0, (cudaStream_t)stream>>>(a);
   return cuda_err(cudaGetLastError(), "mdg_replay_sample launch");
+}
+
+extern "C" int mdg_replay_rows_ingest(const MdgReplayRows* rows, const MdgWindow* w, int64_t slot,
+                                      int32_t whole_window) {
+  int rc = check_rows(rows, 1);
+  if (rc) return rc;
+  if (!w || !w->ring || !w->prefix || !w->timestamp || !w->reset_ts)
+    return set_err(MDG_E_INVALID, "null window ring/prefix/timestamp/reset_ts");
+  if (w->n_feats != rows->n_feats || w->window != rows->window)
+    return set_err(MDG_E_INVALID, "window shape != replay rows shape");
+  if (w->n_valid != w->window) return set_err(MDG_E_INVALID, "replay rows need a full window (n_valid == window)");
+  if (w->head < 0 || w->head >= w->window) return set_err(MDG_E_INVALID, "bad head");
+  if (slot < 0) return set_err(MDG_E_INVALID, "negative slot");
+  if (w->n_envs <= 0) return w->n_envs == 0 ? MDG_OK : set_err(MDG_E_INVALID, "n_envs < 0");
+  RowsIngestArgs a;
+  a.rw = *rows; a.ring = w->ring; a.prefix = w->prefix; a.timestamp = w->timestamp; a.reset_ts = w->reset_ts;
+  a.N = w->n_envs; a.slot = slot; a.head = w->head; a.whole = whole_window != 0;
+  replay_rows_ingest_kernel<<<(unsigned)((a.N + kIngestEnvs - 1) / kIngestEnvs), 256, 0, (cudaStream_t)w->stream>>>(a);
+  return cuda_err(cudaGetLastError(), "mdg_replay_rows_ingest launch");
+}
+
+extern "C" int mdg_replay_sample_rows(const MdgReplay* rp, const MdgReplayRows* rows, int64_t n_envs, int64_t cur_step,
+                                      const double* obs_port, int32_t n_port, int32_t norm_type, int32_t out_dtype,
+                                      int64_t batch, uint64_t seed, uint64_t draw, const MdgReplayBatch* out,
+                                      void* stream) {
+  int rc = check_replay(rp);
+  if (!rc) rc = check_rows_sample(rows, rp, obs_port, n_port, norm_type, out_dtype, out);
+  if (rc) return rc;
+  if (batch <= 0) return batch == 0 ? MDG_OK : set_err(MDG_E_INVALID, "batch < 0");
+  const size_t smem = rows_gather_smem(*rows);
+  static size_t smem_allowed = 48 * 1024;
+  rc = rows_gather_smem_attr(replay_sample_rows_kernel, smem, &smem_allowed);
+  if (rc) return rc;
+  SampleRowsArgs a;
+  a.rp = *rp; a.cur_step = cur_step; a.seed = seed; a.draw = draw;
+  a.g.N = n_envs; a.g.rw = *rows; a.g.obs_port = obs_port; a.g.n_port = n_port; a.g.dtype = out_dtype;
+  a.g.norm = norm_type; a.g.out = *out;
+  replay_sample_rows_kernel<<<(unsigned)batch, kGatherThreads, smem, (cudaStream_t)stream>>>(a);
+  return cuda_err(cudaGetLastError(), "mdg_replay_sample_rows launch");
 }

@@ -8,7 +8,12 @@ DSR/DDR/... shaping) were already produced by the step kernel (``env.shaped_rewa
 Observations are stored once per step (slot ``t % depth``): the price window the agents' nets consume
 (``(N, k, nF)``, normalised, fp32 by default) and the newest portfolio row -- the agents read ``portfolio[:, -1]`` only
 (dqn.py:188-199).  See include/madigan_b200.h for the record layout and the one documented deviation (the
-next_state of a terminal transition)."""
+next_state of a terminal transition).
+
+``store="rows"`` keeps the price observations as raw rows instead: one new row per env-step (k rows when the env
+reset) in a per-env row ring, and the windows of the sampled records are built and normalised at sample time
+(include/madigan_b200.h, "Replay row store").  That writes ~272 B per env-step instead of ~4.2 KB (16 assets, k 64,
+fp32), so the ingest is cheap and a deep replay fits on the device; a sample reads and normalises the raw rows."""
 import ctypes as C
 
 import torch
@@ -19,9 +24,14 @@ from .data import SARSD, State
 
 
 class DeviceReplay:
-    def __init__(self, env, depth=64, capacity=None, n_action=None, norm_type=None, dtype=torch.float32, seed=0):
+    def __init__(self, env, depth=64, capacity=None, n_action=None, norm_type=None, dtype=torch.float32, seed=0,
+                 store="windows", rows=None):
         """``depth``: observation slots (steps of history kept); ``capacity``: transitions in the ring (default
-        N * (depth - nstep - 1), so that a stored transition's state is normally still resident)."""
+        N * (depth - nstep - 1), so that a stored transition's state is normally still resident).
+        ``store``: ``"windows"`` stores each step's normalised windows (``obs_price``); ``"rows"`` stores raw price
+        rows (``rows``, ``row_end``, ``row_count``, ``last_ts``; ``obs_price`` is None) and normalises the sampled
+        windows at sample time.  ``rows``: rows kept per env by the row store, at least ``depth + k - 1``; the default
+        ``depth + 3 (k - 1)`` keeps every record of an env that reset at most twice in ``depth`` steps."""
         self.env, self._lib = env, lib()
         N, k, nA = env.N, env.k, env.nA
         self.N, self.k, self.nF, self.n_port = N, k, nA, nA + 1
@@ -37,9 +47,27 @@ class DeviceReplay:
             raise ValueError(f"capacity {self.capacity} exceeds N * (depth - nstep - 1) = {cap_max}")
         self.n_action = int(n_action) if n_action else nA
         self.norm_type, self.dtype, self.seed = norm_type, dtype, int(seed)
+        if store not in ("windows", "rows"):
+            raise ValueError(f"store must be 'windows' or 'rows', not {store!r}")
+        self.store = store
         dev = env.device
         z = lambda *s, dt: torch.zeros(s, dtype=dt, device=dev)
-        self.obs_price = torch.empty((self.depth, N, k, nA), dtype=dtype, device=dev)
+        if store == "windows":
+            self.obs_price = torch.empty((self.depth, N, k, nA), dtype=dtype, device=dev)
+        else:
+            from .preprocessor import NORM_TYPES
+            self._norm = NORM_TYPES[norm_type]
+            self.n_rows = int(rows) if rows is not None else self.depth + 3 * (k - 1)
+            if self.n_rows < self.depth + k - 1:
+                raise ValueError(f"rows {self.n_rows} < depth + k - 1 = {self.depth + k - 1}")
+            self.obs_price = None
+            self.rows = torch.zeros((N, self.n_rows, nA), dtype=torch.float64, device=dev)
+            self.row_end = z(self.depth, N, dt=torch.int64)
+            self.row_count = z(N, dt=torch.int64)
+            self.last_ts = z(N, dt=torch.int64)
+            self._rr = A.MdgReplayRows(rows=self.rows.data_ptr(), row_end=self.row_end.data_ptr(),
+                                       row_count=self.row_count.data_ptr(), last_ts=self.last_ts.data_ptr(),
+                                       n_rows=self.n_rows, n_feats=nA, window=k)
         self.obs_port = torch.empty((self.depth, N, nA + 1), dtype=torch.float64, device=dev)
         self.t = dict(t_env=z(self.capacity, dt=torch.int32), t_state_slot=z(self.capacity, dt=torch.int32),
                       t_next_slot=z(self.capacity, dt=torch.int32),
@@ -54,22 +82,32 @@ class DeviceReplay:
         self.draws = 0
 
     # ------------------------------------------------------------------ ingest
-    def _store_obs(self, step):
+    def _store_obs(self, step, whole_window=False):
         slot = step % self.depth
-        self.env.window(self.norm_type, dtype=self.dtype, out=self.obs_price[slot])
-        self.obs_port[slot].copy_(self.env.t["obs_port"][self.env.head].t())
+        env = self.env
+        if self.obs_price is not None:
+            env.window(self.norm_type, dtype=self.dtype, out=self.obs_price[slot])
+        else:
+            if env.n_valid < self.k:
+                raise ValueError(f"the row store needs a full window: env.n_valid {env.n_valid} < k {self.k}")
+            T = env.t
+            w = A.MdgWindow(ring=T["obs_price"].data_ptr(), prefix=T["pre_price"].data_ptr(),
+                            timestamp=T["timestamp"].data_ptr(), reset_ts=T["reset_ts"].data_ptr(), n_envs=self.N,
+                            n_feats=self.nF, window=self.k, head=env.head, n_valid=env.n_valid, stream=env._sptr())
+            with torch.cuda.device(env.device):
+                check(self._lib.mdg_replay_rows_ingest(C.byref(self._rr), C.byref(w), slot, int(whole_window)))
+        self.obs_port[slot].copy_(env.t["obs_port"][env.head].t())
 
     def observe_start(self):
         """Store the observation the first action is taken from (after ``env.reset(fill_history=True)``)."""
         with self.env._copy_ctx():
-            self._store_obs(self.step_count)
+            self._store_obs(self.step_count, whole_window=True)
 
     def add(self, action):
         """Call after ``env.step(..., auto_reset=True)`` / ``env.step_actions(...)`` with the action that was taken
         ((N, n_action), any real dtype): stores the new observation and appends the transitions that step popped."""
         env = self.env
-        self.step_count += 1
-        t = self.step_count
+        t = self.step_count + 1
         a = action if (isinstance(action, torch.Tensor) and action.dtype == torch.float64 and action.is_cuda
                        and action.is_contiguous()) else \
             torch.as_tensor(action).to(device=env.device, dtype=torch.float64).contiguous()
@@ -77,6 +115,7 @@ class DeviceReplay:
             raise ValueError(f"action must have shape {(self.N, self.n_action)}")
         with env._copy_ctx():
             self._store_obs(t)
+        self.step_count = t
         T = env.t
         with torch.cuda.device(env.device):
             check(self._lib.mdg_replay_append(
@@ -118,11 +157,16 @@ class DeviceReplay:
         unless the ring is nearly empty or mostly stale)."""
         out, b = self._batch_out(n)
         self.draws += 1
+        dt = A.DTYPE_F32 if self.dtype == torch.float32 else A.DTYPE_F64
         with torch.cuda.device(self.env.device):
-            check(self._lib.mdg_replay_sample(
-                C.byref(self._rp), self.N, self.step_count, self.obs_price.data_ptr(), self.obs_port.data_ptr(),
-                self.k * self.nF, self.n_port, A.DTYPE_F32 if self.dtype == torch.float32 else A.DTYPE_F64, n,
-                self.seed, self.draws, C.byref(b), self.env._sptr()))
+            if self.obs_price is not None:
+                check(self._lib.mdg_replay_sample(
+                    C.byref(self._rp), self.N, self.step_count, self.obs_price.data_ptr(), self.obs_port.data_ptr(),
+                    self.k * self.nF, self.n_port, dt, n, self.seed, self.draws, C.byref(b), self.env._sptr()))
+            else:
+                check(self._lib.mdg_replay_sample_rows(
+                    C.byref(self._rp), C.byref(self._rr), self.N, self.step_count, self.obs_port.data_ptr(),
+                    self.n_port, self._norm, dt, n, self.seed, self.draws, C.byref(b), self.env._sptr()))
         return self._sarsd(out), None
 
 
@@ -138,9 +182,9 @@ class DevicePrioritizedReplay(DeviceReplay):
     records count in the weights' normalisers): include/madigan_b200.h, "Proportional prioritized replay"."""
 
     def __init__(self, env, alpha=0.6, depth=64, capacity=None, n_action=None, norm_type=None, dtype=torch.float32,
-                 seed=0):
+                 seed=0, store="windows", rows=None):
         super().__init__(env, depth=depth, capacity=capacity, n_action=n_action, norm_type=norm_type, dtype=dtype,
-                         seed=seed)
+                         seed=seed, store=store, rows=rows)
         self.alpha = float(alpha)
         if not self.alpha >= 0:
             raise ValueError("alpha must be >= 0")
@@ -181,12 +225,18 @@ class DevicePrioritizedReplay(DeviceReplay):
             pout = self._pout[n] = dict(weights=torch.empty(n, dtype=torch.float64, device=dev),
                                         pos=torch.empty(n, dtype=torch.int64, device=dev))
         self.draws += 1
+        dt = A.DTYPE_F32 if self.dtype == torch.float32 else A.DTYPE_F64
         with torch.cuda.device(self.env.device):
-            check(self._lib.mdg_per_sample(
-                C.byref(self._pr), C.byref(self._rp), self.N, self.step_count, self.obs_price.data_ptr(),
-                self.obs_port.data_ptr(), self.k * self.nF, self.n_port,
-                A.DTYPE_F32 if self.dtype == torch.float32 else A.DTYPE_F64, n, float(beta), self.seed, self.draws,
-                C.byref(b), pout["weights"].data_ptr(), pout["pos"].data_ptr(), self.env._sptr()))
+            if self.obs_price is not None:
+                check(self._lib.mdg_per_sample(
+                    C.byref(self._pr), C.byref(self._rp), self.N, self.step_count, self.obs_price.data_ptr(),
+                    self.obs_port.data_ptr(), self.k * self.nF, self.n_port, dt, n, float(beta), self.seed,
+                    self.draws, C.byref(b), pout["weights"].data_ptr(), pout["pos"].data_ptr(), self.env._sptr()))
+            else:
+                check(self._lib.mdg_per_sample_rows(
+                    C.byref(self._pr), C.byref(self._rp), C.byref(self._rr), self.N, self.step_count,
+                    self.obs_port.data_ptr(), self.n_port, self._norm, dt, n, float(beta), self.seed, self.draws,
+                    C.byref(b), pout["weights"].data_ptr(), pout["pos"].data_ptr(), self.env._sptr()))
         self.last_pos = pout["pos"]
         return self._sarsd(out), pout["weights"]
 
