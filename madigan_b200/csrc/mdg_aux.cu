@@ -169,7 +169,8 @@ __global__ void window_kernel(const __grid_constant__ WindowArgs a) {
   {
     const int Z = blockDim.z, z = threadIdx.z;
     double* cpar = tile + (int64_t)a.envs * a.estride + ((int64_t)el * F + f) * 2;  // (shift, scale) per column
-    normalise_windows(a, tile, col, cpar, nv, Fe, e0, live && f < Fe, z, Z);
+    // a window written as a column block of a wider output is normalised as part of that (k, Ftot) array
+    normalise_windows(a, tile, col, cpar, nv, Fe, Fe == 1 && a.Ftot == a.Fout, e0, live && f < Fe, z, Z);
   }
   __syncthreads();
 

@@ -144,7 +144,8 @@ static __device__ __noinline__ void replay_gather_rows(const MdgReplay& r, const
   {
     const int t = threadIdx.x, f = t % F, el = (t / F) & 1, z = t / (2 * F), Z = NT / (2 * F);
     struct { int norm, sstride, estride, envs; int64_t N; } tl = {a.norm, F, W, 2, 2};  // two windows, both real
-    normalise_windows(tl, rtile, rtile + el * W + f, rtile + 2 * W + (el * F + f) * 2, k, F, 0, z < Z, z, Z);
+    normalise_windows(tl, rtile, rtile + el * W + f, rtile + 2 * W + (el * F + f) * 2, k, F, F == 1, 0, z < Z, z,
+                      Z);
   }
   __syncthreads();
   const int64_t o_b = b * W;
