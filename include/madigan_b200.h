@@ -28,7 +28,7 @@
 extern "C" {
 #endif
 
-#define MDG_ABI_VERSION 14
+#define MDG_ABI_VERSION 15
 #define MDG_MAX_ASSETS 16
 #define MDG_GEN_NPARAM 10
 #define MDG_MAX_NSTEP 64
@@ -272,7 +272,8 @@ enum MdgNorm {
 int mdg_abi_version(void);
 /* sizeof of the ABI structs as compiled: 0 MdgAssetGen 1 MdgParams 2 MdgReward 3 MdgState 4 MdgStepIO
  * 5 MdgLaunch 6 MdgDerived 7 MdgWindow 8 MdgReplay 9 MdgReplayBatch 10 MdgRewardNorm 11 MdgTearsheet
- * 12 MdgPrioritized 13 MdgReplayRows; -1 for an unknown index (lets a binding verify its struct mirror) */
+ * 12 MdgPrioritized 13 MdgReplayRows 14 MdgParamSets; -1 for an unknown index (lets a binding verify its struct
+ * mirror) */
 int mdg_sizeof(int which);
 const char *mdg_last_error(void);
 
@@ -316,6 +317,44 @@ int mdg_step_autoreset(const MdgParams *params, const MdgReward *reward, const M
  * empty ledger, cash=init_cash, timestamp=0, shaper state zero. */
 int mdg_init_state(const MdgParams *params, const MdgReward *reward, const MdgState *state,
                    const MdgLaunch *launch);
+
+/* ---------------------------------------------------------------------------------------------------
+ * Generator parameter sets: the envs of one slab tick different markets (a sweep over settings, or a distribution of
+ * markets for robust training) with the same types, roles, slots and broker settings.
+ *
+ * A parameter set is one value for every p[j] slot (MDG_GEN_NPARAM) of every asset.  The table holds n_sets >= 1 of
+ * them, set-minor: p[(i * MDG_GEN_NPARAM + j) * n_sets + s] is slot j of asset i in set s, so that a warp's reads
+ * are coalesced when every env has its own set (n_sets == n_envs, set_of_env[e] == e) and stay on one 128-byte line
+ * when n_sets <= 16.  Env e reads set s = set_of_env[e]; an index outside [0, n_sets) is clamped, as an unsigned
+ * value, to n_sets - 1, so no index reads outside the table.
+ * With sets, every read of params->gen[i].p[j] by the step, refill and constructor kernels reads the table entry of
+ * the env's set instead.  Nothing else changes: types, roles, noise / uniform slots, gslot, broker settings, rewards
+ * and the Philox draws (keyed on seed, global env id and tick only).  So env e of a launch with sets is bit for bit
+ * env e of a launch without sets whose params->gen[i].p are those of set s.  OUPair reads as without sets: role 0
+ * supplies p[2] (the shared mean's noise), each asset its own p[0] (theta) and p[1] (phi).
+ * The SINE* types are not accepted (their p slots are component counts and offsets into gen_ext):
+ * MDG_E_UNSUPPORTED.  params->gen[i].p must still be filled (the base set: the host-side checks read it).
+ * The table and the assignment are read by each launch on its stream: a change made between launches takes effect at
+ * the next launch, and an episode in progress continues under the new values. */
+typedef struct MdgParamSets {
+  const double *p;           /* device: [nA][MDG_GEN_NPARAM][n_sets], set-minor */
+  const int32_t *set_of_env; /* device: [N] */
+  int32_t n_sets, _pad;
+} MdgParamSets;
+
+/* mdg_step, mdg_step_autoreset, mdg_reset_ws and mdg_init_state with parameter sets.  NULL sets or n_sets < 1:
+ * MDG_E_INVALID; a SINE* asset: MDG_E_UNSUPPORTED.  mdg_reset_ws_sets requires a workspace (NULL: MDG_E_INVALID).
+ * The step kernel of these launches always runs in 128-thread blocks. */
+int mdg_step_sets(const MdgParams *params, const MdgReward *reward, const MdgState *state, const MdgStepIO *io,
+                  const MdgLaunch *launch, const MdgParamSets *sets);
+int mdg_step_autoreset_sets(const MdgParams *params, const MdgReward *reward, const MdgState *state,
+                            const MdgStepIO *io, const MdgLaunch *launch, int fill_ticks, int clear_nstep,
+                            void *workspace, int64_t workspace_bytes, const MdgParamSets *sets);
+int mdg_reset_ws_sets(const MdgParams *params, const MdgState *state, const MdgStepIO *io, const MdgLaunch *launch,
+                      const uint8_t *mask, int fill_ticks, int clear_nstep, void *workspace, int64_t workspace_bytes,
+                      const MdgParamSets *sets);
+int mdg_init_state_sets(const MdgParams *params, const MdgReward *reward, const MdgState *state,
+                        const MdgLaunch *launch, const MdgParamSets *sets);
 
 /* Recompute MdgState.folds from the state tensors (after external writes into them). */
 int mdg_refresh_folds(const MdgParams *params, const MdgState *state, const MdgLaunch *launch);

@@ -5,7 +5,7 @@ checks the struct sizes against the compiled library (``mdg_sizeof``).
 """
 import ctypes as C
 
-MDG_ABI_VERSION = 14
+MDG_ABI_VERSION = 15
 FLAG_FORCE_EXACT_GATE = 1
 FLAG_GENERIC_FILL = 2
 XFORM_NONE, XFORM_PAIR_RATIO, XFORM_RETURNS = 0, 1, 2
@@ -122,6 +122,10 @@ class MdgReplayRows(C.Structure):
                [("n_rows", C.c_int64), ("n_feats", C.c_int32), ("window", C.c_int32)]
 
 
+class MdgParamSets(C.Structure):
+    _fields_ = [("p", _dp), ("set_of_env", _dp), ("n_sets", C.c_int32), ("_pad", C.c_int32)]
+
+
 RN_NULL, RN_SHARPE_FIXED, RN_SORTINO_A, RN_SORTINO_B, RN_SORTINO_C, RN_SHARPE_EWMA = range(6)
 
 
@@ -154,6 +158,13 @@ SYMBOLS = {
     "mdg_step_autoreset": (C.c_int, [_P(MdgParams), _P(MdgReward), _P(MdgState), _P(MdgStepIO), _P(MdgLaunch),
                                      C.c_int, C.c_int, C.c_void_p, C.c_int64]),
     "mdg_init_state": (C.c_int, [_P(MdgParams), _P(MdgReward), _P(MdgState), _P(MdgLaunch)]),
+    "mdg_step_sets": (C.c_int, [_P(MdgParams), _P(MdgReward), _P(MdgState), _P(MdgStepIO), _P(MdgLaunch),
+                                _P(MdgParamSets)]),
+    "mdg_step_autoreset_sets": (C.c_int, [_P(MdgParams), _P(MdgReward), _P(MdgState), _P(MdgStepIO), _P(MdgLaunch),
+                                          C.c_int, C.c_int, C.c_void_p, C.c_int64, _P(MdgParamSets)]),
+    "mdg_reset_ws_sets": (C.c_int, [_P(MdgParams), _P(MdgState), _P(MdgStepIO), _P(MdgLaunch), C.c_void_p,
+                                    C.c_int, C.c_int, C.c_void_p, C.c_int64, _P(MdgParamSets)]),
+    "mdg_init_state_sets": (C.c_int, [_P(MdgParams), _P(MdgReward), _P(MdgState), _P(MdgLaunch), _P(MdgParamSets)]),
     "mdg_refresh_folds": (C.c_int, [_P(MdgParams), _P(MdgState), _P(MdgLaunch)]),
     "mdg_derived": (C.c_int, [_P(MdgParams), _P(MdgState), _P(MdgDerived), _P(MdgLaunch)]),
     "mdg_materialise_window": (C.c_int, [_P(MdgWindow)]),
@@ -194,4 +205,4 @@ def bind(lib):
 
 
 STRUCTS = (MdgAssetGen, MdgParams, MdgReward, MdgState, MdgStepIO, MdgLaunch, MdgDerived, MdgWindow, MdgReplay,
-           MdgReplayBatch, MdgRewardNorm, MdgTearsheet, MdgPrioritized, MdgReplayRows)  # mdg_sizeof order
+           MdgReplayBatch, MdgRewardNorm, MdgTearsheet, MdgPrioritized, MdgReplayRows, MdgParamSets)  # mdg_sizeof order

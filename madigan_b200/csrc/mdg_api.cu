@@ -165,6 +165,11 @@ struct ResetWsArgs {
   int8_t group_of_thread[128];
 };
 
+// the refills of the launches with parameter sets: the table and the assignment after everything the others read
+struct ResetWsSetsArgs : ResetWsArgs {
+  MdgParamSets ps;
+};
+
 __global__ void __launch_bounds__(256) reset_scan_kernel(const __grid_constant__ ResetWsArgs a) {
   const int64_t N = a.L.n_envs;
   const int64_t e = (int64_t)blockIdx.x * 256 + threadIdx.x;
@@ -180,7 +185,8 @@ __global__ void __launch_bounds__(256) reset_scan_kernel(const __grid_constant__
 
 constexpr int kFillBlock = 128;
 
-__global__ void __launch_bounds__(kFillBlock) reset_fill_kernel(const __grid_constant__ ResetWsArgs a) {
+template <bool SETS>
+__device__ __forceinline__ void reset_fill_body(const ResetWsArgs& a) {
   extern __shared__ double zs[];  // [chunk][n_normals]
   const MdgParams& P = a.P;
   const int tid = threadIdx.x;
@@ -196,6 +202,8 @@ __global__ void __launch_bounds__(kFillBlock) reset_fill_kernel(const __grid_con
   for (int d = blockIdx.x; d < count; d += gridDim.x) {
     const int64_t e = a.list[d];
     const long long ts0 = a.S.timestamp[e];
+    int64_t set = 0;  // parameter sets: the listed env's set
+    if constexpr (SETS) set = env_set(static_cast<const ResetWsSetsArgs&>(a).ps, e);
     __syncthreads();  // every thread has read the old timestamp (and the previous env's normals are consumed)
     if (tid == 32) {  // fresh Broker/Account/Portfolio (Env.h:150-165): per-env scalars
       if (a.clear_nstep && a.S.nstep_len) a.S.nstep_len[e] = 0;  // offpolicy_q.py:94
@@ -228,8 +236,12 @@ __global__ void __launch_bounds__(kFillBlock) reset_fill_kernel(const __grid_con
       for (int c = 0; c < cnt; ++c) pr[c] = a.S.price[(int64_t)(i0 + c) * N + e];
       for (int c = 0; c < cnt; ++c) {  // dataSource_->reset() and the empty ledger
         const CtorDraws cd = ctor_draws((uint32_t)(a.L.env_offset + e), a.L.seed, ts0, 2, i0 + c);
-        pr[c] = big ? gen_reset(P.gen[i0 + c], pr[c], gsg, N, P.gen_ext, &cd)
-                    : gen_reset(P.gen[i0 + c], pr[c], gsl, 1, P.gen_ext, &cd);
+        if constexpr (SETS)  // no SINE* source here: the state is in registers
+          pr[c] = gen_reset_p(P.gen[i0 + c], set_params(static_cast<const ResetWsSetsArgs&>(a).ps, set, i0 + c), pr[c],
+                              gsl, 1, P.gen_ext, &cd);
+        else
+          pr[c] = big ? gen_reset(P.gen[i0 + c], pr[c], gsg, N, P.gen_ext, &cd)
+                      : gen_reset(P.gen[i0 + c], pr[c], gsl, 1, P.gen_ext, &cd);
         a.S.ledger[(int64_t)(i0 + c) * N + e] = 0.;
         a.S.mean_entry[(int64_t)(i0 + c) * N + e] = 0.;
         a.S.borrowed[(int64_t)(i0 + c) * N + e] = 0.;
@@ -263,7 +275,12 @@ __global__ void __launch_bounds__(kFillBlock) reset_fill_kernel(const __grid_con
       if (worker) {
         if (is_pair) {  // OUPair::getData (DataSource.cpp:1232-1240) inlined
           const MdgAssetGen& g1 = P.gen[i0 + 1];
-          const double theta0 = g0.p[0], phi0 = g0.p[1], noise = g0.p[2], theta1 = g1.p[0], phi1 = g1.p[1];
+          double theta0 = g0.p[0], phi0 = g0.p[1], noise = g0.p[2], theta1 = g1.p[0], phi1 = g1.p[1];
+          if constexpr (SETS) {
+            const MdgParamSets& ps = static_cast<const ResetWsSetsArgs&>(a).ps;
+            const SetParams q0 = set_params(ps, set, i0), q1 = set_params(ps, set, i0 + 1);
+            theta0 = q0[0]; phi0 = q0[1]; noise = q0[2]; theta1 = q1[0]; phi1 = q1[1];
+          }
           const int s_rw = g0.nslot_aux, s_0 = g0.nslot, s_1 = g1.nslot;
           double m = gsl[0];
 #pragma unroll 4
@@ -293,7 +310,11 @@ __global__ void __launch_bounds__(kFillBlock) reset_fill_kernel(const __grid_con
             dr.z = zs + t * nn;
             dr.uniforms = a.IO.uniforms ? a.IO.uniforms + (int64_t)(t0 + t) * P.n_uniforms * N : nullptr;
             double pair_mean = 0.;
-            pr[0] = gen_tick(g0, pr[0], big ? gsg : gsl, dr, pair_mean, P.gen_ext);
+            if constexpr (SETS)
+              pr[0] = gen_tick_sets(g0, set_params(static_cast<const ResetWsSetsArgs&>(a).ps, set, i0), pr[0], gsl, dr,
+                                    pair_mean);
+            else
+              pr[0] = gen_tick(g0, pr[0], big ? gsg : gsl, dr, pair_mean, P.gen_ext);
             prow[(int64_t)(t0 + t) * na] = pr[0];
           }
         }
@@ -320,6 +341,12 @@ __global__ void __launch_bounds__(kFillBlock) reset_fill_kernel(const __grid_con
     }
   }
 }
+__global__ void __launch_bounds__(kFillBlock) reset_fill_kernel(const __grid_constant__ ResetWsArgs a) {
+  reset_fill_body<false>(a);
+}
+__global__ void __launch_bounds__(kFillBlock) reset_fill_sets_kernel(const __grid_constant__ ResetWsSetsArgs a) {
+  reset_fill_body<true>(a);
+}
 
 // The refill of the all-OU-pairs parameter sets (all_ou_pairs(P)) when the normals come from Philox: one lane per
 // (listed env, pair), np = nA/2 lanes per env, 128/np envs per block.  A pair is an independent process whose three
@@ -338,7 +365,8 @@ __global__ void __launch_bounds__(kFillBlock) reset_fill_kernel(const __grid_con
 #define MDG_FILL_PAIRS_MINB 1
 #endif
 constexpr int kFillPairsUnroll = MDG_FILL_PAIRS_UNROLL;
-__global__ void __launch_bounds__(kFillBlock, MDG_FILL_PAIRS_MINB) reset_fill_pairs_kernel(const __grid_constant__ ResetWsArgs a) {
+template <bool SETS>
+__device__ __forceinline__ void reset_fill_pairs_body(const ResetWsArgs& a) {
   const MdgParams& P = a.P;
   const int tid = threadIdx.x;
   const int na = P.n_assets, np = na >> 1, epb = kFillBlock / np;
@@ -353,7 +381,7 @@ __global__ void __launch_bounds__(kFillBlock, MDG_FILL_PAIRS_MINB) reset_fill_pa
   const uint32_t k0 = (uint32_t)a.L.seed, k1 = (uint32_t)(a.L.seed >> 32);
   const int i0 = 2 * p;
   const MdgAssetGen &g0 = P.gen[i0], &g1 = P.gen[i0 + 1];
-  const double theta0 = g0.p[0], phi0 = g0.p[1], noise = g0.p[2], theta1 = g1.p[0], phi1 = g1.p[1];
+  double theta0 = g0.p[0], phi0 = g0.p[1], noise = g0.p[2], theta1 = g1.p[0], phi1 = g1.p[1];  // SETS: per env below
   // slot s = Philox block s>>1, output s&1: pair p reads blocks b and b+1, b = 3p>>1
   const uint32_t blk = (uint32_t)(3 * p) >> 1;
   const bool odd = p & 1;
@@ -362,6 +390,12 @@ __global__ void __launch_bounds__(kFillBlock, MDG_FILL_PAIRS_MINB) reset_fill_pa
     const bool active = slot < epb && d < count;
     const int64_t e = active ? a.list[d] : 0;
     const long long ts0 = active ? a.S.timestamp[e] : 0;
+    if constexpr (SETS) {  // this lane's pair in the listed env's set (idle lanes read env 0's, and store nothing)
+      const MdgParamSets& ps = static_cast<const ResetWsSetsArgs&>(a).ps;
+      const int64_t set = env_set(ps, e);
+      const SetParams q0 = set_params(ps, set, i0), q1 = set_params(ps, set, i0 + 1);
+      theta0 = q0[0]; phi0 = q0[1]; noise = q0[2]; theta1 = q1[0]; phi1 = q1[1];
+    }
     __syncthreads();  // every lane of an env has read the old timestamp before its pair-0 lane writes the new one
     // idle lanes run the tick loop too (without storing): the loop's shuffles take every lane of the warp
     if (active && p == 0) {  // fresh Broker/Account/Portfolio (Env.h:150-165): per-env scalars
@@ -440,6 +474,13 @@ __global__ void __launch_bounds__(kFillBlock, MDG_FILL_PAIRS_MINB) reset_fill_pa
     }
   }
 }
+__global__ void __launch_bounds__(kFillBlock, MDG_FILL_PAIRS_MINB) reset_fill_pairs_kernel(const __grid_constant__ ResetWsArgs a) {
+  reset_fill_pairs_body<false>(a);
+}
+__global__ void __launch_bounds__(kFillBlock, MDG_FILL_PAIRS_MINB)
+    reset_fill_pairs_sets_kernel(const __grid_constant__ ResetWsSetsArgs a) {
+  reset_fill_pairs_body<true>(a);
+}
 
 // constructor state (Env.h:139-165 before the first tick)
 struct InitArgs {
@@ -448,16 +489,25 @@ struct InitArgs {
   MdgState S;
   MdgLaunch L;
 };
-__global__ void __launch_bounds__(128) init_kernel(const __grid_constant__ InitArgs a) {
+struct InitSetsArgs : InitArgs {
+  MdgParamSets ps;
+};
+// e: computed in the kernels, where the compiler knows the range of threadIdx.x
+template <bool SETS>
+__device__ __forceinline__ void init_body(const InitArgs& a, int64_t e) {
   const int64_t N = a.L.n_envs;
-  const int64_t e = (int64_t)blockIdx.x * 128 + threadIdx.x;
   if (e >= N) return;
   const int na = a.P.n_assets;
   for (int i = 0; i < na; ++i) {
     const MdgAssetGen& g = a.P.gen[i];
     double* gs = a.S.gstate + (int64_t)(g.gslot < 0 ? 0 : g.gslot) * N + e;
     const CtorDraws cd = ctor_draws((uint32_t)(a.L.env_offset + e), a.L.seed, 0, 3, i);
-    a.S.price[(int64_t)i * N + e] = gen_start(g, gs, N, a.P.gen_ext, &cd);
+    if constexpr (SETS) {  // start values (OU mean, Synth phase, trend start) from the env's set
+      const MdgParamSets& ps = static_cast<const InitSetsArgs&>(a).ps;
+      a.S.price[(int64_t)i * N + e] = gen_start_p(g, set_params(ps, env_set(ps, e), i), gs, N, a.P.gen_ext, &cd);
+    } else {
+      a.S.price[(int64_t)i * N + e] = gen_start(g, gs, N, a.P.gen_ext, &cd);
+    }
     a.S.ledger[(int64_t)i * N + e] = 0.;
     a.S.mean_entry[(int64_t)i * N + e] = 0.;
     a.S.borrowed[(int64_t)i * N + e] = 0.;
@@ -475,6 +525,12 @@ __global__ void __launch_bounds__(128) init_kernel(const __grid_constant__ InitA
     if (a.S.shaper_B) a.S.shaper_B[(int64_t)c * N + e] = 0.;
   }
   if (a.S.nstep_len) a.S.nstep_len[e] = 0;
+}
+__global__ void __launch_bounds__(128) init_kernel(const __grid_constant__ InitArgs a) {
+  init_body<false>(a, (int64_t)blockIdx.x * 128 + threadIdx.x);
+}
+__global__ void __launch_bounds__(128) init_sets_kernel(const __grid_constant__ InitSetsArgs a) {
+  init_body<true>(a, (int64_t)blockIdx.x * 128 + threadIdx.x);
 }
 
 // exact left-to-right folds of the portfolio as stored (after external writes into the state tensors)
@@ -529,12 +585,23 @@ static int check_common(const MdgParams* P, const MdgLaunch* L) {
   return MDG_OK;
 }
 
+// parameter sets: a table and an assignment, and only generators whose p slots are plain numbers
+static int check_sets(const MdgParams* P, const MdgParamSets* ps) {
+  if (!ps) return set_err(MDG_E_INVALID, "null parameter sets");
+  if (ps->n_sets < 1) return set_err(MDG_E_INVALID, "parameter sets: n_sets < 1");
+  if (!ps->p || !ps->set_of_env) return set_err(MDG_E_INVALID, "parameter sets: null table / set_of_env");
+  for (int i = 0; i < P->n_assets; ++i)
+    if (P->gen[i].type >= MDG_GEN_SINEADDER)
+      return set_err(MDG_E_UNSUPPORTED, "parameter sets do not support SINE* generators");
+  return MDG_OK;
+}
+
 }  // namespace mdg
 
 using namespace mdg;
 
 static int step_impl(const MdgParams* P, const MdgReward* R, const MdgState* S, const MdgStepIO* IO,
-                     const MdgLaunch* L, int* done_count, int* done_list) {
+                     const MdgLaunch* L, int* done_count, int* done_list, const MdgParamSets* sets = nullptr) {
   int rc = check_common(P, L);
   if (rc) return rc;
   if (!S || !IO) return set_err(MDG_E_INVALID, "null state/io");
@@ -567,12 +634,25 @@ static int step_impl(const MdgParams* P, const MdgReward* R, const MdgState* S, 
   }
   a.done_count = done_count;
   a.done_list = done_list;
-  return launch_step(a);
+  if (!sets) return launch_step(a);
+  StepSetsArgs b;
+  static_cast<StepArgs&>(b) = a;
+  b.ps = *sets;
+  return launch_step<true>(b);
 }
 
 extern "C" int mdg_step(const MdgParams* P, const MdgReward* R, const MdgState* S, const MdgStepIO* IO,
                         const MdgLaunch* L) {
   return step_impl(P, R, S, IO, L, nullptr, nullptr);
+}
+
+extern "C" int mdg_step_sets(const MdgParams* P, const MdgReward* R, const MdgState* S, const MdgStepIO* IO,
+                             const MdgLaunch* L, const MdgParamSets* sets) {
+  int rc = check_common(P, L);
+  if (rc) return rc;
+  rc = check_sets(P, sets);
+  if (rc) return rc;
+  return step_impl(P, R, S, IO, L, nullptr, nullptr, sets);
 }
 
 extern "C" int mdg_reset(const MdgParams* P, const MdgState* S, const MdgStepIO* IO, const MdgLaunch* L,
@@ -648,7 +728,9 @@ constexpr int kFillPairsBlocksPerSm = 2;
 // spreads an env's draws over a block (~12 us).  With few pairs per env that latency is not paid back: one OU pair per
 // env (C3, 65,536 envs, one stream) measured 20.5 us per step with the generic refill, 34.9 with this one.
 constexpr int kFillPairsMinAssets = 8;
-static int launch_fill(const ResetWsArgs& a, int64_t max_listed) {
+// Args: ResetWsArgs, or ResetWsSetsArgs with SETS (the same kernel choice)
+template <bool SETS = false, class Args = ResetWsArgs>
+static int launch_fill(const Args& a, int64_t max_listed) {
   // the count is on the device: size the grid for the most the list can hold, capped at a few blocks per SM
   // (grid-stride; blocks past the end of the list only read the count and take their exit ticket)
   static const int64_t knob = []() {  // MDG_FILL_GRID: profiling knob
@@ -664,23 +746,25 @@ static int launch_fill(const ResetWsArgs& a, int64_t max_listed) {
     const int64_t groups = (max_listed + epb - 1) / epb;
     const int64_t cap = knob ? knob : kFillPairsBlocksPerSm * sm_count();
     const unsigned grid = (unsigned)(groups < cap ? (groups > 0 ? groups : 1) : cap);
-    reset_fill_pairs_kernel<<<grid, kFillBlock, 0, st>>>(a);
+    if constexpr (SETS) reset_fill_pairs_sets_kernel<<<grid, kFillBlock, 0, st>>>(a);
+    else reset_fill_pairs_kernel<<<grid, kFillBlock, 0, st>>>(a);
     return cuda_err(cudaGetLastError(), "reset_fill_pairs launch");
   }
   const int64_t cap = knob ? knob : 148 * 8;
   const unsigned grid = (unsigned)(max_listed < cap ? (max_listed > 0 ? max_listed : 1) : cap);
   const size_t smem = sizeof(double) * (size_t)a.chunk * (size_t)(a.P.n_normals > 0 ? a.P.n_normals : 1);
-  reset_fill_kernel<<<grid, kFillBlock, smem, st>>>(a);
+  if constexpr (SETS) reset_fill_sets_kernel<<<grid, kFillBlock, smem, st>>>(a);
+  else reset_fill_kernel<<<grid, kFillBlock, smem, st>>>(a);
   return cuda_err(cudaGetLastError(), "reset_fill launch");
 }
 }  // namespace mdg
 
-extern "C" int mdg_reset_ws(const MdgParams* P, const MdgState* S, const MdgStepIO* IO, const MdgLaunch* L,
-                            const uint8_t* mask, int fill_ticks, int clear_nstep, void* workspace,
-                            int64_t workspace_bytes) {
-  if (!workspace) return mdg_reset(P, S, IO, L, mask, fill_ticks, clear_nstep);
+static int reset_ws_impl(const MdgParams* P, const MdgState* S, const MdgStepIO* IO, const MdgLaunch* L,
+                         const uint8_t* mask, int fill_ticks, int clear_nstep, void* workspace, int64_t workspace_bytes,
+                         const MdgParamSets* sets) {
   int rc = check_common(P, L);
   if (rc) return rc;
+  if (sets && (rc = check_sets(P, sets))) return rc;
   if (!S || !IO) return set_err(MDG_E_INVALID, "null state/io");
   if (!S->reset_ts || !IO->pre_price) return set_err(MDG_E_INVALID, "state.reset_ts / io.pre_price is null");
   if (L->window < 1 || L->head < 0 || L->head >= L->window) return set_err(MDG_E_INVALID, "bad window/head");
@@ -688,7 +772,7 @@ extern "C" int mdg_reset_ws(const MdgParams* P, const MdgState* S, const MdgStep
   if (fill_ticks > L->window) return set_err(MDG_E_INVALID, "fill_ticks > window");
   const int64_t N = L->n_envs;
   if (N == 0) return MDG_OK;
-  ResetWsArgs a;
+  ResetWsSetsArgs a;
   rc = fill_ws_args(a, P, S, IO, L, fill_ticks, clear_nstep, workspace, workspace_bytes);
   if (rc) return rc;
   a.mask = mask;
@@ -696,42 +780,92 @@ extern "C" int mdg_reset_ws(const MdgParams* P, const MdgState* S, const MdgStep
   cudaError_t ce = cudaMemsetAsync(workspace, 0, 256, st);  // an explicit reset does not rely on the header's state
   if (ce != cudaSuccess) return cuda_err(ce, "mdg_reset_ws memset");
   reset_scan_kernel<<<(unsigned)((N + 255) / 256), 256, 0, st>>>(a);
-  return launch_fill(a, N);
+  if (!sets) return launch_fill(static_cast<const ResetWsArgs&>(a), N);
+  a.ps = *sets;
+  return launch_fill<true>(a, N);
 }
 
-extern "C" int mdg_step_autoreset(const MdgParams* P, const MdgReward* R, const MdgState* S, const MdgStepIO* IO,
-                                  const MdgLaunch* L, int fill_ticks, int clear_nstep, void* workspace,
-                                  int64_t workspace_bytes) {
+extern "C" int mdg_reset_ws(const MdgParams* P, const MdgState* S, const MdgStepIO* IO, const MdgLaunch* L,
+                            const uint8_t* mask, int fill_ticks, int clear_nstep, void* workspace,
+                            int64_t workspace_bytes) {
+  if (!workspace) return mdg_reset(P, S, IO, L, mask, fill_ticks, clear_nstep);
+  return reset_ws_impl(P, S, IO, L, mask, fill_ticks, clear_nstep, workspace, workspace_bytes, nullptr);
+}
+
+extern "C" int mdg_reset_ws_sets(const MdgParams* P, const MdgState* S, const MdgStepIO* IO, const MdgLaunch* L,
+                                 const uint8_t* mask, int fill_ticks, int clear_nstep, void* workspace,
+                                 int64_t workspace_bytes, const MdgParamSets* sets) {
+  if (!sets) return set_err(MDG_E_INVALID, "null parameter sets");
+  if (!workspace) return set_err(MDG_E_INVALID, "mdg_reset_ws_sets needs a workspace");
+  return reset_ws_impl(P, S, IO, L, mask, fill_ticks, clear_nstep, workspace, workspace_bytes, sets);
+}
+
+static int step_autoreset_impl(const MdgParams* P, const MdgReward* R, const MdgState* S, const MdgStepIO* IO,
+                               const MdgLaunch* L, int fill_ticks, int clear_nstep, void* workspace,
+                               int64_t workspace_bytes, const MdgParamSets* sets) {
   int rc = check_common(P, L);
   if (rc) return rc;
+  if (sets && (rc = check_sets(P, sets))) return rc;
   if (!workspace) return set_err(MDG_E_INVALID, "mdg_step_autoreset needs a workspace");
   if (!S || !IO) return set_err(MDG_E_INVALID, "null state/io");
   if (!S->reset_ts || !IO->pre_price) return set_err(MDG_E_INVALID, "state.reset_ts / io.pre_price is null");
   if (fill_ticks < 1) fill_ticks = 1;
   if (fill_ticks > L->window) return set_err(MDG_E_INVALID, "fill_ticks > window");
   if (L->n_envs == 0) return MDG_OK;
-  ResetWsArgs a;
+  ResetWsSetsArgs a;
   MdgStepIO io = *IO;  // the reset draws from Philox (no injected stream) and takes no units
   io.units = nullptr; io.normals = nullptr; io.uniforms = nullptr; io.actions = nullptr; io.weights = nullptr;
   rc = fill_ws_args(a, P, S, &io, L, fill_ticks, clear_nstep, workspace, workspace_bytes);
   if (rc) return rc;
-  rc = step_impl(P, R, S, IO, L, a.count, a.list);  // the step kernel appends the finished envs to the list
+  rc = step_impl(P, R, S, IO, L, a.count, a.list, sets);  // the step kernel appends the finished envs to the list
   if (rc) return rc;
-  return launch_fill(a, L->n_envs);
+  if (!sets) return launch_fill(static_cast<const ResetWsArgs&>(a), L->n_envs);
+  a.ps = *sets;
+  return launch_fill<true>(a, L->n_envs);
 }
 
-extern "C" int mdg_init_state(const MdgParams* P, const MdgReward* R, const MdgState* S, const MdgLaunch* L) {
+extern "C" int mdg_step_autoreset(const MdgParams* P, const MdgReward* R, const MdgState* S, const MdgStepIO* IO,
+                                  const MdgLaunch* L, int fill_ticks, int clear_nstep, void* workspace,
+                                  int64_t workspace_bytes) {
+  return step_autoreset_impl(P, R, S, IO, L, fill_ticks, clear_nstep, workspace, workspace_bytes, nullptr);
+}
+
+extern "C" int mdg_step_autoreset_sets(const MdgParams* P, const MdgReward* R, const MdgState* S, const MdgStepIO* IO,
+                                       const MdgLaunch* L, int fill_ticks, int clear_nstep, void* workspace,
+                                       int64_t workspace_bytes, const MdgParamSets* sets) {
+  if (!sets) return set_err(MDG_E_INVALID, "null parameter sets");
+  return step_autoreset_impl(P, R, S, IO, L, fill_ticks, clear_nstep, workspace, workspace_bytes, sets);
+}
+
+static int init_state_impl(const MdgParams* P, const MdgReward* R, const MdgState* S, const MdgLaunch* L,
+                           const MdgParamSets* sets) {
   int rc = check_common(P, L);
   if (rc) return rc;
+  if (sets && (rc = check_sets(P, sets))) return rc;
   if (!S) return set_err(MDG_E_INVALID, "null state");
   if (L->n_envs == 0) return MDG_OK;
-  InitArgs a;
+  InitSetsArgs a;
   a.P = *P;
   if (R) a.R = *R; else { memset(&a.R, 0, sizeof(a.R)); a.R.nstep = 1; }
   a.S = *S; a.L = *L;
   const unsigned grid = (unsigned)((L->n_envs + 128 - 1) / 128);
-  init_kernel<<<grid, 128, 0, (cudaStream_t)L->stream>>>(a);
+  if (sets) {
+    a.ps = *sets;
+    init_sets_kernel<<<grid, 128, 0, (cudaStream_t)L->stream>>>(a);
+  } else {
+    init_kernel<<<grid, 128, 0, (cudaStream_t)L->stream>>>(static_cast<const InitArgs&>(a));
+  }
   return cuda_err(cudaGetLastError(), "mdg_init_state launch");
+}
+
+extern "C" int mdg_init_state(const MdgParams* P, const MdgReward* R, const MdgState* S, const MdgLaunch* L) {
+  return init_state_impl(P, R, S, L, nullptr);
+}
+
+extern "C" int mdg_init_state_sets(const MdgParams* P, const MdgReward* R, const MdgState* S, const MdgLaunch* L,
+                                   const MdgParamSets* sets) {
+  if (!sets) return set_err(MDG_E_INVALID, "null parameter sets");
+  return init_state_impl(P, R, S, L, sets);
 }
 
 extern "C" int mdg_refresh_folds(const MdgParams* P, const MdgState* S, const MdgLaunch* L) {
@@ -774,6 +908,7 @@ extern "C" int mdg_sizeof(int which) {
     case 11: return (int)sizeof(MdgTearsheet);
     case 12: return (int)sizeof(MdgPrioritized);
     case 13: return (int)sizeof(MdgReplayRows);
+    case 14: return (int)sizeof(MdgParamSets);
   }
   return -1;
 }

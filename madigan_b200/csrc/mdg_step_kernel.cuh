@@ -39,6 +39,12 @@ struct StepArgs {
   alignas(64) CUtensorMap tm_units;
 };
 
+// the launches with parameter sets (mdg_step_sets): the table and the assignment, after everything the other launches
+// read, so that their kernels' parameters are unchanged
+struct StepSetsArgs : StepArgs {
+  MdgParamSets ps;
+};
+
 constexpr int kBlock = 128;
 
 // experiment knobs (MDG_EXTRA_NVCC_FLAGS + MDG_LIB_VARIANT, see build.py); the defaults are the measured best
@@ -549,7 +555,7 @@ __device__ __forceinline__ unsigned long long global_ns() {
 #define MDG_PCLK(slot)
 #endif
 
-template <bool PAIRS, int BS, bool ACTIONS, bool TX2, bool BULK>
+template <bool PAIRS, int BS, bool ACTIONS, bool TX2, bool BULK, bool SETS = false>
 __device__ __forceinline__ void step_body(const StepArgs& a) {
   MDG_PCLK(0);
 #ifdef MDG_PHASE_CLOCKS
@@ -575,6 +581,9 @@ __device__ __forceinline__ void step_body(const StepArgs& a) {
   // vectors (one per pair) that bypass L1, so that the 64 KB of unit lines per SM do not evict the prefetched state
   const bool units_v2 = MDG_UNITS_CG && PAIRS && mode == MDG_MODE_MULTI && a.units_v2;
   if (e >= N) return;
+  // parameter sets: this env's set (SETS only; the table's address and n_sets stay kernel-parameter operands)
+  uint32_t set = 0;
+  if constexpr (SETS) set = (uint32_t)env_set(static_cast<const StepSetsArgs&>(a).ps, e);
   // Bulk staging (all-pairs kernel, whole blocks only): the nine 1-KB state rows a block needs for a pair are
   // contiguous in the [rows][N] tensors, so one elected thread fetches them with nine cp.async.bulk copies into a
   // two-stage shared-memory ring, two pairs ahead, completion on an mbarrier per stage.  The bytes are in flight
@@ -827,10 +836,21 @@ __device__ __forceinline__ void step_body(const StepArgs& a) {
         z0 = st[(4 * p + 1) * BS];
         z1 = st[(4 * p + 2) * BS];
       }
-      mean += mean * (z_rw * g0.p[2]);
-      gst(&S.gstate[(int64_t)g0.gslot * N + e], mean);
-      const double newp0 = price[0] + ((g0.p[0] * (mean - price[0])) + mean * (z0 * g0.p[1]));
-      const double newp1 = price[1] + ((g1.p[0] * (mean - price[1])) + mean * (z1 * g1.p[1]));
+      double newp0, newp1;
+      if constexpr (SETS) {  // the pair's five values of this env's set
+        const MdgParamSets& ps = static_cast<const StepSetsArgs&>(a).ps;
+        const SetParams q0 = set_params(ps, set, 2 * p), q1 = set_params(ps, set, 2 * p + 1);
+        const double s_theta0 = q0[0], s_phi0 = q0[1], s_noise = q0[2], s_theta1 = q1[0], s_phi1 = q1[1];
+        mean += mean * (z_rw * s_noise);
+        gst(&S.gstate[(int64_t)g0.gslot * N + e], mean);
+        newp0 = price[0] + ((s_theta0 * (mean - price[0])) + mean * (z0 * s_phi0));
+        newp1 = price[1] + ((s_theta1 * (mean - price[1])) + mean * (z1 * s_phi1));
+      } else {
+        mean += mean * (z_rw * g0.p[2]);
+        gst(&S.gstate[(int64_t)g0.gslot * N + e], mean);
+        newp0 = price[0] + ((g0.p[0] * (mean - price[0])) + mean * (z0 * g0.p[1]));
+        newp1 = price[1] + ((g1.p[0] * (mean - price[1])) + mean * (z1 * g1.p[1]));
+      }
       post_tick<true, BS>(a, A, N, e, na, 2 * p, cur[0], newp0, prev_val[0], tp[0], tu[0], tc[0], st);
       post_tick<true, BS>(a, A, N, e, na, 2 * p + 1, cur[1], newp1, prev_val[1], tp[1], tu[1], tc[1], st);
       MDG_PCLK(6 + 4 * p);
@@ -860,7 +880,24 @@ __device__ __forceinline__ void step_body(const StepArgs& a) {
       // generator tick of this asset (DataSource.cpp getData family)
       const MdgAssetGen& g = P.gen[i];
       double newp;
-      if (g.type == MDG_GEN_OUPAIR) {  // OUPair::getData :1232-1240 (draw order rw, x0, x1)
+      if constexpr (SETS) {  // the same bodies, parameters from this env's set
+        const SetParams sp = set_params(static_cast<const StepSetsArgs&>(a).ps, set, i);
+        if (g.type == MDG_GEN_OUPAIR) {
+          if (g.role == 0) {
+            double* mrow = S.gstate + (int64_t)g.gslot * N + e;
+            double m = *mrow;
+            m += m * (draw_normal(dr, g.nslot_aux) * sp[2]);
+            *mrow = m;
+            pair_mean = m;
+          }
+          newp = price + ((sp[0] * (pair_mean - price)) + pair_mean * (draw_normal(dr, g.nslot) * sp[1]));
+        } else if (g.type == MDG_GEN_OU) {
+          newp = price + ((sp[1] * (sp[0] - price)) + sp[0] * sp[2] * draw_normal(dr, g.nslot));
+        } else {
+          double* gs = S.gstate + (int64_t)(g.gslot < 0 ? 0 : g.gslot) * N + e;
+          newp = gen_tick_sets(g, sp, price, gs, dr, pair_mean);
+        }
+      } else if (g.type == MDG_GEN_OUPAIR) {  // OUPair::getData :1232-1240 (draw order rw, x0, x1)
         if (g.role == 0) {
           double* mrow = S.gstate + (int64_t)g.gslot * N + e;
           double m = *mrow;
@@ -1022,6 +1059,12 @@ __global__ void __launch_bounds__(BS, MINB) step_kernel(const __grid_constant__ 
   step_body<PAIRS, BS, ACTIONS, (MINB < 4) || (BULK && MDG_BULK_TX2), BULK>(a);  // MINB 3 = the multi-wave register budget
 }
 
+// the same instantiations for the launches with parameter sets (mdg_step_sets): 128-thread blocks only
+template <bool PAIRS, int BS, int MINB, bool ACTIONS, bool BULK = false>
+__global__ void __launch_bounds__(BS, MINB) step_sets_kernel(const __grid_constant__ StepSetsArgs a) {
+  step_body<PAIRS, BS, ACTIONS, (MINB < 4) || (BULK && MDG_BULK_TX2), BULK, true>(a);
+}
+
 // 64-thread blocks, seven per SM (one-wave launches): at 128 registers (registers are granted per warp in units that make 136 or 144 x 14 warps overflow the file: measured two waves)
 #ifndef MDG_BS64_REGS
 #define MDG_BS64_REGS 128
@@ -1111,7 +1154,16 @@ static inline bool step_tensor_map(const StepMapKey& k, CUtensorMap* out) {
   return true;
 }
 
-static inline int launch_step(StepArgs& a) {
+// one 128-thread instantiation of the step kernel, with or without parameter sets
+template <bool SETS, bool PAIRS, int MINB, bool ACT, bool BULK, class Args>
+static inline void launch_step128(const Args& a, unsigned grid, size_t smem, cudaStream_t st) {
+  if constexpr (SETS) step_sets_kernel<PAIRS, 128, MINB, ACT, BULK><<<grid, 128, smem, st>>>(a);
+  else step_kernel<PAIRS, 128, MINB, ACT, BULK><<<grid, 128, smem, st>>>(a);
+}
+
+// Args: StepArgs, or StepSetsArgs with SETS
+template <bool SETS = false, class Args = StepArgs>
+static inline int launch_step(Args& a) {
   const int64_t N = a.L.n_envs;
   cudaStream_t st = (cudaStream_t)a.L.stream;
   const bool pairs = all_ou_pairs(a.P);
@@ -1136,7 +1188,7 @@ static inline int launch_step(StepArgs& a) {
   // Measured (profiles/block_times.py, r2_notes.md): the launch still ends with the youngest block of the fullest SMs
   // at ~30.5 us either way; 36.2 against 37.1 us for a lone launch, no difference inside bench.py -- not the default.
   static const int bs64_on = [] { const char* v = getenv("MDG_BS64"); return v ? atoi(v) : 0; }();
-  const int bs = (pairs && bs64_on && N <= 148 * 7 * 64) ? 64 : 128;
+  const int bs = (!SETS && pairs && bs64_on && N <= 148 * 7 * 64) ? 64 : 128;  // no 64-thread sets instantiation
   const unsigned grid = (unsigned)((N + bs - 1) / bs);
   a.bulk = (pairs && !bulk_off && N % bs == 0 && al16(a.S.price) && al16(a.S.ledger) && al16(a.S.mean_entry) &&
             al16(a.S.borrowed) && al16(a.S.gstate)) ? 1 : 0;
@@ -1165,34 +1217,43 @@ static inline int launch_step(StepArgs& a) {
         const cudaError_t r_ = cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, 56 * 1024);
         if (r_ != cudaSuccess) e_ = r_;
       };
-      set((const void*)step_kernel<true, 128, 4, true, true>); set((const void*)step_kernel<true, 128, 4, false, true>);
-      set((const void*)step_kernel<true, 128, 3, true, true>); set((const void*)step_kernel<true, 128, 3, false, true>);
+      if constexpr (SETS) {
+        set((const void*)step_sets_kernel<true, 128, 4, true, true>);
+        set((const void*)step_sets_kernel<true, 128, 4, false, true>);
+        set((const void*)step_sets_kernel<true, 128, 3, true, true>);
+        set((const void*)step_sets_kernel<true, 128, 3, false, true>);
+      } else {
+        set((const void*)step_kernel<true, 128, 4, true, true>); set((const void*)step_kernel<true, 128, 4, false, true>);
+        set((const void*)step_kernel<true, 128, 3, true, true>); set((const void*)step_kernel<true, 128, 3, false, true>);
+      }
       return e_;
     }();
     if (attr != cudaSuccess) return cuda_err(attr, "mdg_step shared-memory opt-in");
   }
   const bool acts = a.L.mode == MDG_MODE_MULTI && (a.IO.actions || a.IO.weights);
-#define MDG_LAUNCH(PAIRS_, MINB_, ACT_) step_kernel<PAIRS_, 128, MINB_, ACT_><<<grid, 128, smem, st>>>(a)
+#define MDG_LAUNCH(PAIRS_, MINB_, ACT_, BULK_) launch_step128<SETS, PAIRS_, MINB_, ACT_, BULK_>(a, grid, smem, st)
   if (bs == 64) {
-    if (a.bulk) {
-      if (acts) step_kernel64<true, true><<<grid, 64, smem, st>>>(a);
-      else step_kernel64<false, true><<<grid, 64, smem, st>>>(a);
-    } else {
-      if (acts) step_kernel64<true, false><<<grid, 64, smem, st>>>(a);
-      else step_kernel64<false, false><<<grid, 64, smem, st>>>(a);
+    if constexpr (!SETS) {
+      if (a.bulk) {
+        if (acts) step_kernel64<true, true><<<grid, 64, smem, st>>>(a);
+        else step_kernel64<false, true><<<grid, 64, smem, st>>>(a);
+      } else {
+        if (acts) step_kernel64<true, false><<<grid, 64, smem, st>>>(a);
+        else step_kernel64<false, false><<<grid, 64, smem, st>>>(a);
+      }
     }
   } else if (small && a.bulk) {
-    if (acts) step_kernel<true, 128, 4, true, true><<<grid, 128, smem, st>>>(a);
-    else step_kernel<true, 128, 4, false, true><<<grid, 128, smem, st>>>(a);
+    if (acts) MDG_LAUNCH(true, 4, true, true);
+    else MDG_LAUNCH(true, 4, false, true);
   } else if (a.bulk) {
-    if (acts) step_kernel<true, 128, 3, true, true><<<grid, 128, smem, st>>>(a);
-    else step_kernel<true, 128, 3, false, true><<<grid, 128, smem, st>>>(a);
+    if (acts) MDG_LAUNCH(true, 3, true, true);
+    else MDG_LAUNCH(true, 3, false, true);
   } else if (small) {
-    if (pairs) { if (acts) MDG_LAUNCH(true, 4, true); else MDG_LAUNCH(true, 4, false); }
-    else { if (acts) MDG_LAUNCH(false, 4, true); else MDG_LAUNCH(false, 4, false); }
+    if (pairs) { if (acts) MDG_LAUNCH(true, 4, true, false); else MDG_LAUNCH(true, 4, false, false); }
+    else { if (acts) MDG_LAUNCH(false, 4, true, false); else MDG_LAUNCH(false, 4, false, false); }
   } else {
-    if (pairs) { if (acts) MDG_LAUNCH(true, 3, true); else MDG_LAUNCH(true, 3, false); }
-    else { if (acts) MDG_LAUNCH(false, 3, true); else MDG_LAUNCH(false, 3, false); }
+    if (pairs) { if (acts) MDG_LAUNCH(true, 3, true, false); else MDG_LAUNCH(true, 3, false, false); }
+    else { if (acts) MDG_LAUNCH(false, 3, true, false); else MDG_LAUNCH(false, 3, false, false); }
   }
 #undef MDG_LAUNCH
   return cuda_err(cudaGetLastError(), "mdg_step launch");

@@ -268,6 +268,59 @@ def build_generator_table(data_source_type, data_source_config=None, with_ext=Fa
     return out + (tab.ext,) if with_ext else out
 
 
+# Reference key name of every p[] slot per generator type, in the order _add_source fills them (include/madigan_b200.h
+# lists the same slots).  Parameter sets (make_param_table) can vary every one of them.
+PARAM_SLOTS = {
+    "Synth": ("freq", "mu", "amp", "phase", "dX", "noise"),
+    "SawTooth": ("freq", "mu", "amp", "phase", "dX", "noise"),
+    "Triangle": ("freq", "mu", "amp", "phase", "dX", "noise"),
+    "Gaussian": ("mean", "var"),
+    "OU": ("mean", "theta", "phi"),
+    "OUPair": ("theta", "phi", "noise"),
+    "SimpleTrend": ("trend_prob", "min_period", "max_period", "noise", "start", "dYMin", "dYMax"),
+    "TrendOU": ("trend_prob", "min_period", "max_period", "dYMin", "dYMax", "start", "theta", "phi", "noise_trend",
+                "ema_alpha"),
+    "TrendyOU": ("trend_prob", "min_period", "max_period", "dYMin", "dYMax", "start", "theta", "phi", "noise_trend",
+                 "ema_alpha"),
+}
+_SINE_TYPES = (A.GEN_SINEADDER, A.GEN_SINEDYNAMIC, A.GEN_SINEDYNAMICTREND)
+_STRUCTURE = ("type", "role", "nslot", "nslot_aux", "uslot", "gslot", "partner")
+
+
+def make_param_table(data_source_type, base_config, set_configs):
+    """Generator parameter table of a multi-set ``Env``: a ``(nA, MDG_GEN_NPARAM, S)`` float64 array whose
+    ``[:, :, s]`` holds the ``p`` slots of every asset built from ``set_configs[s]`` (set-minor, the layout of
+    ``MdgParamSets.p``).  Every set must describe the same assets as ``base_config``: same names, types, roles and
+    noise / uniform / state slots; only the parameter values may differ.  SINE* sources are not supported (their slots
+    are component counts and table offsets).  Raises ValueError naming the first asset that breaks either rule."""
+    names, base, n_g, n_n, n_u = build_generator_table(data_source_type, base_config)
+    for i, rec in enumerate(base):
+        if rec["type"] in _SINE_TYPES:
+            raise ValueError(f"asset {i} ({names[i]}): SINE* sources do not support parameter sets")
+    set_configs = list(set_configs)
+    if not set_configs:
+        raise ValueError("parameter sets: need at least one set")
+    table = np.empty((len(base), A.MDG_GEN_NPARAM, len(set_configs)), dtype=np.float64)
+    built = {}  # one build per distinct config object (an int S passes the base config S times)
+    for s, cfg in enumerate(set_configs):
+        if id(cfg) not in built:
+            built[id(cfg)] = build_generator_table(data_source_type, cfg)
+        names_s, recs, n_g_s, n_n_s, n_u_s = built[id(cfg)]
+        for i in range(max(len(base), len(recs))):
+            if i >= len(recs) or i >= len(base):
+                name = names[i] if i < len(base) else names_s[i]
+                raise ValueError(f"parameter set {s}: asset {i} ({name}) is not in both the base and the set")
+            if names_s[i] != names[i]:
+                raise ValueError(f"parameter set {s}: asset {i} is {names_s[i]}, the base has {names[i]}")
+            for key in _STRUCTURE:
+                if recs[i][key] != base[i][key]:
+                    raise ValueError(f"parameter set {s}: asset {i} ({names[i]}) differs from the base in {key}")
+        if (n_g_s, n_n_s, n_u_s) != (n_g, n_n, n_u):  # implied by the slots above; kept as a guard on the builder
+            raise ValueError(f"parameter set {s}: generator state / noise rows differ from the base")
+        table[:, :, s] = [r["p"] for r in recs]
+    return table
+
+
 def make_params(data_source_type, data_source_config=None, init_cash=1_000_000.,
                 required_margin=0., maintenance_margin=0., slippage_rel=0., slippage_abs=0.,
                 transaction_cost_rel=0., transaction_cost_abs=0.):

@@ -13,7 +13,7 @@ import torch
 from .. import _abi as A
 from .._lib import check, lib
 from ..utils.data import BrokerResponse, EnvInfo, State
-from .data_source import make_params, make_reward
+from .data_source import make_param_table, make_params, make_reward
 
 
 def _cfg_get(cfg, key, default=None):
@@ -93,11 +93,17 @@ def _reset_workspace(lib_, P, n_envs, fill_ticks, device, stream_ptr=None, strea
 
 class Env:
     def __init__(self, dataSourceType, initCash=1_000_000., config=None, *, n_envs=None, device=None,
-                 window=None, seed=None, env_offset=0, reward=None):
+                 window=None, seed=None, env_offset=0, reward=None, param_sets=None, param_set=None):
         """``Env(data_source_type, init_cash, config)`` as the reference (env.cpp:843-849); the batched
         keys ``n_envs``, ``seed``, ``device``, ``window_length`` may come from ``config`` or keywords.
         ``reward``: None (env reward only) or a dict with ``reward_shaper_config``, ``nstep_return``,
-        ``discount``, ``reduce_rewards`` to also compute the agent + shaped rewards in the step kernel."""
+        ``discount``, ``reduce_rewards`` to also compute the agent + shaped rewards in the step kernel.
+        ``param_sets``: generator parameter sets, so that the envs of the slab tick different markets -- a list of
+        ``data_source_config`` dicts for ``dataSourceType`` (same assets as the base config, other values), or an int
+        ``S`` for S copies of the base config (to be edited through ``param_table``).  ``param_set``: the ``(N,)``
+        integer set of every env, ``arange(N) % S`` by default.  Env e then equals, bit for bit, env e of a plain Env
+        built from its set's config with the same ``n_envs``, ``seed`` and ``env_offset``
+        (see ``make_param_table``, ``assign_param_sets``)."""
         self._lib = lib()
         if not torch.cuda.is_available():
             raise RuntimeError("madigan_b200.Env needs a CUDA device (sm_100a); there is no CPU fallback")
@@ -132,6 +138,9 @@ class Env:
                                  n_assets=self.nA)
         self.ra = 1 if self.R.reduce_rewards else self.nA
         self._alloc()
+        self._PS = None  # MdgParamSets of an env with parameter sets
+        if param_sets is not None:
+            self._init_param_sets(dataSourceType, ds_cfg, param_sets, param_set)
         self.head = 0
         self.n_valid = 0
         self._gstep = 0
@@ -140,7 +149,12 @@ class Env:
         self.launches = 0  # kernels launched so far (bench.py's gpu_launches)
         self.flags = 0     # MdgLaunch.flags (validation: A.FLAG_FORCE_EXACT_GATE, A.FLAG_GENERIC_FILL)
         with torch.cuda.device(self.device):
-            check(self._lib.mdg_init_state(C.byref(self.P), C.byref(self.R), C.byref(self._S), C.byref(self._launch())))
+            if self._PS is None:
+                check(self._lib.mdg_init_state(C.byref(self.P), C.byref(self.R), C.byref(self._S),
+                                               C.byref(self._launch())))
+            else:
+                check(self._lib.mdg_init_state_sets(C.byref(self.P), C.byref(self.R), C.byref(self._S),
+                                                    C.byref(self._launch()), self._pPS))
             self.launches += 1
             # the constructor consumes one generator tick (Env.h:160)
             self._reset_launch(None, 1, False, None, None)
@@ -194,6 +208,77 @@ class Env:
         self._states = [None] * k
         self._want_multi, self._want_single = torch.Size((N, nA)), torch.Size((N,))
         self._done_u8 = t["done"].view(torch.uint8)
+
+    # ------------------------------------------------------------------ generator parameter sets
+    def _init_param_sets(self, ds_type, ds_cfg, param_sets, param_set):
+        if isinstance(param_sets, bool) or not isinstance(param_sets, (int, list, tuple)):
+            raise TypeError("param_sets must be a list of data_source_config dicts or an int")
+        if isinstance(param_sets, int):
+            if param_sets < 1:
+                raise ValueError("param_sets must be >= 1")
+            param_sets = [ds_cfg] * param_sets
+        table = make_param_table(ds_type, ds_cfg, param_sets)  # (nA, NPARAM, S), set-minor
+        S = table.shape[2]
+        # [nA][NPARAM][S] storage, as MdgParamSets.p reads it
+        self._ptab = torch.from_numpy(table).to(self.device).contiguous()
+        self._pset = torch.arange(self.N, device=self.device, dtype=torch.int32) % S
+        if param_set is not None:
+            self.assign_param_sets(param_set)
+        self._PS = A.MdgParamSets(p=self._ptab.data_ptr(), set_of_env=self._pset.data_ptr(), n_sets=S)
+        self._pPS = C.byref(self._PS)
+
+    @property
+    def n_param_sets(self):
+        """Number of generator parameter sets (0: the env was built without ``param_sets``)."""
+        return 0 if self._PS is None else int(self._PS.n_sets)
+
+    @property
+    def param_table(self):
+        """``(S, nA, MDG_GEN_NPARAM)`` fp64 device view of the parameter sets: ``param_table[s, i, j]`` is slot j
+        (``data_source.PARAM_SLOTS``) of asset i in set s.  Writable in place; every launch reads the table as it
+        stands on the env's stream, so a change takes effect at the next step or reset and an episode in progress
+        continues under the new values.  None without parameter sets."""
+        return None if self._PS is None else self._ptab.permute(2, 0, 1)
+
+    @property
+    def param_set(self):
+        """``(N,)`` int32: the parameter set of every env (read it; change it with ``assign_param_sets``)."""
+        return None if self._PS is None else self._pset
+
+    def assign_param_sets(self, ids, mask=None):
+        """Set the parameter set of every env (``mask=None``) or of the envs where ``mask`` (N,) is true to ``ids``
+        (an (N,) integer tensor/array, or one int).  Checks the range with one host synchronisation (a setup call, not
+        one for the hot loop), then writes on the env's stream.  The change takes effect at the next launch: an episode
+        in progress continues under the new values.  For a new market per episode, step without ``auto_reset``, then
+        ``assign_param_sets(new_ids, mask=done)`` and ``reset(mask=done, fill_history=True)``: the refill already
+        ticks the new set."""
+        if self._PS is None and not hasattr(self, "_pset"):
+            raise RuntimeError("this Env was built without param_sets")
+        S = self._ptab.shape[2]
+        with self._device_ctx():
+            ids = torch.as_tensor(ids, device=self.device)
+            if ids.dtype.is_floating_point or ids.dtype.is_complex or ids.dtype == torch.bool:
+                raise ValueError(f"parameter set ids must be integers, got {ids.dtype}")
+            if ids.dim() == 0:
+                ids = ids.expand(self.N)
+            if tuple(ids.shape) != (self.N,):
+                raise ValueError(f"parameter set ids must have shape ({self.N},), got {tuple(ids.shape)}")
+            lo, hi = (int(v) for v in torch.aminmax(ids))
+            if lo < 0 or hi >= S:
+                raise ValueError(f"parameter set ids must be in [0, {S}), got [{lo}, {hi}]")
+            m = None
+            if mask is not None:
+                m = torch.as_tensor(mask, device=self.device)
+                if tuple(m.shape) != (self.N,):
+                    raise ValueError(f"mask must have shape ({self.N},)")
+                m = m.to(torch.bool)
+            if self._stream is not None:
+                self._stream.wait_stream(torch.cuda.current_stream(self.device))
+            with self._copy_ctx():
+                if m is None:
+                    self._pset.copy_(ids)
+                else:
+                    self._pset.copy_(torch.where(m, ids.to(torch.int32), self._pset))
 
     def _launch(self, mode=A.MODE_HOLD, asset_idx=0):
         """The (persistent) launch descriptor, refreshed for this call: the host path of a step is a handful of
@@ -282,9 +367,14 @@ class Env:
             if tuple(m.shape) != (self.N,):
                 raise ValueError(f"mask must have shape ({self.N},)")
         ws = _reset_workspace(self._lib, self.P, self.N, int(fill_ticks), self.device, self._stream_ptr, self._stream)
-        check(self._lib.mdg_reset_ws(C.byref(self.P), C.byref(self._S), C.byref(io), C.byref(self._launch()),
-                                     None if m is None else m.data_ptr(), int(fill_ticks), int(clear_nstep),
-                                     ws.data_ptr(), ws.numel()))
+        if self._PS is None:
+            check(self._lib.mdg_reset_ws(C.byref(self.P), C.byref(self._S), C.byref(io), C.byref(self._launch()),
+                                         None if m is None else m.data_ptr(), int(fill_ticks), int(clear_nstep),
+                                         ws.data_ptr(), ws.numel()))
+        else:
+            check(self._lib.mdg_reset_ws_sets(C.byref(self.P), C.byref(self._S), C.byref(io), C.byref(self._launch()),
+                                              None if m is None else m.data_ptr(), int(fill_ticks), int(clear_nstep),
+                                              ws.data_ptr(), ws.numel(), self._pPS))
         self.launches += 2  # list scan + refill kernel
         self._version += 1
         del keep
@@ -358,12 +448,18 @@ class Env:
             self.head = head0  # the ring head moves only once the launch has been accepted
             if auto_reset and keep is None and tearsheet is None:  # step + masked reset + history fill in one trip through the binding
                 ws = _reset_workspace(self._lib, self.P, self.N, self.k, self.device, self._stream_ptr, self._stream)
-                check(self._lib.mdg_step_autoreset(self._pP, self._pR, self._pS, self._pIO, self._pL, self.k, 1,
-                                                   ws.data_ptr(), ws.numel()))
+                if self._PS is None:
+                    check(self._lib.mdg_step_autoreset(self._pP, self._pR, self._pS, self._pIO, self._pL, self.k, 1,
+                                                       ws.data_ptr(), ws.numel()))
+                else:
+                    self._step_autoreset_call(ws)
                 self.launches += 2  # step kernel (appends the finished envs to the list) + refill kernel
                 auto_reset = False
             else:
-                check(self._lib.mdg_step(self._pP, self._pR, self._pS, self._pIO, self._pL))
+                if self._PS is None:
+                    check(self._lib.mdg_step(self._pP, self._pR, self._pS, self._pIO, self._pL))
+                else:
+                    check(self._lib.mdg_step_sets(self._pP, self._pR, self._pS, self._pIO, self._pL, self._pPS))
                 self.launches += 1
             self.head = L.head
             self.n_valid = min(self.k, self.n_valid + 1)
@@ -376,6 +472,20 @@ class Env:
                 self._reset_launch(self.t["done"], self.k, True, None, None)
         t = self.t
         return self._state(), t["reward"], t["done"], self._info
+
+    def _step_call(self):
+        if self._PS is None:
+            check(self._lib.mdg_step(self._pP, self._pR, self._pS, self._pIO, self._pL))
+        else:
+            check(self._lib.mdg_step_sets(self._pP, self._pR, self._pS, self._pIO, self._pL, self._pPS))
+
+    def _step_autoreset_call(self, ws):
+        if self._PS is None:
+            check(self._lib.mdg_step_autoreset(self._pP, self._pR, self._pS, self._pIO, self._pL, self.k, 1,
+                                               ws.data_ptr(), ws.numel()))
+        else:
+            check(self._lib.mdg_step_autoreset_sets(self._pP, self._pR, self._pS, self._pIO, self._pL, self.k, 1,
+                                                    ws.data_ptr(), ws.numel(), self._pPS))
 
     def step_actions(self, actions, *, action_atoms, unit_size, normals=None, uniforms=None, auto_reset=False):
         """``env.step(agent.action_to_transaction(actions))`` in one launch: ``actions`` is an (N, nA) integer tensor
@@ -414,12 +524,11 @@ class Env:
                 L.action_atoms, L.unit_size = int(action_atoms), float(unit_size)
                 if auto_reset and keep is None:
                     ws = _reset_workspace(self._lib, self.P, self.N, self.k, self.device, self._stream_ptr, self._stream)
-                    check(self._lib.mdg_step_autoreset(self._pP, self._pR, self._pS, self._pIO, self._pL, self.k, 1,
-                                                       ws.data_ptr(), ws.numel()))
+                    self._step_autoreset_call(ws)
                     self.launches += 1  # + the refill kernel
                     auto_reset = False
                 else:
-                    check(self._lib.mdg_step(self._pP, self._pR, self._pS, self._pIO, self._pL))
+                    self._step_call()
             finally:
                 io.actions = None
             self.head = L.head
@@ -470,12 +579,11 @@ class Env:
                 self.head = head0
                 if auto_reset and keep is None:
                     ws = _reset_workspace(self._lib, self.P, self.N, self.k, self.device, self._stream_ptr, self._stream)
-                    check(self._lib.mdg_step_autoreset(self._pP, self._pR, self._pS, self._pIO, self._pL, self.k, 1,
-                                                       ws.data_ptr(), ws.numel()))
+                    self._step_autoreset_call(ws)
                     self.launches += 1  # + the refill kernel
                     auto_reset = False
                 else:
-                    check(self._lib.mdg_step(self._pP, self._pR, self._pS, self._pIO, self._pL))
+                    self._step_call()
             finally:
                 io.weights = None
             self.head = L.head
@@ -704,11 +812,15 @@ class Env:
     def state_dict(self):
         """Checkpoint of the env (the reference cannot checkpoint its env: wall-clock seeded RNG)."""
         sd = {k_: v.clone() for k_, v in self.t.items() if k_ not in self._STAGING}
+        if self._PS is not None:
+            sd["param_table"] = self._ptab.clone()  # [nA][NPARAM][S] storage
+            sd["param_set"] = self._pset.clone()
         sd["_meta"] = dict(head=self.head, n_valid=self.n_valid, gstep=self._gstep, seed=self.seed,
                            env_offset=self.env_offset, n_envs=self.N, n_assets=self.nA, window=self.k,
                            nstep=int(self.R.nstep), ra=self.ra, shaper=int(self.R.shaper),
                            margins=(self.P.required_margin, self.P.maintenance_margin),
-                           costs=(self.P.tcost_rel, self.P.tcost_abs, self.P.slippage_rel, self.P.slippage_abs))
+                           costs=(self.P.tcost_rel, self.P.tcost_abs, self.P.slippage_rel, self.P.slippage_abs),
+                           n_sets=self.n_param_sets)
         return sd
 
     def load_state_dict(self, sd):
@@ -718,6 +830,12 @@ class Env:
         for k_, v in mine.items():
             if k_ in m and m[k_] != v:
                 raise ValueError(f"checkpoint was taken from an Env with {k_}={m[k_]}, this one has {k_}={v}")
+        if m.get("n_sets", 0) != self.n_param_sets:
+            raise ValueError(f"checkpoint was taken from an Env with {m.get('n_sets', 0)} parameter sets, this one has "
+                             f"{self.n_param_sets}")
+        if self._PS is not None:
+            self._ptab.copy_(sd["param_table"])
+            self._pset.copy_(sd["param_set"])
         for k_, v in sd.items():
             if k_ == "_meta" or k_ in self._STAGING or k_ not in self.t:
                 continue
