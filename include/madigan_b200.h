@@ -28,9 +28,10 @@
 extern "C" {
 #endif
 
-#define MDG_ABI_VERSION 15
+#define MDG_ABI_VERSION 16
 #define MDG_MAX_ASSETS 16
 #define MDG_GEN_NPARAM 10
+#define MDG_BROKER_NPARAM 7 /* broker settings per set (MdgBrokerSlot): rows of a broker table */
 #define MDG_MAX_NSTEP 64
 #define MDG_MAX_SINE_COMPONENTS 16 /* 3 random bools per component share one 53-bit uniform */
 #define MDG_MAX_SINE_TRENDS 4
@@ -320,7 +321,8 @@ int mdg_init_state(const MdgParams *params, const MdgReward *reward, const MdgSt
 
 /* ---------------------------------------------------------------------------------------------------
  * Generator parameter sets: the envs of one slab tick different markets (a sweep over settings, or a distribution of
- * markets for robust training) with the same types, roles, slots and broker settings.
+ * markets for robust training) with the same types, roles and slots; broker settings per set: the _sets_broker
+ * launches below.
  *
  * A parameter set is one value for every p[j] slot (MDG_GEN_NPARAM) of every asset.  The table holds n_sets >= 1 of
  * them, set-minor: p[(i * MDG_GEN_NPARAM + j) * n_sets + s] is slot j of asset i in set s, so that a warp's reads
@@ -356,12 +358,51 @@ int mdg_reset_ws_sets(const MdgParams *params, const MdgState *state, const MdgS
 int mdg_init_state_sets(const MdgParams *params, const MdgReward *reward, const MdgState *state,
                         const MdgLaunch *launch, const MdgParamSets *sets);
 
+/* ---------------------------------------------------------------------------------------------------
+ * Broker sets: the seven broker settings of MdgParams per parameter set, so that the envs of one slab also trade under
+ * different frictions (costs, slippage, margins, starting cash).
+ *
+ * The broker table is device memory [MDG_BROKER_NPARAM][n_sets], set-minor like MdgParamSets.p:
+ * broker[k * n_sets + s] is slot k (MdgBrokerSlot, MdgParams field order) of set s.  It is indexed by the same
+ * sets->set_of_env, with the same unsigned clamp to n_sets - 1.  With a broker table, every read of one of the seven
+ * MdgParams fields by the step, refill, constructor and derived-accounting kernels reads the env's entry instead, and
+ * the step kernel's risk-gate constants are computed per env with the same expressions as from MdgParams.  So env e
+ * of such a launch is bit for bit env e of a launch without sets whose MdgParams hold the generator slots and the
+ * broker settings of set s.  The values are not range-checked (neither are the MdgParams fields): any value, NaN
+ * included, behaves per env as the same value does in MdgParams.  The table is read by each launch on its stream, as
+ * the parameter-set table is.
+ * broker == NULL: exactly the corresponding _sets launch (mdg_derived_sets_broker: mdg_derived).  NULL sets or
+ * n_sets < 1: MDG_E_INVALID; a SINE* asset: MDG_E_UNSUPPORTED; mdg_reset_ws_sets_broker requires a workspace. */
+enum MdgBrokerSlot {
+  MDG_BROKER_INIT_CASH = 0,
+  MDG_BROKER_REQUIRED_MARGIN = 1,
+  MDG_BROKER_MAINTENANCE_MARGIN = 2,
+  MDG_BROKER_SLIPPAGE_REL = 3,
+  MDG_BROKER_SLIPPAGE_ABS = 4,
+  MDG_BROKER_TCOST_REL = 5,
+  MDG_BROKER_TCOST_ABS = 6
+};
+int mdg_step_sets_broker(const MdgParams *params, const MdgReward *reward, const MdgState *state,
+                         const MdgStepIO *io, const MdgLaunch *launch, const MdgParamSets *sets, const double *broker);
+int mdg_step_autoreset_sets_broker(const MdgParams *params, const MdgReward *reward, const MdgState *state,
+                                   const MdgStepIO *io, const MdgLaunch *launch, int fill_ticks, int clear_nstep,
+                                   void *workspace, int64_t workspace_bytes, const MdgParamSets *sets,
+                                   const double *broker);
+int mdg_reset_ws_sets_broker(const MdgParams *params, const MdgState *state, const MdgStepIO *io,
+                             const MdgLaunch *launch, const uint8_t *mask, int fill_ticks, int clear_nstep,
+                             void *workspace, int64_t workspace_bytes, const MdgParamSets *sets, const double *broker);
+int mdg_init_state_sets_broker(const MdgParams *params, const MdgReward *reward, const MdgState *state,
+                               const MdgLaunch *launch, const MdgParamSets *sets, const double *broker);
+
 /* Recompute MdgState.folds from the state tensors (after external writes into them). */
 int mdg_refresh_folds(const MdgParams *params, const MdgState *state, const MdgLaunch *launch);
 
 /* Portfolio's derived accounting for every env. */
 int mdg_derived(const MdgParams *params, const MdgState *state, const MdgDerived *out,
                 const MdgLaunch *launch);
+/* ... with broker sets: required_margin and maintenance_margin of every env from its set (see MdgBrokerSlot) */
+int mdg_derived_sets_broker(const MdgParams *params, const MdgState *state, const MdgDerived *out,
+                            const MdgLaunch *launch, const MdgParamSets *sets, const double *broker);
 
 /* StackerDiscrete.current_data price window (preprocessor.py:183-189) with the
  * normalisers of preprocessor.py:53-107: ring [k][F][N] -> out (N,k,F) or (N,F,k).

@@ -5,12 +5,13 @@ checks the struct sizes against the compiled library (``mdg_sizeof``).
 """
 import ctypes as C
 
-MDG_ABI_VERSION = 15
+MDG_ABI_VERSION = 16
 FLAG_FORCE_EXACT_GATE = 1
 FLAG_GENERIC_FILL = 2
 XFORM_NONE, XFORM_PAIR_RATIO, XFORM_RETURNS = 0, 1, 2
 MDG_MAX_ASSETS = 16
 MDG_GEN_NPARAM = 10
+MDG_BROKER_NPARAM = 7  # broker table rows, MdgParams field order (data_source.BROKER_SLOTS)
 MDG_MAX_NSTEP = 64
 MDG_MAX_SINE_COMPONENTS = 16
 MDG_MAX_SINE_TRENDS = 4
@@ -165,8 +166,19 @@ SYMBOLS = {
     "mdg_reset_ws_sets": (C.c_int, [_P(MdgParams), _P(MdgState), _P(MdgStepIO), _P(MdgLaunch), C.c_void_p,
                                     C.c_int, C.c_int, C.c_void_p, C.c_int64, _P(MdgParamSets)]),
     "mdg_init_state_sets": (C.c_int, [_P(MdgParams), _P(MdgReward), _P(MdgState), _P(MdgLaunch), _P(MdgParamSets)]),
+    "mdg_step_sets_broker": (C.c_int, [_P(MdgParams), _P(MdgReward), _P(MdgState), _P(MdgStepIO), _P(MdgLaunch),
+                                       _P(MdgParamSets), C.c_void_p]),
+    "mdg_step_autoreset_sets_broker": (C.c_int, [_P(MdgParams), _P(MdgReward), _P(MdgState), _P(MdgStepIO),
+                                                 _P(MdgLaunch), C.c_int, C.c_int, C.c_void_p, C.c_int64,
+                                                 _P(MdgParamSets), C.c_void_p]),
+    "mdg_reset_ws_sets_broker": (C.c_int, [_P(MdgParams), _P(MdgState), _P(MdgStepIO), _P(MdgLaunch), C.c_void_p,
+                                           C.c_int, C.c_int, C.c_void_p, C.c_int64, _P(MdgParamSets), C.c_void_p]),
+    "mdg_init_state_sets_broker": (C.c_int, [_P(MdgParams), _P(MdgReward), _P(MdgState), _P(MdgLaunch),
+                                             _P(MdgParamSets), C.c_void_p]),
     "mdg_refresh_folds": (C.c_int, [_P(MdgParams), _P(MdgState), _P(MdgLaunch)]),
     "mdg_derived": (C.c_int, [_P(MdgParams), _P(MdgState), _P(MdgDerived), _P(MdgLaunch)]),
+    "mdg_derived_sets_broker": (C.c_int, [_P(MdgParams), _P(MdgState), _P(MdgDerived), _P(MdgLaunch),
+                                          _P(MdgParamSets), C.c_void_p]),
     "mdg_materialise_window": (C.c_int, [_P(MdgWindow)]),
     "mdg_replay_append": (C.c_int, [_P(MdgReplay), C.c_int64, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p,
                                     C.c_void_p, C.c_void_p, C.c_void_p]),

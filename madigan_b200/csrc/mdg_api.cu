@@ -169,6 +169,10 @@ struct ResetWsArgs {
 struct ResetWsSetsArgs : ResetWsArgs {
   MdgParamSets ps;
 };
+// ... with broker sets: the broker table, [MDG_BROKER_NPARAM][n_sets]
+struct ResetWsBrokerArgs : ResetWsSetsArgs {
+  const double* broker;
+};
 
 __global__ void __launch_bounds__(256) reset_scan_kernel(const __grid_constant__ ResetWsArgs a) {
   const int64_t N = a.L.n_envs;
@@ -185,7 +189,7 @@ __global__ void __launch_bounds__(256) reset_scan_kernel(const __grid_constant__
 
 constexpr int kFillBlock = 128;
 
-template <bool SETS>
+template <bool SETS, bool BROKER = false>
 __device__ __forceinline__ void reset_fill_body(const ResetWsArgs& a) {
   extern __shared__ double zs[];  // [chunk][n_normals]
   const MdgParams& P = a.P;
@@ -194,9 +198,9 @@ __device__ __forceinline__ void reset_fill_body(const ResetWsArgs& a) {
   const int fill = a.fill_ticks, k = a.L.window, chunk = a.chunk, nlead = a.n_groups;
   const int64_t N = a.L.n_envs;
   const int count = *(volatile int*)a.count;
-  const double cash = P.init_cash;
-  const double eq = cash + 0. - 0.;              // flat portfolio: equity == cash
-  const bool eq_plain = eq > 0. && eq < 1e300;   // then (0*p)/eq == 0*p exactly
+  const double cash0 = P.init_cash;
+  const double eq0 = cash0 + 0. - 0.;              // flat portfolio: equity == cash
+  const bool eq_plain0 = eq0 > 0. && eq0 < 1e300;  // then (0*p)/eq == 0*p exactly
   const uint32_t k0 = (uint32_t)a.L.seed, k1 = (uint32_t)(a.L.seed >> 32);
   const uint32_t magic = (uint32_t)((0x100000000ull + (uint32_t)nb - 1) / (uint32_t)(nb > 0 ? nb : 1));  // ceil(2^32 / nb)
   for (int d = blockIdx.x; d < count; d += gridDim.x) {
@@ -204,6 +208,14 @@ __device__ __forceinline__ void reset_fill_body(const ResetWsArgs& a) {
     const long long ts0 = a.S.timestamp[e];
     int64_t set = 0;  // parameter sets: the listed env's set
     if constexpr (SETS) set = env_set(static_cast<const ResetWsSetsArgs&>(a).ps, e);
+    double cash = cash0, eq = eq0;
+    bool eq_plain = eq_plain0;
+    if constexpr (BROKER) {  // the fresh portfolio's cash from the listed env's set
+      const ResetWsBrokerArgs& b = static_cast<const ResetWsBrokerArgs&>(a);
+      cash = broker_value(b.broker, b.ps.n_sets, set, MDG_BROKER_INIT_CASH);
+      eq = cash + 0. - 0.;
+      eq_plain = eq > 0. && eq < 1e300;
+    }
     __syncthreads();  // every thread has read the old timestamp (and the previous env's normals are consumed)
     if (tid == 32) {  // fresh Broker/Account/Portfolio (Env.h:150-165): per-env scalars
       if (a.clear_nstep && a.S.nstep_len) a.S.nstep_len[e] = 0;  // offpolicy_q.py:94
@@ -347,6 +359,9 @@ __global__ void __launch_bounds__(kFillBlock) reset_fill_kernel(const __grid_con
 __global__ void __launch_bounds__(kFillBlock) reset_fill_sets_kernel(const __grid_constant__ ResetWsSetsArgs a) {
   reset_fill_body<true>(a);
 }
+__global__ void __launch_bounds__(kFillBlock) reset_fill_sets_broker_kernel(const __grid_constant__ ResetWsBrokerArgs a) {
+  reset_fill_body<true, true>(a);
+}
 
 // The refill of the all-OU-pairs parameter sets (all_ou_pairs(P)) when the normals come from Philox: one lane per
 // (listed env, pair), np = nA/2 lanes per env, 128/np envs per block.  A pair is an independent process whose three
@@ -365,7 +380,7 @@ __global__ void __launch_bounds__(kFillBlock) reset_fill_sets_kernel(const __gri
 #define MDG_FILL_PAIRS_MINB 1
 #endif
 constexpr int kFillPairsUnroll = MDG_FILL_PAIRS_UNROLL;
-template <bool SETS>
+template <bool SETS, bool BROKER = false>
 __device__ __forceinline__ void reset_fill_pairs_body(const ResetWsArgs& a) {
   const MdgParams& P = a.P;
   const int tid = threadIdx.x;
@@ -375,9 +390,9 @@ __device__ __forceinline__ void reset_fill_pairs_body(const ResetWsArgs& a) {
   const int64_t N = a.L.n_envs;
   const int listed = *(volatile int*)a.count;
   const int count = (int64_t)listed < N ? listed : (int)N;  // a stale header cannot index past the list
-  const double cash = P.init_cash;
-  const double eq = cash + 0. - 0.;              // flat portfolio: equity == cash
-  const bool eq_plain = eq > 0. && eq < 1e300;   // then (0*p)/eq == 0*p exactly
+  const double cash0 = P.init_cash;
+  const double eq0 = cash0 + 0. - 0.;              // flat portfolio: equity == cash
+  const bool eq_plain0 = eq0 > 0. && eq0 < 1e300;  // then (0*p)/eq == 0*p exactly
   const uint32_t k0 = (uint32_t)a.L.seed, k1 = (uint32_t)(a.L.seed >> 32);
   const int i0 = 2 * p;
   const MdgAssetGen &g0 = P.gen[i0], &g1 = P.gen[i0 + 1];
@@ -390,11 +405,18 @@ __device__ __forceinline__ void reset_fill_pairs_body(const ResetWsArgs& a) {
     const bool active = slot < epb && d < count;
     const int64_t e = active ? a.list[d] : 0;
     const long long ts0 = active ? a.S.timestamp[e] : 0;
+    double cash = cash0, eq = eq0;
+    bool eq_plain = eq_plain0;
     if constexpr (SETS) {  // this lane's pair in the listed env's set (idle lanes read env 0's, and store nothing)
       const MdgParamSets& ps = static_cast<const ResetWsSetsArgs&>(a).ps;
       const int64_t set = env_set(ps, e);
       const SetParams q0 = set_params(ps, set, i0), q1 = set_params(ps, set, i0 + 1);
       theta0 = q0[0]; phi0 = q0[1]; noise = q0[2]; theta1 = q1[0]; phi1 = q1[1];
+      if constexpr (BROKER) {  // the fresh portfolio's cash from the set too
+        cash = broker_value(static_cast<const ResetWsBrokerArgs&>(a).broker, ps.n_sets, set, MDG_BROKER_INIT_CASH);
+        eq = cash + 0. - 0.;
+        eq_plain = eq > 0. && eq < 1e300;
+      }
     }
     __syncthreads();  // every lane of an env has read the old timestamp before its pair-0 lane writes the new one
     // idle lanes run the tick loop too (without storing): the loop's shuffles take every lane of the warp
@@ -481,6 +503,10 @@ __global__ void __launch_bounds__(kFillBlock, MDG_FILL_PAIRS_MINB)
     reset_fill_pairs_sets_kernel(const __grid_constant__ ResetWsSetsArgs a) {
   reset_fill_pairs_body<true>(a);
 }
+__global__ void __launch_bounds__(kFillBlock, MDG_FILL_PAIRS_MINB)
+    reset_fill_pairs_sets_broker_kernel(const __grid_constant__ ResetWsBrokerArgs a) {
+  reset_fill_pairs_body<true, true>(a);
+}
 
 // constructor state (Env.h:139-165 before the first tick)
 struct InitArgs {
@@ -492,8 +518,11 @@ struct InitArgs {
 struct InitSetsArgs : InitArgs {
   MdgParamSets ps;
 };
+struct InitBrokerArgs : InitSetsArgs {
+  const double* broker;
+};
 // e: computed in the kernels, where the compiler knows the range of threadIdx.x
-template <bool SETS>
+template <bool SETS, bool BROKER = false>
 __device__ __forceinline__ void init_body(const InitArgs& a, int64_t e) {
   const int64_t N = a.L.n_envs;
   if (e >= N) return;
@@ -512,12 +541,17 @@ __device__ __forceinline__ void init_body(const InitArgs& a, int64_t e) {
     a.S.mean_entry[(int64_t)i * N + e] = 0.;
     a.S.borrowed[(int64_t)i * N + e] = 0.;
   }
-  a.S.cash[e] = a.P.init_cash;
+  double cash = a.P.init_cash;
+  if constexpr (BROKER) {  // the env's set's starting cash
+    const InitBrokerArgs& b = static_cast<const InitBrokerArgs&>(a);
+    cash = broker_value(b.broker, b.ps.n_sets, env_set(b.ps, e), MDG_BROKER_INIT_CASH);
+  }
+  a.S.cash[e] = cash;
   a.S.timestamp[e] = 0;
   if (a.S.reset_ts) a.S.reset_ts[e] = 0;
   if (a.S.folds) {
     for (int r = 0; r < 4; ++r) a.S.folds[(int64_t)r * N + e] = 0.;
-    a.S.folds[(int64_t)MDG_FOLD_G * N + e] = fabs(a.P.init_cash);
+    a.S.folds[(int64_t)MDG_FOLD_G * N + e] = fabs(cash);
   }
   const int ra = a.R.reduce_rewards ? 1 : na;
   for (int c = 0; c < ra; ++c) {
@@ -531,6 +565,9 @@ __global__ void __launch_bounds__(128) init_kernel(const __grid_constant__ InitA
 }
 __global__ void __launch_bounds__(128) init_sets_kernel(const __grid_constant__ InitSetsArgs a) {
   init_body<true>(a, (int64_t)blockIdx.x * 128 + threadIdx.x);
+}
+__global__ void __launch_bounds__(128) init_sets_broker_kernel(const __grid_constant__ InitBrokerArgs a) {
+  init_body<true, true>(a, (int64_t)blockIdx.x * 128 + threadIdx.x);
 }
 
 // exact left-to-right folds of the portfolio as stored (after external writes into the state tensors)
@@ -585,23 +622,13 @@ static int check_common(const MdgParams* P, const MdgLaunch* L) {
   return MDG_OK;
 }
 
-// parameter sets: a table and an assignment, and only generators whose p slots are plain numbers
-static int check_sets(const MdgParams* P, const MdgParamSets* ps) {
-  if (!ps) return set_err(MDG_E_INVALID, "null parameter sets");
-  if (ps->n_sets < 1) return set_err(MDG_E_INVALID, "parameter sets: n_sets < 1");
-  if (!ps->p || !ps->set_of_env) return set_err(MDG_E_INVALID, "parameter sets: null table / set_of_env");
-  for (int i = 0; i < P->n_assets; ++i)
-    if (P->gen[i].type >= MDG_GEN_SINEADDER)
-      return set_err(MDG_E_UNSUPPORTED, "parameter sets do not support SINE* generators");
-  return MDG_OK;
-}
-
 }  // namespace mdg
 
 using namespace mdg;
 
 static int step_impl(const MdgParams* P, const MdgReward* R, const MdgState* S, const MdgStepIO* IO,
-                     const MdgLaunch* L, int* done_count, int* done_list, const MdgParamSets* sets = nullptr) {
+                     const MdgLaunch* L, int* done_count, int* done_list, const MdgParamSets* sets = nullptr,
+                     const double* broker = nullptr) {
   int rc = check_common(P, L);
   if (rc) return rc;
   if (!S || !IO) return set_err(MDG_E_INVALID, "null state/io");
@@ -635,10 +662,12 @@ static int step_impl(const MdgParams* P, const MdgReward* R, const MdgState* S, 
   a.done_count = done_count;
   a.done_list = done_list;
   if (!sets) return launch_step(a);
-  StepSetsArgs b;
+  StepSetsBrokerArgs b;
   static_cast<StepArgs&>(b) = a;
   b.ps = *sets;
-  return launch_step<true>(b);
+  b.broker = broker;
+  if (!broker) return launch_step<true>(static_cast<StepSetsArgs&>(b));
+  return launch_step<true, true>(b);
 }
 
 extern "C" int mdg_step(const MdgParams* P, const MdgReward* R, const MdgState* S, const MdgStepIO* IO,
@@ -646,13 +675,18 @@ extern "C" int mdg_step(const MdgParams* P, const MdgReward* R, const MdgState* 
   return step_impl(P, R, S, IO, L, nullptr, nullptr);
 }
 
-extern "C" int mdg_step_sets(const MdgParams* P, const MdgReward* R, const MdgState* S, const MdgStepIO* IO,
-                             const MdgLaunch* L, const MdgParamSets* sets) {
+extern "C" int mdg_step_sets_broker(const MdgParams* P, const MdgReward* R, const MdgState* S, const MdgStepIO* IO,
+                                    const MdgLaunch* L, const MdgParamSets* sets, const double* broker) {
   int rc = check_common(P, L);
   if (rc) return rc;
   rc = check_sets(P, sets);
   if (rc) return rc;
-  return step_impl(P, R, S, IO, L, nullptr, nullptr, sets);
+  return step_impl(P, R, S, IO, L, nullptr, nullptr, sets, broker);
+}
+
+extern "C" int mdg_step_sets(const MdgParams* P, const MdgReward* R, const MdgState* S, const MdgStepIO* IO,
+                             const MdgLaunch* L, const MdgParamSets* sets) {
+  return mdg_step_sets_broker(P, R, S, IO, L, sets, nullptr);
 }
 
 extern "C" int mdg_reset(const MdgParams* P, const MdgState* S, const MdgStepIO* IO, const MdgLaunch* L,
@@ -728,8 +762,8 @@ constexpr int kFillPairsBlocksPerSm = 2;
 // spreads an env's draws over a block (~12 us).  With few pairs per env that latency is not paid back: one OU pair per
 // env (C3, 65,536 envs, one stream) measured 20.5 us per step with the generic refill, 34.9 with this one.
 constexpr int kFillPairsMinAssets = 8;
-// Args: ResetWsArgs, or ResetWsSetsArgs with SETS (the same kernel choice)
-template <bool SETS = false, class Args = ResetWsArgs>
+// Args: ResetWsArgs, ResetWsSetsArgs with SETS, or ResetWsBrokerArgs with SETS and BROKER (the same kernel choice)
+template <bool SETS = false, bool BROKER = false, class Args = ResetWsArgs>
 static int launch_fill(const Args& a, int64_t max_listed) {
   // the count is on the device: size the grid for the most the list can hold, capped at a few blocks per SM
   // (grid-stride; blocks past the end of the list only read the count and take their exit ticket)
@@ -746,14 +780,16 @@ static int launch_fill(const Args& a, int64_t max_listed) {
     const int64_t groups = (max_listed + epb - 1) / epb;
     const int64_t cap = knob ? knob : kFillPairsBlocksPerSm * sm_count();
     const unsigned grid = (unsigned)(groups < cap ? (groups > 0 ? groups : 1) : cap);
-    if constexpr (SETS) reset_fill_pairs_sets_kernel<<<grid, kFillBlock, 0, st>>>(a);
+    if constexpr (BROKER) reset_fill_pairs_sets_broker_kernel<<<grid, kFillBlock, 0, st>>>(a);
+    else if constexpr (SETS) reset_fill_pairs_sets_kernel<<<grid, kFillBlock, 0, st>>>(a);
     else reset_fill_pairs_kernel<<<grid, kFillBlock, 0, st>>>(a);
     return cuda_err(cudaGetLastError(), "reset_fill_pairs launch");
   }
   const int64_t cap = knob ? knob : 148 * 8;
   const unsigned grid = (unsigned)(max_listed < cap ? (max_listed > 0 ? max_listed : 1) : cap);
   const size_t smem = sizeof(double) * (size_t)a.chunk * (size_t)(a.P.n_normals > 0 ? a.P.n_normals : 1);
-  if constexpr (SETS) reset_fill_sets_kernel<<<grid, kFillBlock, smem, st>>>(a);
+  if constexpr (BROKER) reset_fill_sets_broker_kernel<<<grid, kFillBlock, smem, st>>>(a);
+  else if constexpr (SETS) reset_fill_sets_kernel<<<grid, kFillBlock, smem, st>>>(a);
   else reset_fill_kernel<<<grid, kFillBlock, smem, st>>>(a);
   return cuda_err(cudaGetLastError(), "reset_fill launch");
 }
@@ -761,7 +797,7 @@ static int launch_fill(const Args& a, int64_t max_listed) {
 
 static int reset_ws_impl(const MdgParams* P, const MdgState* S, const MdgStepIO* IO, const MdgLaunch* L,
                          const uint8_t* mask, int fill_ticks, int clear_nstep, void* workspace, int64_t workspace_bytes,
-                         const MdgParamSets* sets) {
+                         const MdgParamSets* sets, const double* broker = nullptr) {
   int rc = check_common(P, L);
   if (rc) return rc;
   if (sets && (rc = check_sets(P, sets))) return rc;
@@ -772,7 +808,7 @@ static int reset_ws_impl(const MdgParams* P, const MdgState* S, const MdgStepIO*
   if (fill_ticks > L->window) return set_err(MDG_E_INVALID, "fill_ticks > window");
   const int64_t N = L->n_envs;
   if (N == 0) return MDG_OK;
-  ResetWsSetsArgs a;
+  ResetWsBrokerArgs a;
   rc = fill_ws_args(a, P, S, IO, L, fill_ticks, clear_nstep, workspace, workspace_bytes);
   if (rc) return rc;
   a.mask = mask;
@@ -782,7 +818,9 @@ static int reset_ws_impl(const MdgParams* P, const MdgState* S, const MdgStepIO*
   reset_scan_kernel<<<(unsigned)((N + 255) / 256), 256, 0, st>>>(a);
   if (!sets) return launch_fill(static_cast<const ResetWsArgs&>(a), N);
   a.ps = *sets;
-  return launch_fill<true>(a, N);
+  a.broker = broker;
+  if (!broker) return launch_fill<true>(static_cast<const ResetWsSetsArgs&>(a), N);
+  return launch_fill<true, true>(a, N);
 }
 
 extern "C" int mdg_reset_ws(const MdgParams* P, const MdgState* S, const MdgStepIO* IO, const MdgLaunch* L,
@@ -792,17 +830,24 @@ extern "C" int mdg_reset_ws(const MdgParams* P, const MdgState* S, const MdgStep
   return reset_ws_impl(P, S, IO, L, mask, fill_ticks, clear_nstep, workspace, workspace_bytes, nullptr);
 }
 
+extern "C" int mdg_reset_ws_sets_broker(const MdgParams* P, const MdgState* S, const MdgStepIO* IO,
+                                        const MdgLaunch* L, const uint8_t* mask, int fill_ticks, int clear_nstep,
+                                        void* workspace, int64_t workspace_bytes, const MdgParamSets* sets,
+                                        const double* broker) {
+  if (!sets) return set_err(MDG_E_INVALID, "null parameter sets");
+  if (!workspace) return set_err(MDG_E_INVALID, "mdg_reset_ws_sets needs a workspace");
+  return reset_ws_impl(P, S, IO, L, mask, fill_ticks, clear_nstep, workspace, workspace_bytes, sets, broker);
+}
+
 extern "C" int mdg_reset_ws_sets(const MdgParams* P, const MdgState* S, const MdgStepIO* IO, const MdgLaunch* L,
                                  const uint8_t* mask, int fill_ticks, int clear_nstep, void* workspace,
                                  int64_t workspace_bytes, const MdgParamSets* sets) {
-  if (!sets) return set_err(MDG_E_INVALID, "null parameter sets");
-  if (!workspace) return set_err(MDG_E_INVALID, "mdg_reset_ws_sets needs a workspace");
-  return reset_ws_impl(P, S, IO, L, mask, fill_ticks, clear_nstep, workspace, workspace_bytes, sets);
+  return mdg_reset_ws_sets_broker(P, S, IO, L, mask, fill_ticks, clear_nstep, workspace, workspace_bytes, sets, nullptr);
 }
 
 static int step_autoreset_impl(const MdgParams* P, const MdgReward* R, const MdgState* S, const MdgStepIO* IO,
                                const MdgLaunch* L, int fill_ticks, int clear_nstep, void* workspace,
-                               int64_t workspace_bytes, const MdgParamSets* sets) {
+                               int64_t workspace_bytes, const MdgParamSets* sets, const double* broker = nullptr) {
   int rc = check_common(P, L);
   if (rc) return rc;
   if (sets && (rc = check_sets(P, sets))) return rc;
@@ -812,16 +857,18 @@ static int step_autoreset_impl(const MdgParams* P, const MdgReward* R, const Mdg
   if (fill_ticks < 1) fill_ticks = 1;
   if (fill_ticks > L->window) return set_err(MDG_E_INVALID, "fill_ticks > window");
   if (L->n_envs == 0) return MDG_OK;
-  ResetWsSetsArgs a;
+  ResetWsBrokerArgs a;
   MdgStepIO io = *IO;  // the reset draws from Philox (no injected stream) and takes no units
   io.units = nullptr; io.normals = nullptr; io.uniforms = nullptr; io.actions = nullptr; io.weights = nullptr;
   rc = fill_ws_args(a, P, S, &io, L, fill_ticks, clear_nstep, workspace, workspace_bytes);
   if (rc) return rc;
-  rc = step_impl(P, R, S, IO, L, a.count, a.list, sets);  // the step kernel appends the finished envs to the list
+  rc = step_impl(P, R, S, IO, L, a.count, a.list, sets, broker);  // the step kernel appends the finished envs to the list
   if (rc) return rc;
   if (!sets) return launch_fill(static_cast<const ResetWsArgs&>(a), L->n_envs);
   a.ps = *sets;
-  return launch_fill<true>(a, L->n_envs);
+  a.broker = broker;
+  if (!broker) return launch_fill<true>(static_cast<const ResetWsSetsArgs&>(a), L->n_envs);
+  return launch_fill<true, true>(a, L->n_envs);
 }
 
 extern "C" int mdg_step_autoreset(const MdgParams* P, const MdgReward* R, const MdgState* S, const MdgStepIO* IO,
@@ -830,28 +877,40 @@ extern "C" int mdg_step_autoreset(const MdgParams* P, const MdgReward* R, const 
   return step_autoreset_impl(P, R, S, IO, L, fill_ticks, clear_nstep, workspace, workspace_bytes, nullptr);
 }
 
+extern "C" int mdg_step_autoreset_sets_broker(const MdgParams* P, const MdgReward* R, const MdgState* S,
+                                              const MdgStepIO* IO, const MdgLaunch* L, int fill_ticks, int clear_nstep,
+                                              void* workspace, int64_t workspace_bytes, const MdgParamSets* sets,
+                                              const double* broker) {
+  if (!sets) return set_err(MDG_E_INVALID, "null parameter sets");
+  return step_autoreset_impl(P, R, S, IO, L, fill_ticks, clear_nstep, workspace, workspace_bytes, sets, broker);
+}
+
 extern "C" int mdg_step_autoreset_sets(const MdgParams* P, const MdgReward* R, const MdgState* S, const MdgStepIO* IO,
                                        const MdgLaunch* L, int fill_ticks, int clear_nstep, void* workspace,
                                        int64_t workspace_bytes, const MdgParamSets* sets) {
-  if (!sets) return set_err(MDG_E_INVALID, "null parameter sets");
-  return step_autoreset_impl(P, R, S, IO, L, fill_ticks, clear_nstep, workspace, workspace_bytes, sets);
+  return mdg_step_autoreset_sets_broker(P, R, S, IO, L, fill_ticks, clear_nstep, workspace, workspace_bytes, sets,
+                                        nullptr);
 }
 
 static int init_state_impl(const MdgParams* P, const MdgReward* R, const MdgState* S, const MdgLaunch* L,
-                           const MdgParamSets* sets) {
+                           const MdgParamSets* sets, const double* broker = nullptr) {
   int rc = check_common(P, L);
   if (rc) return rc;
   if (sets && (rc = check_sets(P, sets))) return rc;
   if (!S) return set_err(MDG_E_INVALID, "null state");
   if (L->n_envs == 0) return MDG_OK;
-  InitSetsArgs a;
+  InitBrokerArgs a;
   a.P = *P;
   if (R) a.R = *R; else { memset(&a.R, 0, sizeof(a.R)); a.R.nstep = 1; }
   a.S = *S; a.L = *L;
   const unsigned grid = (unsigned)((L->n_envs + 128 - 1) / 128);
-  if (sets) {
+  if (sets && broker) {
     a.ps = *sets;
-    init_sets_kernel<<<grid, 128, 0, (cudaStream_t)L->stream>>>(a);
+    a.broker = broker;
+    init_sets_broker_kernel<<<grid, 128, 0, (cudaStream_t)L->stream>>>(a);
+  } else if (sets) {
+    a.ps = *sets;
+    init_sets_kernel<<<grid, 128, 0, (cudaStream_t)L->stream>>>(static_cast<const InitSetsArgs&>(a));
   } else {
     init_kernel<<<grid, 128, 0, (cudaStream_t)L->stream>>>(static_cast<const InitArgs&>(a));
   }
@@ -862,10 +921,15 @@ extern "C" int mdg_init_state(const MdgParams* P, const MdgReward* R, const MdgS
   return init_state_impl(P, R, S, L, nullptr);
 }
 
+extern "C" int mdg_init_state_sets_broker(const MdgParams* P, const MdgReward* R, const MdgState* S,
+                                          const MdgLaunch* L, const MdgParamSets* sets, const double* broker) {
+  if (!sets) return set_err(MDG_E_INVALID, "null parameter sets");
+  return init_state_impl(P, R, S, L, sets, broker);
+}
+
 extern "C" int mdg_init_state_sets(const MdgParams* P, const MdgReward* R, const MdgState* S, const MdgLaunch* L,
                                    const MdgParamSets* sets) {
-  if (!sets) return set_err(MDG_E_INVALID, "null parameter sets");
-  return init_state_impl(P, R, S, L, sets);
+  return mdg_init_state_sets_broker(P, R, S, L, sets, nullptr);
 }
 
 extern "C" int mdg_refresh_folds(const MdgParams* P, const MdgState* S, const MdgLaunch* L) {

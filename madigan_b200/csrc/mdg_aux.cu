@@ -27,10 +27,15 @@ struct DerivedArgs {
   MdgDerived D;
   int64_t N;
 };
+// ... with broker sets: the margins of every env from its set
+struct DerivedBrokerArgs : DerivedArgs {
+  MdgParamSets ps;
+  const double* broker;
+};
 
-__global__ void __launch_bounds__(kBlockA) derived_kernel(const __grid_constant__ DerivedArgs a) {
+template <bool BROKER>
+__device__ __forceinline__ void derived_body(const DerivedArgs& a, int64_t e) {
   const int64_t N = a.N;
-  const int64_t e = (int64_t)blockIdx.x * kBlockA + threadIdx.x;
   if (e >= N) return;
   const int na = a.P.n_assets;
   const MdgState& S = a.S;
@@ -57,11 +62,18 @@ __global__ void __launch_bounds__(kBlockA) derived_kernel(const __grid_constant_
   if (D.asset_value) D.asset_value[e] = av;
   if (D.pnl) D.pnl[e] = pnl;
   if (D.balance) D.balance[e] = balance;
-  if (D.available_margin) D.available_margin[e] = (balance + pnl) / a.P.required_margin;  // :229-231
-  if (D.used_margin) D.used_margin[e] = a.P.required_margin * um;                          // :199-201
+  double reqM = a.P.required_margin, maintM = a.P.maintenance_margin;
+  if constexpr (BROKER) {
+    const DerivedBrokerArgs& b = static_cast<const DerivedBrokerArgs&>(a);
+    const int64_t set = env_set(b.ps, e);
+    reqM = broker_value(b.broker, b.ps.n_sets, set, MDG_BROKER_REQUIRED_MARGIN);
+    maintM = broker_value(b.broker, b.ps.n_sets, set, MDG_BROKER_MAINTENANCE_MARGIN);
+  }
+  if (D.available_margin) D.available_margin[e] = (balance + pnl) / reqM;  // :229-231
+  if (D.used_margin) D.used_margin[e] = reqM * um;                          // :199-201
   if (D.borrowed_margin) D.borrowed_margin[e] = bms;
   if (D.borrowed_asset_value) D.borrowed_asset_value[e] = bav;  // :219-223
-  if (D.risk) D.risk[e] = margin_call(cash, av, ml, bms, se, a.P.maintenance_margin) ? MDG_RISK_MARGIN_CALL : MDG_RISK_GREEN;
+  if (D.risk) D.risk[e] = margin_call(cash, av, ml, bms, se, maintM) ? MDG_RISK_MARGIN_CALL : MDG_RISK_GREEN;
   const double w0 = (cash - bms) / equity;
   // abs-normalisers: sum |.| left to right (:144-148, :164-168)
   double sabs = 0., sabs_full = fabs(w0);
@@ -89,6 +101,12 @@ __global__ void __launch_bounds__(kBlockA) derived_kernel(const __grid_constant_
     if (D.position_values_full) D.position_values_full[(int64_t)(j + 1) * N + e] = pv;  // :174-178
     if (D.ledger_full) D.ledger_full[(int64_t)(j + 1) * N + e] = l;                      // :157-161
   }
+}
+__global__ void __launch_bounds__(kBlockA) derived_kernel(const __grid_constant__ DerivedArgs a) {
+  derived_body<false>(a, (int64_t)blockIdx.x * kBlockA + threadIdx.x);
+}
+__global__ void __launch_bounds__(kBlockA) derived_broker_kernel(const __grid_constant__ DerivedBrokerArgs a) {
+  derived_body<true>(a, (int64_t)blockIdx.x * kBlockA + threadIdx.x);
 }
 
 // ---------------------------------------------------------------------------
@@ -618,6 +636,23 @@ extern "C" int mdg_derived(const MdgParams* P, const MdgState* S, const MdgDeriv
   a.P = *P; a.S = *S; a.D = *D; a.N = L->n_envs;
   const unsigned grid = (unsigned)((a.N + kBlockA - 1) / kBlockA);
   derived_kernel<<<grid, kBlockA, 0, (cudaStream_t)L->stream>>>(a);
+  return cuda_err(cudaGetLastError(), "mdg_derived launch");
+}
+
+extern "C" int mdg_derived_sets_broker(const MdgParams* P, const MdgState* S, const MdgDerived* D, const MdgLaunch* L,
+                                       const MdgParamSets* sets, const double* broker) {
+  if (!P || !S || !D || !L) return set_err(MDG_E_INVALID, "null argument");
+  if (P->n_assets < 1 || P->n_assets > MDG_MAX_ASSETS) return set_err(MDG_E_UNSUPPORTED, "n_assets out of range");
+  const int rc = check_sets(P, sets);
+  if (rc) return rc;
+  if (!broker) return mdg_derived(P, S, D, L);
+  if (L->n_envs <= 0) return L->n_envs == 0 ? MDG_OK : set_err(MDG_E_INVALID, "n_envs < 0");
+  DerivedBrokerArgs a;
+  a.P = *P; a.S = *S; a.D = *D; a.N = L->n_envs;
+  a.ps = *sets;
+  a.broker = broker;
+  const unsigned grid = (unsigned)((a.N + kBlockA - 1) / kBlockA);
+  derived_broker_kernel<<<grid, kBlockA, 0, (cudaStream_t)L->stream>>>(a);
   return cuda_err(cudaGetLastError(), "mdg_derived launch");
 }
 

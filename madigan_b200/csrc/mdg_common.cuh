@@ -194,6 +194,21 @@ __device__ __forceinline__ int64_t env_set(const MdgParamSets& ps, int64_t e) {
   const unsigned s = (unsigned)ps.set_of_env[e], last = (unsigned)(ps.n_sets - 1);
   return (int64_t)(s < last ? s : last);
 }
+// broker sets: slot k (MdgBrokerSlot) of set `set` in a broker table, [MDG_BROKER_NPARAM][n_sets] set-minor
+__device__ __forceinline__ double broker_value(const double* __restrict__ broker, int32_t n_sets, int64_t set, int k) {
+  return __ldg(broker + (int64_t)k * n_sets + set);
+}
+
+// parameter sets (host): a table and an assignment, and only generators whose p slots are plain numbers
+static inline int check_sets(const MdgParams* P, const MdgParamSets* ps) {
+  if (!ps) return set_err(MDG_E_INVALID, "null parameter sets");
+  if (ps->n_sets < 1) return set_err(MDG_E_INVALID, "parameter sets: n_sets < 1");
+  if (!ps->p || !ps->set_of_env) return set_err(MDG_E_INVALID, "parameter sets: null table / set_of_env");
+  for (int i = 0; i < P->n_assets; ++i)
+    if (P->gen[i].type >= MDG_GEN_SINEADDER)
+      return set_err(MDG_E_UNSUPPORTED, "parameter sets do not support SINE* generators");
+  return MDG_OK;
+}
 
 // One getData() of asset i (DataSource.cpp).  `price` is the asset's current price
 // (== generator value for every synthetic source), gs points at gstate row gslot for

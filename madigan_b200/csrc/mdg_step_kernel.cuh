@@ -44,6 +44,10 @@ struct StepArgs {
 struct StepSetsArgs : StepArgs {
   MdgParamSets ps;
 };
+// ... and with broker sets (mdg_step_sets_broker): the broker table, [MDG_BROKER_NPARAM][n_sets]
+struct StepSetsBrokerArgs : StepSetsArgs {
+  const double* broker;
+};
 
 constexpr int kBlock = 128;
 
@@ -319,7 +323,48 @@ struct StepAcc {
   bool bad_risk;
 };
 
-struct StepConsts {};  // the gate constants are kernel parameters (StepArgs.c_*); `c` is passed along as a tag
+// The broker settings the step kernel reads, and the risk-gate constants made from them.
+// StepConsts: kernel parameters (MdgParams, and StepArgs.c_* that launch_step computes from it); `c` is only a tag.
+struct StepConsts {
+  __device__ __forceinline__ double init_cash(const StepArgs& a) const { return a.P.init_cash; }
+  __device__ __forceinline__ double reqM(const StepArgs& a) const { return a.c_reqM; }
+  __device__ __forceinline__ double maintM(const StepArgs& a) const { return a.c_maintM; }
+  __device__ __forceinline__ double slip_rel(const StepArgs& a) const { return a.P.slippage_rel; }
+  __device__ __forceinline__ double slip_abs(const StepArgs& a) const { return a.P.slippage_abs; }
+  __device__ __forceinline__ double tcost_rel(const StepArgs& a) const { return a.P.tcost_rel; }
+  __device__ __forceinline__ double tcost_abs(const StepArgs& a) const { return a.P.tcost_abs; }
+  __device__ __forceinline__ int reqM_ok(const StepArgs& a) const { return a.c_reqM_ok; }
+  __device__ __forceinline__ double band_scale(const StepArgs& a) const { return a.c_band_scale; }
+  __device__ __forceinline__ double g1(const StepArgs& a) const { return a.c_g1; }
+  __device__ __forceinline__ double g2(const StepArgs& a) const { return a.c_g2; }
+};
+// BrokerConsts (broker sets): the env's entry of the broker table, loaded next to each use (the table is a few hundred
+// bytes and stays in L1 / L2; only the 32-bit set index is live), and the gate constants computed per env with
+// launch_step's expressions, so that every decision is the one a launch with these values in MdgParams takes
+struct BrokerConsts {
+  uint32_t set;
+  __device__ __forceinline__ double at(const StepArgs& a, int k) const {
+    const StepSetsBrokerArgs& b = static_cast<const StepSetsBrokerArgs&>(a);
+    return broker_value(b.broker, b.ps.n_sets, set, k);
+  }
+  __device__ __forceinline__ double init_cash(const StepArgs& a) const { return at(a, MDG_BROKER_INIT_CASH); }
+  __device__ __forceinline__ double reqM(const StepArgs& a) const { return at(a, MDG_BROKER_REQUIRED_MARGIN); }
+  __device__ __forceinline__ double maintM(const StepArgs& a) const { return at(a, MDG_BROKER_MAINTENANCE_MARGIN); }
+  __device__ __forceinline__ double slip_rel(const StepArgs& a) const { return at(a, MDG_BROKER_SLIPPAGE_REL); }
+  __device__ __forceinline__ double slip_abs(const StepArgs& a) const { return at(a, MDG_BROKER_SLIPPAGE_ABS); }
+  __device__ __forceinline__ double tcost_rel(const StepArgs& a) const { return at(a, MDG_BROKER_TCOST_REL); }
+  __device__ __forceinline__ double tcost_abs(const StepArgs& a) const { return at(a, MDG_BROKER_TCOST_ABS); }
+  __device__ __forceinline__ int reqM_ok(const StepArgs& a) const {
+    const double r = reqM(a);
+    return (r > 0. && r <= 1e6) ? 1 : 0;
+  }
+  __device__ __forceinline__ double band_scale(const StepArgs& a) const {
+    const double r = reqM(a);
+    return 1e-9 * (1. + fabs(maintM(a))) * (r > 1. ? r : 1.);
+  }
+  __device__ __forceinline__ double g1(const StepArgs& a) const { return 6. + 3. * fabs(slip_rel(a)) + fabs(tcost_rel(a)); }
+  __device__ __forceinline__ double g2(const StepArgs& a) const { return 3. * fabs(slip_abs(a)); }
+};
 
 // Broker::handleTransaction(port, i, units) (Broker.cpp:124-142) for one asset whose state is in registers:
 // risk gate (Portfolio.cpp:254-279), slippage/cost (Broker.cpp:171-178), ledger update (Portfolio.cpp:284-323).
@@ -330,12 +375,11 @@ struct StepConsts {};  // the gate constants are kernel parameters (StepArgs.c_*
 // (G = sum of magnitudes); a decision is taken from the running sums only when it clears its threshold by
 // 1e-9 * G.  Otherwise -- a knife-edge, NaN/Inf, a non-positive required margin -- the exact left-to-right
 // folds decide (exact_gate).  Decisions, and therefore ledgers, are bit-identical to the oracle's either way.
-template <bool TX2>
-__device__ __forceinline__ void tx_asset(const StepArgs& a, const StepConsts& c, StepAcc& A, int64_t N, int64_t e,
+template <bool TX2, class C>
+__device__ __forceinline__ void tx_asset(const StepArgs& a, const C& c, StepAcc& A, int64_t N, int64_t e,
                                          int na, int i, double price, double& cur, double& mep, double& bm,
                                          double units, double& tp, double& tu, double& tc, int& risk,
                                          double& prev_val) {
-  const MdgParams& P = a.P;
   const MdgState& S = a.S;
   prev_val = cur * price;  // offpolicy_q.py:141
   tp = 0.; tu = 0.; tc = 0.;
@@ -345,26 +389,26 @@ __device__ __forceinline__ void tx_asset(const StepArgs& a, const StepConsts& c,
     if (!opposite || units > -1 * cur) {  // Portfolio.cpp:257-258: only these orders are gated
       const double amt = fabs(price * (opposite ? units + cur : units));
       const double bal = A.cash + A.rSE, pnl = A.rAV - A.rML, x = bal + pnl;
-      const double band = a.c_band_scale * (A.G + amt);
-      const double d1 = x - amt * a.c_reqM;  // availableMargin <= |amount|  <=>  d1 <= 0
+      const double band = c.band_scale(a) * (A.G + amt);
+      const double d1 = x - amt * c.reqM(a);  // availableMargin <= |amount|  <=>  d1 <= 0
       bool certain;
       int r_fast;
       if constexpr (TX2) {
         // multi-wave variant (168 registers): predicate arithmetic instead of short-circuit branches, the same
         // decisions; 3.5 % faster at 1 M envs, but it costs registers the one-wave variant does not have
-        const double m = a.c_maintM * pnl;
+        const double m = c.maintM(a) * pnl;
         const double d3 = (A.cash + A.rAV - A.rBM) + m, d4 = x + m;  // Portfolio::checkRisk() first (:268), :243-252
         const bool ok1 = (fabs(d1) > band) & (fabs(bal) > band);
         const bool ok2 = (fabs(d3) > band) & (fabs(d4) > band);
-        certain = a.c_reqM_ok & ok1 & (opposite | ok2);
+        certain = c.reqM_ok(a) & ok1 & (opposite | ok2);
         const bool insuff = (d1 <= 0.) | (bal <= 0.);
         const bool mcall = !opposite & ((d3 <= 0.) | (d4 <= 0.));
         r_fast = mcall ? MDG_RISK_MARGIN_CALL : (insuff ? MDG_RISK_INSUFF_MARGIN : MDG_RISK_GREEN);
       } else {
-        certain = a.c_reqM_ok && fabs(d1) > band && fabs(bal) > band;
+        certain = c.reqM_ok(a) && fabs(d1) > band && fabs(bal) > band;
         r_fast = (d1 <= 0. || bal <= 0.) ? MDG_RISK_INSUFF_MARGIN : MDG_RISK_GREEN;
         if (!opposite) {  // Portfolio::checkRisk() first (:268), :243-252
-          const double m = a.c_maintM * pnl;
+          const double m = c.maintM(a) * pnl;
           const double d3 = (A.cash + A.rAV - A.rBM) + m, d4 = x + m;
           certain = certain && fabs(d3) > band && fabs(d4) > band;
           if (d3 <= 0. || d4 <= 0.) r_fast = MDG_RISK_MARGIN_CALL;
@@ -372,13 +416,13 @@ __device__ __forceinline__ void tx_asset(const StepArgs& a, const StepConsts& c,
       }
       risk = (certain && !a.c_force_exact)
                  ? r_fast
-                 : exact_gate(S, N, e, na, A.cash, a.c_reqM, a.c_maintM, i, units, A.pav, A.pml, A.pbm, A.pse);
+                 : exact_gate(S, N, e, na, A.cash, c.reqM(a), c.maintM(a), i, units, A.pav, A.pml, A.pbm, A.pse);
     }
     if (risk == MDG_RISK_GREEN) {
       // Broker::applySlippage / getTransactionCost  Broker.cpp:171-178
-      const double slippage = (price * P.slippage_rel) + P.slippage_abs;
+      const double slippage = (price * c.slip_rel(a)) + c.slip_abs(a);
       const double transactionPrice = units < 0 ? (price - slippage) : (price + slippage);
-      const double transactionCost = fabs(units * price) * P.tcost_rel + P.tcost_abs;
+      const double transactionCost = fabs(units * price) * c.tcost_rel(a) + c.tcost_abs(a);
       tp = transactionPrice; tu = units; tc = transactionCost;
       // Portfolio::handleTransaction  Portfolio.cpp:284-323
       const double o_ml = mep * cur, o_bm = bm;
@@ -394,7 +438,7 @@ __device__ __forceinline__ void tx_asset(const StepArgs& a, const StepConsts& c,
         mep += (transactionPrice - mep) * (units / (units + cur));
       }
       const double amount = transactionPrice * units;
-      const double marginToUse = amount * a.c_reqM;
+      const double marginToUse = amount * c.reqM(a);
       const double marginToBorrow = amount - marginToUse;
       bm += marginToBorrow;
       A.cash -= (marginToUse + transactionCost);
@@ -427,7 +471,7 @@ __device__ __forceinline__ void tx_asset(const StepArgs& a, const StepConsts& c,
       // every new term's magnitude is at most its old magnitude (already in G) plus |units|*(|price|+|tp|), three
       // terms, plus the cost; with |tp| <= |price|(1+|slip_rel|)+|slip_abs| and |cost| <= |units price||tc_rel|+|tc_abs|
       // that is |units| * (|price| * g1 + g2) (+ |tc_abs|, added once per asset in the prologue)
-      A.G += fabs(tu) * (fabs(price) * a.c_g1 + a.c_g2);
+      A.G += fabs(tu) * (fabs(price) * c.g1(a) + c.g2(a));
     } else if (risk != MDG_RISK_INSUFF_MARGIN) {
       A.bad_risk = true;
     }
@@ -555,8 +599,9 @@ __device__ __forceinline__ unsigned long long global_ns() {
 #define MDG_PCLK(slot)
 #endif
 
-template <bool PAIRS, int BS, bool ACTIONS, bool TX2, bool BULK, bool SETS = false>
+template <bool PAIRS, int BS, bool ACTIONS, bool TX2, bool BULK, bool SETS = false, bool BROKER = false>
 __device__ __forceinline__ void step_body(const StepArgs& a) {
+  static_assert(SETS || !BROKER, "broker sets index the parameter sets' assignment");
   MDG_PCLK(0);
 #ifdef MDG_PHASE_CLOCKS
   if (threadIdx.x == 0 && blockIdx.x < 1024) {
@@ -735,7 +780,11 @@ __device__ __forceinline__ void step_body(const StepArgs& a) {
   // availableMargin of the incoming portfolio (Portfolio.cpp:229-231), one scale for every asset
   // (a template parameter: the three extra live values cost 3 % in the units kernel at its 128-register budget)
   const int8_t* arow = (ACTIONS && mode == MDG_MODE_MULTI && a.IO.actions) ? a.IO.actions + e * na : nullptr;
-  const double act_scale = arow ? a.L.unit_size * (((A.cash + A.rSE) + (A.rAV - A.rML)) / P.required_margin) : 0.;
+  const auto c = [&] {  // the broker settings: kernel parameters, or this env's set (BROKER)
+    if constexpr (BROKER) return BrokerConsts{set};
+    else return StepConsts{};
+  }();
+  const double act_scale = arow ? a.L.unit_size * (((A.cash + A.rSE) + (A.rAV - A.rML)) / c.reqM(a)) : 0.;
   const int act_half = a.L.action_atoms / 2;
   // DDPG.action_to_transaction (ddpg.py:182-207), likewise: target weights (cash first) -> units
   const float* wrow = (ACTIONS && mode == MDG_MODE_MULTI && a.IO.weights) ? a.IO.weights + e * (na + 1) : nullptr;
@@ -745,8 +794,7 @@ __device__ __forceinline__ void step_body(const StepArgs& a) {
     for (int j = 1; j <= na; ++j) w_sum = w_sum + wrow[j];
   }
 
-  const StepConsts c{};  // (tag: the values live in the kernel parameters, StepArgs.c_*)
-  A.G += na * fabs(P.tcost_abs);  // the absolute cost of up to nA transactions
+  A.G += na * fabs(c.tcost_abs(a));  // the absolute cost of up to nA transactions
 
   MDG_PCLK(1);
   if (PAIRS) {
@@ -916,7 +964,7 @@ __device__ __forceinline__ void step_body(const StepArgs& a) {
     }
   }
 
-  const double cash = A.cash, nav = A.nav, pml = A.pml, pbm = A.pbm, pse = A.pse, maintM = a.c_maintM;
+  const double cash = A.cash, nav = A.nav, pml = A.pml, pbm = A.pbm, pse = A.pse, maintM = c.maintM(a);
   MDG_PCLK(39);
   const int head = a.L.head;
   // BrokerResponse.marginCall (Broker.cpp:135,156): Portfolio::checkRisk() after the last transaction
@@ -935,7 +983,7 @@ __device__ __forceinline__ void step_body(const StepArgs& a) {
   const double clampv = (mode == MDG_MODE_SINGLE) ? 0.01 : 0.3;
   gst(&a.IO.reward[e], fast_log(dmax(currentEq / prevEq, clampv)));
   const bool mc = margin_call(cash, nav, pml, pbm, pse, maintM);
-  bool done = mc || (currentEq < 0.1 * P.init_cash);
+  bool done = mc || (currentEq < 0.1 * c.init_cash(a));
   if (mode != MDG_MODE_HOLD) done = done || bad_risk;
   a.IO.done[e] = done ? 1 : 0;
   if (a.done_count) {  // auto-reset: finished envs append themselves to the reset list (warp-aggregated)
@@ -1064,6 +1112,11 @@ template <bool PAIRS, int BS, int MINB, bool ACTIONS, bool BULK = false>
 __global__ void __launch_bounds__(BS, MINB) step_sets_kernel(const __grid_constant__ StepSetsArgs a) {
   step_body<PAIRS, BS, ACTIONS, (MINB < 4) || (BULK && MDG_BULK_TX2), BULK, true>(a);
 }
+// ... and with broker sets (mdg_step_sets_broker)
+template <bool PAIRS, int BS, int MINB, bool ACTIONS, bool BULK = false>
+__global__ void __launch_bounds__(BS, MINB) step_sets_broker_kernel(const __grid_constant__ StepSetsBrokerArgs a) {
+  step_body<PAIRS, BS, ACTIONS, (MINB < 4) || (BULK && MDG_BULK_TX2), BULK, true, true>(a);
+}
 
 // 64-thread blocks, seven per SM (one-wave launches): at 128 registers (registers are granted per warp in units that make 136 or 144 x 14 warps overflow the file: measured two waves)
 #ifndef MDG_BS64_REGS
@@ -1154,15 +1207,16 @@ static inline bool step_tensor_map(const StepMapKey& k, CUtensorMap* out) {
   return true;
 }
 
-// one 128-thread instantiation of the step kernel, with or without parameter sets
-template <bool SETS, bool PAIRS, int MINB, bool ACT, bool BULK, class Args>
+// one 128-thread instantiation of the step kernel, with or without parameter sets (and broker sets)
+template <bool SETS, bool BROKER, bool PAIRS, int MINB, bool ACT, bool BULK, class Args>
 static inline void launch_step128(const Args& a, unsigned grid, size_t smem, cudaStream_t st) {
-  if constexpr (SETS) step_sets_kernel<PAIRS, 128, MINB, ACT, BULK><<<grid, 128, smem, st>>>(a);
+  if constexpr (BROKER) step_sets_broker_kernel<PAIRS, 128, MINB, ACT, BULK><<<grid, 128, smem, st>>>(a);
+  else if constexpr (SETS) step_sets_kernel<PAIRS, 128, MINB, ACT, BULK><<<grid, 128, smem, st>>>(a);
   else step_kernel<PAIRS, 128, MINB, ACT, BULK><<<grid, 128, smem, st>>>(a);
 }
 
-// Args: StepArgs, or StepSetsArgs with SETS
-template <bool SETS = false, class Args = StepArgs>
+// Args: StepArgs, StepSetsArgs with SETS, or StepSetsBrokerArgs with SETS and BROKER
+template <bool SETS = false, bool BROKER = false, class Args = StepArgs>
 static inline int launch_step(Args& a) {
   const int64_t N = a.L.n_envs;
   cudaStream_t st = (cudaStream_t)a.L.stream;
@@ -1217,7 +1271,12 @@ static inline int launch_step(Args& a) {
         const cudaError_t r_ = cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, 56 * 1024);
         if (r_ != cudaSuccess) e_ = r_;
       };
-      if constexpr (SETS) {
+      if constexpr (BROKER) {
+        set((const void*)step_sets_broker_kernel<true, 128, 4, true, true>);
+        set((const void*)step_sets_broker_kernel<true, 128, 4, false, true>);
+        set((const void*)step_sets_broker_kernel<true, 128, 3, true, true>);
+        set((const void*)step_sets_broker_kernel<true, 128, 3, false, true>);
+      } else if constexpr (SETS) {
         set((const void*)step_sets_kernel<true, 128, 4, true, true>);
         set((const void*)step_sets_kernel<true, 128, 4, false, true>);
         set((const void*)step_sets_kernel<true, 128, 3, true, true>);
@@ -1231,7 +1290,7 @@ static inline int launch_step(Args& a) {
     if (attr != cudaSuccess) return cuda_err(attr, "mdg_step shared-memory opt-in");
   }
   const bool acts = a.L.mode == MDG_MODE_MULTI && (a.IO.actions || a.IO.weights);
-#define MDG_LAUNCH(PAIRS_, MINB_, ACT_, BULK_) launch_step128<SETS, PAIRS_, MINB_, ACT_, BULK_>(a, grid, smem, st)
+#define MDG_LAUNCH(PAIRS_, MINB_, ACT_, BULK_) launch_step128<SETS, BROKER, PAIRS_, MINB_, ACT_, BULK_>(a, grid, smem, st)
   if (bs == 64) {
     if constexpr (!SETS) {
       if (a.bulk) {

@@ -14,12 +14,15 @@ def _get(cfg, key, default=None):
 
 def make_env(config, test=False, **batched):
     """Same keys as the reference; the batched ones (``n_envs``, ``seed``, ``device``) may be in
-    ``config`` or passed as keywords."""
+    ``config`` or passed as keywords, and every other keyword goes to ``Env``.  With ``broker_sets`` the config's
+    margins, costs and slippage are the base values of the broker sets, and no setter is called."""
     config = copy.deepcopy(config)
     if test and "data_source_config_test" in config.keys():
         config["data_source_config"] = config["data_source_config_test"]
     if _get(config, "env_type") in ("Synth",):
         env = Env(_get(config, "data_source_type"), _get(config, "init_cash"), config, **batched)
+        if batched.get("broker_sets") is not None:
+            return env
         env.setRequiredMargin(_get(config, "required_margin"))
         env.setMaintenanceMargin(_get(config, "maintenance_margin"))
         env.setTransactionCost(_get(config, "transaction_cost_rel"), _get(config, "transaction_cost_abs"))

@@ -12,6 +12,7 @@ Deviations, all listed in SURVEY.md Appendix A:
   * ``SimpleTrend`` takes config keys, never positions (A10).
 """
 import math
+import numbers
 
 import numpy as np
 
@@ -318,6 +319,40 @@ def make_param_table(data_source_type, base_config, set_configs):
         if (n_g_s, n_n_s, n_u_s) != (n_g, n_n, n_u):  # implied by the slots above; kept as a guard on the builder
             raise ValueError(f"parameter set {s}: generator state / noise rows differ from the base")
         table[:, :, s] = [r["p"] for r in recs]
+    return table
+
+
+# The broker settings a broker set holds, in MdgParams field order (the rows of the broker table, MdgBrokerSlot); the
+# names are make_env's config keys
+BROKER_SLOTS = ("init_cash", "required_margin", "maintenance_margin", "slippage_rel", "slippage_abs",
+                "transaction_cost_rel", "transaction_cost_abs")
+
+
+def _broker_values(d, what):
+    for key, v in d.items():
+        if key not in BROKER_SLOTS:
+            raise ValueError(f"{what}: unknown broker setting {key!r} (known: {', '.join(BROKER_SLOTS)})")
+        if isinstance(v, bool) or not isinstance(v, numbers.Real):
+            raise ValueError(f"{what}: {key} must be a number, got {v!r}")
+    return d
+
+
+def make_broker_table(base, set_dicts):
+    """Broker table of an ``Env`` with broker sets: a ``(MDG_BROKER_NPARAM, S)`` float64 array whose column s holds the
+    seven ``BROKER_SLOTS`` of ``set_dicts[s]`` (set-minor, the layout the ``_sets_broker`` launches read).  ``base``
+    maps every slot to its base value; a key a set omits takes the base value.  An unknown key or a value that is not a
+    real number raises ValueError.  Values are not range-checked (the setters do not check them either)."""
+    base = _broker_values(dict(base), "base")
+    missing = [k for k in BROKER_SLOTS if k not in base]
+    if missing:
+        raise ValueError(f"base: missing broker settings {missing}")
+    set_dicts = list(set_dicts)
+    if not set_dicts:
+        raise ValueError("broker sets: need at least one set")
+    table = np.empty((A.MDG_BROKER_NPARAM, len(set_dicts)), dtype=np.float64)
+    for s, d in enumerate(set_dicts):
+        d = _broker_values(dict(d or {}), f"broker set {s}")
+        table[:, s] = [float(d.get(k, base[k])) for k in BROKER_SLOTS]
     return table
 
 

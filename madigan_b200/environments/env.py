@@ -13,7 +13,7 @@ import torch
 from .. import _abi as A
 from .._lib import check, lib
 from ..utils.data import BrokerResponse, EnvInfo, State
-from .data_source import make_param_table, make_params, make_reward
+from .data_source import BROKER_SLOTS, make_broker_table, make_param_table, make_params, make_reward
 
 
 def _cfg_get(cfg, key, default=None):
@@ -26,6 +26,12 @@ def _cfg_get(cfg, key, default=None):
     except TypeError:
         pass
     return getattr(cfg, key, default)
+
+
+# MdgParams field of each broker setting (data_source.BROKER_SLOTS)
+_P_FIELD = dict(init_cash="init_cash", required_margin="required_margin", maintenance_margin="maintenance_margin",
+                slippage_rel="slippage_rel", slippage_abs="slippage_abs", transaction_cost_rel="tcost_rel",
+                transaction_cost_abs="tcost_abs")
 
 
 class Asset:
@@ -93,7 +99,8 @@ def _reset_workspace(lib_, P, n_envs, fill_ticks, device, stream_ptr=None, strea
 
 class Env:
     def __init__(self, dataSourceType, initCash=1_000_000., config=None, *, n_envs=None, device=None,
-                 window=None, seed=None, env_offset=0, reward=None, param_sets=None, param_set=None):
+                 window=None, seed=None, env_offset=0, reward=None, param_sets=None, param_set=None,
+                 broker_sets=None):
         """``Env(data_source_type, init_cash, config)`` as the reference (env.cpp:843-849); the batched
         keys ``n_envs``, ``seed``, ``device``, ``window_length`` may come from ``config`` or keywords.
         ``reward``: None (env reward only) or a dict with ``reward_shaper_config``, ``nstep_return``,
@@ -103,7 +110,14 @@ class Env:
         ``S`` for S copies of the base config (to be edited through ``param_table``).  ``param_set``: the ``(N,)``
         integer set of every env, ``arange(N) % S`` by default.  Env e then equals, bit for bit, env e of a plain Env
         built from its set's config with the same ``n_envs``, ``seed`` and ``env_offset``
-        (see ``make_param_table``, ``assign_param_sets``)."""
+        (see ``make_param_table``, ``assign_param_sets``).
+        ``broker_sets``: broker settings per parameter set, so that the envs also trade under different frictions -- a
+        list of dicts over ``data_source.BROKER_SLOTS`` (a key a set omits takes the base value), or an int ``S`` for S
+        copies of the base values (to be edited through ``broker_table``).  The base values are ``initCash`` and the
+        same keys in ``config`` (0 when absent).  With ``param_sets`` its length must be S; without, the generator
+        table is S copies of the base config.  One index per env selects both tables: env e then equals, bit for bit,
+        env e of a plain Env of its set's config with ``setRequiredMargin / setMaintenanceMargin / setSlippage /
+        setTransactionCost`` and ``initCash`` at its broker set's values (see ``make_broker_table``)."""
         self._lib = lib()
         if not torch.cuda.is_available():
             raise RuntimeError("madigan_b200.Env needs a CUDA device (sm_100a); there is no CPU fallback")
@@ -139,8 +153,22 @@ class Env:
         self.ra = 1 if self.R.reduce_rewards else self.nA
         self._alloc()
         self._PS = None  # MdgParamSets of an env with parameter sets
+        self._btab, self._bptr = None, None  # broker table [MDG_BROKER_NPARAM][S] and its address (broker sets)
+        if broker_sets is not None:
+            btab = self._broker_table(config, broker_sets)
+            S = btab.shape[1]
+            if param_sets is None:
+                param_sets = S
+            elif (param_sets if isinstance(param_sets, int) else len(param_sets)) != S:
+                raise ValueError(f"broker_sets has {S} sets, param_sets has "
+                                 f"{param_sets if isinstance(param_sets, int) else len(param_sets)}")
         if param_sets is not None:
             self._init_param_sets(dataSourceType, ds_cfg, param_sets, param_set)
+        if broker_sets is not None:
+            self._btab = torch.from_numpy(btab).to(self.device).contiguous()
+            self._bptr = self._btab.data_ptr()
+            for k_, v in self._broker_base.items():  # MdgParams holds the base values, as a plain Env's would
+                setattr(self.P, _P_FIELD[k_], v)
         self.head = 0
         self.n_valid = 0
         self._gstep = 0
@@ -153,8 +181,8 @@ class Env:
                 check(self._lib.mdg_init_state(C.byref(self.P), C.byref(self.R), C.byref(self._S),
                                                C.byref(self._launch())))
             else:
-                check(self._lib.mdg_init_state_sets(C.byref(self.P), C.byref(self.R), C.byref(self._S),
-                                                    C.byref(self._launch()), self._pPS))
+                check(self._lib.mdg_init_state_sets_broker(C.byref(self.P), C.byref(self.R), C.byref(self._S),
+                                                           C.byref(self._launch()), self._pPS, self._bptr))
             self.launches += 1
             # the constructor consumes one generator tick (Env.h:160)
             self._reset_launch(None, 1, False, None, None)
@@ -226,6 +254,42 @@ class Env:
             self.assign_param_sets(param_set)
         self._PS = A.MdgParamSets(p=self._ptab.data_ptr(), set_of_env=self._pset.data_ptr(), n_sets=S)
         self._pPS = C.byref(self._PS)
+
+    def _broker_table(self, config, broker_sets):
+        """(MDG_BROKER_NPARAM, S) numpy table of ``broker_sets``; resolves the base values"""
+        if isinstance(broker_sets, bool) or not isinstance(broker_sets, (int, list, tuple)):
+            raise TypeError("broker_sets must be a list of dicts over data_source.BROKER_SLOTS or an int")
+        if isinstance(broker_sets, int):
+            if broker_sets < 1:
+                raise ValueError("broker_sets must be >= 1")
+            broker_sets = [{}] * broker_sets
+        base = {k: float(_cfg_get(config, k, 0.)) for k in BROKER_SLOTS[1:]}
+        self._broker_base = dict(init_cash=self._initCash, **base)
+        return make_broker_table(self._broker_base, broker_sets)
+
+    @property
+    def broker_table(self):
+        """``(S, MDG_BROKER_NPARAM)`` fp64 device view of the broker sets: ``broker_table[s, k]`` is setting k
+        (``data_source.BROKER_SLOTS``) of set s.  Writable in place, with ``param_table``'s semantics: every launch reads
+        it as it stands on the env's stream, so a change takes effect at the next step or reset.  After an in-place
+        write, call ``invalidate()`` before reading derived properties (``availableMargin``, ``usedMargin``,
+        ``checkRisk()``), which are cached per step.  None without broker sets."""
+        return None if self._btab is None else self._btab.t()
+
+    def _per_env(self, k):
+        """(N,) broker setting k of every env's set (out-of-range set indices clamp as in the kernels)"""
+        S = self._btab.shape[1]
+        with self._copy_ctx():
+            s = self._pset.long()
+            return self._btab[k][torch.where((s < 0) | (s >= S), S - 1, s)]
+
+    def _set_broker(self, **values):
+        """the setters of an Env with broker sets: the field of every set, on the env's stream"""
+        if self._stream is not None:
+            self._stream.wait_stream(torch.cuda.current_stream(self.device))
+        with self._device_ctx(), self._copy_ctx():
+            for k_, v in values.items():
+                self._btab[BROKER_SLOTS.index(k_)].fill_(v)
 
     @property
     def n_param_sets(self):
@@ -333,19 +397,28 @@ class Env:
         return ptrs[0], ptrs[1], keep
 
     # ------------------------------------------------------------------ setters (Env.h:94-111)
+    # With broker sets, each setter writes its field into every set: the Env's envs all take the value.
     def setRequiredMargin(self, reqM):
         self.P.required_margin = float(reqM)
+        if self._btab is not None:
+            self._set_broker(required_margin=float(reqM))
         self._version += 1
 
     def setMaintenanceMargin(self, mainM):
         self.P.maintenance_margin = float(mainM)
+        if self._btab is not None:
+            self._set_broker(maintenance_margin=float(mainM))
         self._version += 1
 
     def setSlippage(self, slippagePct=0., slippageAbs=0.):
         self.P.slippage_rel, self.P.slippage_abs = float(slippagePct), float(slippageAbs)
+        if self._btab is not None:
+            self._set_broker(slippage_rel=float(slippagePct), slippage_abs=float(slippageAbs))
 
     def setTransactionCost(self, transactionPct=0., transactionAbs=0.):
         self.P.tcost_rel, self.P.tcost_abs = float(transactionPct), float(transactionAbs)
+        if self._btab is not None:
+            self._set_broker(transaction_cost_rel=float(transactionPct), transaction_cost_abs=float(transactionAbs))
 
     # ------------------------------------------------------------------ reset / step
     def _reset_launch(self, mask, fill_ticks, clear_nstep, normals, uniforms):
@@ -372,9 +445,10 @@ class Env:
                                          None if m is None else m.data_ptr(), int(fill_ticks), int(clear_nstep),
                                          ws.data_ptr(), ws.numel()))
         else:
-            check(self._lib.mdg_reset_ws_sets(C.byref(self.P), C.byref(self._S), C.byref(io), C.byref(self._launch()),
-                                              None if m is None else m.data_ptr(), int(fill_ticks), int(clear_nstep),
-                                              ws.data_ptr(), ws.numel(), self._pPS))
+            check(self._lib.mdg_reset_ws_sets_broker(C.byref(self.P), C.byref(self._S), C.byref(io),
+                                                     C.byref(self._launch()), None if m is None else m.data_ptr(),
+                                                     int(fill_ticks), int(clear_nstep), ws.data_ptr(), ws.numel(),
+                                                     self._pPS, self._bptr))
         self.launches += 2  # list scan + refill kernel
         self._version += 1
         del keep
@@ -459,7 +533,7 @@ class Env:
                 if self._PS is None:
                     check(self._lib.mdg_step(self._pP, self._pR, self._pS, self._pIO, self._pL))
                 else:
-                    check(self._lib.mdg_step_sets(self._pP, self._pR, self._pS, self._pIO, self._pL, self._pPS))
+                    self._step_call()
                 self.launches += 1
             self.head = L.head
             self.n_valid = min(self.k, self.n_valid + 1)
@@ -477,15 +551,16 @@ class Env:
         if self._PS is None:
             check(self._lib.mdg_step(self._pP, self._pR, self._pS, self._pIO, self._pL))
         else:
-            check(self._lib.mdg_step_sets(self._pP, self._pR, self._pS, self._pIO, self._pL, self._pPS))
+            check(self._lib.mdg_step_sets_broker(self._pP, self._pR, self._pS, self._pIO, self._pL, self._pPS,
+                                                 self._bptr))
 
     def _step_autoreset_call(self, ws):
         if self._PS is None:
             check(self._lib.mdg_step_autoreset(self._pP, self._pR, self._pS, self._pIO, self._pL, self.k, 1,
                                                ws.data_ptr(), ws.numel()))
         else:
-            check(self._lib.mdg_step_autoreset_sets(self._pP, self._pR, self._pS, self._pIO, self._pL, self.k, 1,
-                                                    ws.data_ptr(), ws.numel(), self._pPS))
+            check(self._lib.mdg_step_autoreset_sets_broker(self._pP, self._pR, self._pS, self._pIO, self._pL, self.k,
+                                                           1, ws.data_ptr(), ws.numel(), self._pPS, self._bptr))
 
     def step_actions(self, actions, *, action_atoms, unit_size, normals=None, uniforms=None, auto_reset=False):
         """``env.step(agent.action_to_transaction(actions))`` in one launch: ``actions`` is an (N, nA) integer tensor
@@ -638,7 +713,12 @@ class Env:
                 setattr(D, n, v.data_ptr())
             self._D = D
         with torch.cuda.device(self.device):
-            check(self._lib.mdg_derived(C.byref(self.P), C.byref(self._S), C.byref(self._D), C.byref(self._launch())))
+            if self._PS is None:
+                check(self._lib.mdg_derived(C.byref(self.P), C.byref(self._S), C.byref(self._D),
+                                            C.byref(self._launch())))
+            else:
+                check(self._lib.mdg_derived_sets_broker(C.byref(self.P), C.byref(self._S), C.byref(self._D),
+                                                        C.byref(self._launch()), self._pPS, self._bptr))
         self.launches += 1
         self._derived_version = self._version
         return self._d
@@ -720,12 +800,13 @@ class Env:
     def assets(self): return [Asset(n) for n in self._asset_names]
     @property
     def isDateTime(self): return False
+    # with broker sets: the (N,) values of every env's set
     @property
-    def initCash(self): return self._initCash
+    def initCash(self): return self._initCash if self._btab is None else self._per_env(0)
     @property
-    def requiredMargin(self): return self.P.required_margin
+    def requiredMargin(self): return self.P.required_margin if self._btab is None else self._per_env(1)
     @property
-    def maintenanceMargin(self): return self.P.maintenance_margin
+    def maintenanceMargin(self): return self.P.maintenance_margin if self._btab is None else self._per_env(2)
     @property
     def dataSourceType(self): return self._dataSourceType
     @property
@@ -815,12 +896,14 @@ class Env:
         if self._PS is not None:
             sd["param_table"] = self._ptab.clone()  # [nA][NPARAM][S] storage
             sd["param_set"] = self._pset.clone()
+        if self._btab is not None:
+            sd["broker_table"] = self._btab.clone()  # [MDG_BROKER_NPARAM][S] storage
         sd["_meta"] = dict(head=self.head, n_valid=self.n_valid, gstep=self._gstep, seed=self.seed,
                            env_offset=self.env_offset, n_envs=self.N, n_assets=self.nA, window=self.k,
                            nstep=int(self.R.nstep), ra=self.ra, shaper=int(self.R.shaper),
                            margins=(self.P.required_margin, self.P.maintenance_margin),
                            costs=(self.P.tcost_rel, self.P.tcost_abs, self.P.slippage_rel, self.P.slippage_abs),
-                           n_sets=self.n_param_sets)
+                           n_sets=self.n_param_sets, broker_sets=self._btab is not None)
         return sd
 
     def load_state_dict(self, sd):
@@ -833,9 +916,15 @@ class Env:
         if m.get("n_sets", 0) != self.n_param_sets:
             raise ValueError(f"checkpoint was taken from an Env with {m.get('n_sets', 0)} parameter sets, this one has "
                              f"{self.n_param_sets}")
+        if m.get("broker_sets", False) != (self._btab is not None):
+            has = lambda b: "with" if b else "without"
+            raise ValueError(f"checkpoint was taken from an Env {has(m.get('broker_sets', False))} broker sets, this one "
+                             f"is {has(self._btab is not None)}")
         if self._PS is not None:
             self._ptab.copy_(sd["param_table"])
             self._pset.copy_(sd["param_set"])
+        if self._btab is not None:
+            self._btab.copy_(sd["broker_table"])
         for k_, v in sd.items():
             if k_ == "_meta" or k_ in self._STAGING or k_ not in self.t:
                 continue
