@@ -273,8 +273,8 @@ enum MdgNorm {
 int mdg_abi_version(void);
 /* sizeof of the ABI structs as compiled: 0 MdgAssetGen 1 MdgParams 2 MdgReward 3 MdgState 4 MdgStepIO
  * 5 MdgLaunch 6 MdgDerived 7 MdgWindow 8 MdgReplay 9 MdgReplayBatch 10 MdgRewardNorm 11 MdgTearsheet
- * 12 MdgPrioritized 13 MdgReplayRows 14 MdgParamSets; -1 for an unknown index (lets a binding verify its struct
- * mirror) */
+ * 12 MdgPrioritized 13 MdgReplayRows 14 MdgParamSets 15 MdgSetDraw; -1 for an unknown index (lets a binding verify
+ * its struct mirror) */
 int mdg_sizeof(int which);
 const char *mdg_last_error(void);
 
@@ -393,6 +393,41 @@ int mdg_reset_ws_sets_broker(const MdgParams *params, const MdgState *state, con
                              void *workspace, int64_t workspace_bytes, const MdgParamSets *sets, const double *broker);
 int mdg_init_state_sets_broker(const MdgParams *params, const MdgReward *reward, const MdgState *state,
                                const MdgLaunch *launch, const MdgParamSets *sets, const double *broker);
+
+/* ---------------------------------------------------------------------------------------------------
+ * Per-episode set draw: every refill of a listed env draws the env's parameter set anew (a new market per episode,
+ * for training that is robust to the market), inside the launches a training loop already makes.
+ *
+ * cdf holds n_sets doubles (n_sets of the call's MdgParamSets): the cumulative sums of the weights, left to right,
+ * over their total, with cdf[n_sets - 1] == 1.0 exactly; a set of weight 0 repeats its predecessor's entry and is never
+ * drawn.  The draw of env e at tick t takes Philox4x32-10 with key (seed lo, seed hi) and counter
+ * (env_offset + e, 4 << 16, t lo, t hi), x0 = (out[1] << 32) | out[0], u = (x0 >> 11) 2^-53, and yields the number
+ * of cdf entries <= u (clamped to n_sets - 1).  It depends on (seed, global env id, tick, cdf) only, and uses Philox
+ * also when the normals / uniforms are injected.
+ *   - Refill (mdg_reset_ws_sets_draw, mdg_step_autoreset_sets_draw, both refill kernels): t is the env's timestamp
+ *     before the refill; the refill writes episode_set[e] = the set the env had (clamped as the kernels read it) and
+ *     set_of_env[e] = the drawn set, and runs the new episode (generator restart, history ticks, starting cash) in
+ *     the drawn set.  Every refill advances the timestamp, so no two draws of one env share a counter.
+ *   - Constructor (mdg_init_state_sets_draw): t = 0; it writes set_of_env[e] before the start values and the starting
+ *     cash are read, and episode_set[e] = -1 (no episode has finished).
+ * So these launches WRITE sets->set_of_env.  The step kernel is unchanged: it reads the set the refill left.
+ * draw == NULL: exactly the corresponding _sets_broker launch (broker may be NULL: the _sets launch).  A draw whose
+ * cdf or episode_set is NULL: MDG_E_INVALID; otherwise the checks of the _sets_broker launches. */
+typedef struct MdgSetDraw {
+  const double *cdf;    /* device: [n_sets] */
+  int32_t *episode_set; /* device: [N], written for each listed env */
+} MdgSetDraw;
+int mdg_step_autoreset_sets_draw(const MdgParams *params, const MdgReward *reward, const MdgState *state,
+                                 const MdgStepIO *io, const MdgLaunch *launch, int fill_ticks, int clear_nstep,
+                                 void *workspace, int64_t workspace_bytes, const MdgParamSets *sets,
+                                 const double *broker, const MdgSetDraw *draw);
+int mdg_reset_ws_sets_draw(const MdgParams *params, const MdgState *state, const MdgStepIO *io,
+                           const MdgLaunch *launch, const uint8_t *mask, int fill_ticks, int clear_nstep,
+                           void *workspace, int64_t workspace_bytes, const MdgParamSets *sets, const double *broker,
+                           const MdgSetDraw *draw);
+int mdg_init_state_sets_draw(const MdgParams *params, const MdgReward *reward, const MdgState *state,
+                             const MdgLaunch *launch, const MdgParamSets *sets, const double *broker,
+                             const MdgSetDraw *draw);
 
 /* Recompute MdgState.folds from the state tensors (after external writes into them). */
 int mdg_refresh_folds(const MdgParams *params, const MdgState *state, const MdgLaunch *launch);

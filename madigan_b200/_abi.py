@@ -127,6 +127,10 @@ class MdgParamSets(C.Structure):
     _fields_ = [("p", _dp), ("set_of_env", _dp), ("n_sets", C.c_int32), ("_pad", C.c_int32)]
 
 
+class MdgSetDraw(C.Structure):
+    _fields_ = [("cdf", _dp), ("episode_set", _dp)]
+
+
 RN_NULL, RN_SHARPE_FIXED, RN_SORTINO_A, RN_SORTINO_B, RN_SORTINO_C, RN_SHARPE_EWMA = range(6)
 
 
@@ -175,6 +179,14 @@ SYMBOLS = {
                                            C.c_int, C.c_int, C.c_void_p, C.c_int64, _P(MdgParamSets), C.c_void_p]),
     "mdg_init_state_sets_broker": (C.c_int, [_P(MdgParams), _P(MdgReward), _P(MdgState), _P(MdgLaunch),
                                              _P(MdgParamSets), C.c_void_p]),
+    "mdg_step_autoreset_sets_draw": (C.c_int, [_P(MdgParams), _P(MdgReward), _P(MdgState), _P(MdgStepIO),
+                                               _P(MdgLaunch), C.c_int, C.c_int, C.c_void_p, C.c_int64,
+                                               _P(MdgParamSets), C.c_void_p, _P(MdgSetDraw)]),
+    "mdg_reset_ws_sets_draw": (C.c_int, [_P(MdgParams), _P(MdgState), _P(MdgStepIO), _P(MdgLaunch), C.c_void_p,
+                                         C.c_int, C.c_int, C.c_void_p, C.c_int64, _P(MdgParamSets), C.c_void_p,
+                                         _P(MdgSetDraw)]),
+    "mdg_init_state_sets_draw": (C.c_int, [_P(MdgParams), _P(MdgReward), _P(MdgState), _P(MdgLaunch),
+                                           _P(MdgParamSets), C.c_void_p, _P(MdgSetDraw)]),
     "mdg_refresh_folds": (C.c_int, [_P(MdgParams), _P(MdgState), _P(MdgLaunch)]),
     "mdg_derived": (C.c_int, [_P(MdgParams), _P(MdgState), _P(MdgDerived), _P(MdgLaunch)]),
     "mdg_derived_sets_broker": (C.c_int, [_P(MdgParams), _P(MdgState), _P(MdgDerived), _P(MdgLaunch),
@@ -217,4 +229,5 @@ def bind(lib):
 
 
 STRUCTS = (MdgAssetGen, MdgParams, MdgReward, MdgState, MdgStepIO, MdgLaunch, MdgDerived, MdgWindow, MdgReplay,
-           MdgReplayBatch, MdgRewardNorm, MdgTearsheet, MdgPrioritized, MdgReplayRows, MdgParamSets)  # mdg_sizeof order
+           MdgReplayBatch, MdgRewardNorm, MdgTearsheet, MdgPrioritized, MdgReplayRows, MdgParamSets,
+           MdgSetDraw)  # mdg_sizeof order

@@ -173,6 +173,10 @@ struct ResetWsSetsArgs : ResetWsArgs {
 struct ResetWsBrokerArgs : ResetWsSetsArgs {
   const double* broker;
 };
+// ... with the per-episode set draw (broker: NULL without broker sets)
+struct ResetWsDrawArgs : ResetWsBrokerArgs {
+  MdgSetDraw draw;
+};
 
 __global__ void __launch_bounds__(256) reset_scan_kernel(const __grid_constant__ ResetWsArgs a) {
   const int64_t N = a.L.n_envs;
@@ -189,7 +193,7 @@ __global__ void __launch_bounds__(256) reset_scan_kernel(const __grid_constant__
 
 constexpr int kFillBlock = 128;
 
-template <bool SETS, bool BROKER = false>
+template <bool SETS, bool BROKER = false, bool DRAW = false>
 __device__ __forceinline__ void reset_fill_body(const ResetWsArgs& a) {
   extern __shared__ double zs[];  // [chunk][n_normals]
   const MdgParams& P = a.P;
@@ -208,6 +212,12 @@ __device__ __forceinline__ void reset_fill_body(const ResetWsArgs& a) {
     const long long ts0 = a.S.timestamp[e];
     int64_t set = 0;  // parameter sets: the listed env's set
     if constexpr (SETS) set = env_set(static_cast<const ResetWsSetsArgs&>(a).ps, e);
+    int64_t old_set = 0;
+    if constexpr (DRAW) {  // the new episode's set: every thread draws it (a function of seed, env, ts0 and cdf only)
+      const ResetWsDrawArgs& w = static_cast<const ResetWsDrawArgs&>(a);
+      old_set = set;
+      set = draw_set(w.draw.cdf, w.ps.n_sets, (uint32_t)(a.L.env_offset + e), (unsigned long long)ts0, k0, k1);
+    }
     double cash = cash0, eq = eq0;
     bool eq_plain = eq_plain0;
     if constexpr (BROKER) {  // the fresh portfolio's cash from the listed env's set
@@ -216,8 +226,13 @@ __device__ __forceinline__ void reset_fill_body(const ResetWsArgs& a) {
       eq = cash + 0. - 0.;
       eq_plain = eq > 0. && eq < 1e300;
     }
-    __syncthreads();  // every thread has read the old timestamp (and the previous env's normals are consumed)
+    __syncthreads();  // every thread has read the old timestamp and set (and the previous env's normals are consumed)
     if (tid == 32) {  // fresh Broker/Account/Portfolio (Env.h:150-165): per-env scalars
+      if constexpr (DRAW) {
+        const ResetWsDrawArgs& w = static_cast<const ResetWsDrawArgs&>(a);
+        w.draw.episode_set[e] = (int32_t)old_set;
+        const_cast<int32_t*>(w.ps.set_of_env)[e] = (int32_t)set;
+      }
       if (a.clear_nstep && a.S.nstep_len) a.S.nstep_len[e] = 0;  // offpolicy_q.py:94
       a.S.cash[e] = cash;
       if (a.S.folds) {  // flat portfolio: every fold is a sum of zeros
@@ -362,6 +377,12 @@ __global__ void __launch_bounds__(kFillBlock) reset_fill_sets_kernel(const __gri
 __global__ void __launch_bounds__(kFillBlock) reset_fill_sets_broker_kernel(const __grid_constant__ ResetWsBrokerArgs a) {
   reset_fill_body<true, true>(a);
 }
+__global__ void __launch_bounds__(kFillBlock) reset_fill_sets_draw_kernel(const __grid_constant__ ResetWsDrawArgs a) {
+  reset_fill_body<true, false, true>(a);
+}
+__global__ void __launch_bounds__(kFillBlock) reset_fill_sets_broker_draw_kernel(const __grid_constant__ ResetWsDrawArgs a) {
+  reset_fill_body<true, true, true>(a);
+}
 
 // The refill of the all-OU-pairs parameter sets (all_ou_pairs(P)) when the normals come from Philox: one lane per
 // (listed env, pair), np = nA/2 lanes per env, 128/np envs per block.  A pair is an independent process whose three
@@ -380,7 +401,7 @@ __global__ void __launch_bounds__(kFillBlock) reset_fill_sets_broker_kernel(cons
 #define MDG_FILL_PAIRS_MINB 1
 #endif
 constexpr int kFillPairsUnroll = MDG_FILL_PAIRS_UNROLL;
-template <bool SETS, bool BROKER = false>
+template <bool SETS, bool BROKER = false, bool DRAW = false>
 __device__ __forceinline__ void reset_fill_pairs_body(const ResetWsArgs& a) {
   const MdgParams& P = a.P;
   const int tid = threadIdx.x;
@@ -407,9 +428,16 @@ __device__ __forceinline__ void reset_fill_pairs_body(const ResetWsArgs& a) {
     const long long ts0 = active ? a.S.timestamp[e] : 0;
     double cash = cash0, eq = eq0;
     bool eq_plain = eq_plain0;
+    int64_t old_set = 0, new_set = 0;  // DRAW
     if constexpr (SETS) {  // this lane's pair in the listed env's set (idle lanes read env 0's, and store nothing)
       const MdgParamSets& ps = static_cast<const ResetWsSetsArgs&>(a).ps;
-      const int64_t set = env_set(ps, e);
+      int64_t set = env_set(ps, e);
+      if constexpr (DRAW) {  // every lane of the env draws the same set (its np lanes may span warps)
+        old_set = set;
+        set = draw_set(static_cast<const ResetWsDrawArgs&>(a).draw.cdf, ps.n_sets, (uint32_t)(a.L.env_offset + e),
+                       (unsigned long long)ts0, k0, k1);
+        new_set = set;
+      }
       const SetParams q0 = set_params(ps, set, i0), q1 = set_params(ps, set, i0 + 1);
       theta0 = q0[0]; phi0 = q0[1]; noise = q0[2]; theta1 = q1[0]; phi1 = q1[1];
       if constexpr (BROKER) {  // the fresh portfolio's cash from the set too
@@ -418,9 +446,14 @@ __device__ __forceinline__ void reset_fill_pairs_body(const ResetWsArgs& a) {
         eq_plain = eq > 0. && eq < 1e300;
       }
     }
-    __syncthreads();  // every lane of an env has read the old timestamp before its pair-0 lane writes the new one
+    __syncthreads();  // every lane of an env has read the old timestamp (and set) before its pair-0 lane writes the new one
     // idle lanes run the tick loop too (without storing): the loop's shuffles take every lane of the warp
     if (active && p == 0) {  // fresh Broker/Account/Portfolio (Env.h:150-165): per-env scalars
+      if constexpr (DRAW) {
+        const ResetWsDrawArgs& w = static_cast<const ResetWsDrawArgs&>(a);
+        w.draw.episode_set[e] = (int32_t)old_set;
+        const_cast<int32_t*>(w.ps.set_of_env)[e] = (int32_t)new_set;
+      }
       if (a.clear_nstep && a.S.nstep_len) a.S.nstep_len[e] = 0;  // offpolicy_q.py:94
       a.S.cash[e] = cash;
       if (a.S.folds) {  // flat portfolio: every fold is a sum of zeros
@@ -507,6 +540,14 @@ __global__ void __launch_bounds__(kFillBlock, MDG_FILL_PAIRS_MINB)
     reset_fill_pairs_sets_broker_kernel(const __grid_constant__ ResetWsBrokerArgs a) {
   reset_fill_pairs_body<true, true>(a);
 }
+__global__ void __launch_bounds__(kFillBlock, MDG_FILL_PAIRS_MINB)
+    reset_fill_pairs_sets_draw_kernel(const __grid_constant__ ResetWsDrawArgs a) {
+  reset_fill_pairs_body<true, false, true>(a);
+}
+__global__ void __launch_bounds__(kFillBlock, MDG_FILL_PAIRS_MINB)
+    reset_fill_pairs_sets_broker_draw_kernel(const __grid_constant__ ResetWsDrawArgs a) {
+  reset_fill_pairs_body<true, true, true>(a);
+}
 
 // constructor state (Env.h:139-165 before the first tick)
 struct InitArgs {
@@ -521,19 +562,30 @@ struct InitSetsArgs : InitArgs {
 struct InitBrokerArgs : InitSetsArgs {
   const double* broker;
 };
+struct InitDrawArgs : InitBrokerArgs {
+  MdgSetDraw draw;
+};
 // e: computed in the kernels, where the compiler knows the range of threadIdx.x
-template <bool SETS, bool BROKER = false>
+template <bool SETS, bool BROKER = false, bool DRAW = false>
 __device__ __forceinline__ void init_body(const InitArgs& a, int64_t e) {
   const int64_t N = a.L.n_envs;
   if (e >= N) return;
   const int na = a.P.n_assets;
+  int64_t drawn = 0;
+  if constexpr (DRAW) {  // the first episode's set: the draw at tick 0, before anything reads the set
+    const InitDrawArgs& w = static_cast<const InitDrawArgs&>(a);
+    drawn = draw_set(w.draw.cdf, w.ps.n_sets, (uint32_t)(a.L.env_offset + e), 0ull, (uint32_t)a.L.seed,
+                     (uint32_t)(a.L.seed >> 32));
+    const_cast<int32_t*>(w.ps.set_of_env)[e] = (int32_t)drawn;
+    w.draw.episode_set[e] = -1;  // no episode has finished yet
+  }
   for (int i = 0; i < na; ++i) {
     const MdgAssetGen& g = a.P.gen[i];
     double* gs = a.S.gstate + (int64_t)(g.gslot < 0 ? 0 : g.gslot) * N + e;
     const CtorDraws cd = ctor_draws((uint32_t)(a.L.env_offset + e), a.L.seed, 0, 3, i);
     if constexpr (SETS) {  // start values (OU mean, Synth phase, trend start) from the env's set
       const MdgParamSets& ps = static_cast<const InitSetsArgs&>(a).ps;
-      a.S.price[(int64_t)i * N + e] = gen_start_p(g, set_params(ps, env_set(ps, e), i), gs, N, a.P.gen_ext, &cd);
+      a.S.price[(int64_t)i * N + e] = gen_start_p(g, set_params(ps, DRAW ? drawn : env_set(ps, e), i), gs, N, a.P.gen_ext, &cd);
     } else {
       a.S.price[(int64_t)i * N + e] = gen_start(g, gs, N, a.P.gen_ext, &cd);
     }
@@ -544,7 +596,7 @@ __device__ __forceinline__ void init_body(const InitArgs& a, int64_t e) {
   double cash = a.P.init_cash;
   if constexpr (BROKER) {  // the env's set's starting cash
     const InitBrokerArgs& b = static_cast<const InitBrokerArgs&>(a);
-    cash = broker_value(b.broker, b.ps.n_sets, env_set(b.ps, e), MDG_BROKER_INIT_CASH);
+    cash = broker_value(b.broker, b.ps.n_sets, DRAW ? drawn : env_set(b.ps, e), MDG_BROKER_INIT_CASH);
   }
   a.S.cash[e] = cash;
   a.S.timestamp[e] = 0;
@@ -568,6 +620,12 @@ __global__ void __launch_bounds__(128) init_sets_kernel(const __grid_constant__ 
 }
 __global__ void __launch_bounds__(128) init_sets_broker_kernel(const __grid_constant__ InitBrokerArgs a) {
   init_body<true, true>(a, (int64_t)blockIdx.x * 128 + threadIdx.x);
+}
+__global__ void __launch_bounds__(128) init_sets_draw_kernel(const __grid_constant__ InitDrawArgs a) {
+  init_body<true, false, true>(a, (int64_t)blockIdx.x * 128 + threadIdx.x);
+}
+__global__ void __launch_bounds__(128) init_sets_broker_draw_kernel(const __grid_constant__ InitDrawArgs a) {
+  init_body<true, true, true>(a, (int64_t)blockIdx.x * 128 + threadIdx.x);
 }
 
 // exact left-to-right folds of the portfolio as stored (after external writes into the state tensors)
@@ -762,8 +820,9 @@ constexpr int kFillPairsBlocksPerSm = 2;
 // spreads an env's draws over a block (~12 us).  With few pairs per env that latency is not paid back: one OU pair per
 // env (C3, 65,536 envs, one stream) measured 20.5 us per step with the generic refill, 34.9 with this one.
 constexpr int kFillPairsMinAssets = 8;
-// Args: ResetWsArgs, ResetWsSetsArgs with SETS, or ResetWsBrokerArgs with SETS and BROKER (the same kernel choice)
-template <bool SETS = false, bool BROKER = false, class Args = ResetWsArgs>
+// Args: ResetWsArgs, ResetWsSetsArgs with SETS, ResetWsBrokerArgs with SETS and BROKER, or ResetWsDrawArgs with SETS
+// and DRAW (the same kernel choice)
+template <bool SETS = false, bool BROKER = false, bool DRAW = false, class Args = ResetWsArgs>
 static int launch_fill(const Args& a, int64_t max_listed) {
   // the count is on the device: size the grid for the most the list can hold, capped at a few blocks per SM
   // (grid-stride; blocks past the end of the list only read the count and take their exit ticket)
@@ -780,7 +839,9 @@ static int launch_fill(const Args& a, int64_t max_listed) {
     const int64_t groups = (max_listed + epb - 1) / epb;
     const int64_t cap = knob ? knob : kFillPairsBlocksPerSm * sm_count();
     const unsigned grid = (unsigned)(groups < cap ? (groups > 0 ? groups : 1) : cap);
-    if constexpr (BROKER) reset_fill_pairs_sets_broker_kernel<<<grid, kFillBlock, 0, st>>>(a);
+    if constexpr (DRAW && BROKER) reset_fill_pairs_sets_broker_draw_kernel<<<grid, kFillBlock, 0, st>>>(a);
+    else if constexpr (DRAW) reset_fill_pairs_sets_draw_kernel<<<grid, kFillBlock, 0, st>>>(a);
+    else if constexpr (BROKER) reset_fill_pairs_sets_broker_kernel<<<grid, kFillBlock, 0, st>>>(a);
     else if constexpr (SETS) reset_fill_pairs_sets_kernel<<<grid, kFillBlock, 0, st>>>(a);
     else reset_fill_pairs_kernel<<<grid, kFillBlock, 0, st>>>(a);
     return cuda_err(cudaGetLastError(), "reset_fill_pairs launch");
@@ -788,16 +849,36 @@ static int launch_fill(const Args& a, int64_t max_listed) {
   const int64_t cap = knob ? knob : 148 * 8;
   const unsigned grid = (unsigned)(max_listed < cap ? (max_listed > 0 ? max_listed : 1) : cap);
   const size_t smem = sizeof(double) * (size_t)a.chunk * (size_t)(a.P.n_normals > 0 ? a.P.n_normals : 1);
-  if constexpr (BROKER) reset_fill_sets_broker_kernel<<<grid, kFillBlock, smem, st>>>(a);
+  if constexpr (DRAW && BROKER) reset_fill_sets_broker_draw_kernel<<<grid, kFillBlock, smem, st>>>(a);
+  else if constexpr (DRAW) reset_fill_sets_draw_kernel<<<grid, kFillBlock, smem, st>>>(a);
+  else if constexpr (BROKER) reset_fill_sets_broker_kernel<<<grid, kFillBlock, smem, st>>>(a);
   else if constexpr (SETS) reset_fill_sets_kernel<<<grid, kFillBlock, smem, st>>>(a);
   else reset_fill_kernel<<<grid, kFillBlock, smem, st>>>(a);
   return cuda_err(cudaGetLastError(), "reset_fill launch");
 }
 }  // namespace mdg
 
+namespace mdg {
+// a per-episode set draw needs its cdf and its episode_set
+static int check_draw(const MdgSetDraw* draw) {
+  if (draw && (!draw->cdf || !draw->episode_set)) return set_err(MDG_E_INVALID, "set draw: null cdf / episode_set");
+  return MDG_OK;
+}
+// the refill of a launch with parameter sets: a.ps and a.broker are set
+static int launch_fill_sets(ResetWsDrawArgs& a, int64_t max_listed, const MdgSetDraw* draw) {
+  if (draw) {
+    a.draw = *draw;
+    if (a.broker) return launch_fill<true, true, true>(a, max_listed);
+    return launch_fill<true, false, true>(a, max_listed);
+  }
+  if (!a.broker) return launch_fill<true>(static_cast<const ResetWsSetsArgs&>(a), max_listed);
+  return launch_fill<true, true>(static_cast<const ResetWsBrokerArgs&>(a), max_listed);
+}
+}  // namespace mdg
+
 static int reset_ws_impl(const MdgParams* P, const MdgState* S, const MdgStepIO* IO, const MdgLaunch* L,
                          const uint8_t* mask, int fill_ticks, int clear_nstep, void* workspace, int64_t workspace_bytes,
-                         const MdgParamSets* sets, const double* broker = nullptr) {
+                         const MdgParamSets* sets, const double* broker = nullptr, const MdgSetDraw* draw = nullptr) {
   int rc = check_common(P, L);
   if (rc) return rc;
   if (sets && (rc = check_sets(P, sets))) return rc;
@@ -808,7 +889,7 @@ static int reset_ws_impl(const MdgParams* P, const MdgState* S, const MdgStepIO*
   if (fill_ticks > L->window) return set_err(MDG_E_INVALID, "fill_ticks > window");
   const int64_t N = L->n_envs;
   if (N == 0) return MDG_OK;
-  ResetWsBrokerArgs a;
+  ResetWsDrawArgs a;
   rc = fill_ws_args(a, P, S, IO, L, fill_ticks, clear_nstep, workspace, workspace_bytes);
   if (rc) return rc;
   a.mask = mask;
@@ -819,8 +900,7 @@ static int reset_ws_impl(const MdgParams* P, const MdgState* S, const MdgStepIO*
   if (!sets) return launch_fill(static_cast<const ResetWsArgs&>(a), N);
   a.ps = *sets;
   a.broker = broker;
-  if (!broker) return launch_fill<true>(static_cast<const ResetWsSetsArgs&>(a), N);
-  return launch_fill<true, true>(a, N);
+  return launch_fill_sets(a, N, draw);
 }
 
 extern "C" int mdg_reset_ws(const MdgParams* P, const MdgState* S, const MdgStepIO* IO, const MdgLaunch* L,
@@ -830,13 +910,23 @@ extern "C" int mdg_reset_ws(const MdgParams* P, const MdgState* S, const MdgStep
   return reset_ws_impl(P, S, IO, L, mask, fill_ticks, clear_nstep, workspace, workspace_bytes, nullptr);
 }
 
+extern "C" int mdg_reset_ws_sets_draw(const MdgParams* P, const MdgState* S, const MdgStepIO* IO, const MdgLaunch* L,
+                                      const uint8_t* mask, int fill_ticks, int clear_nstep, void* workspace,
+                                      int64_t workspace_bytes, const MdgParamSets* sets, const double* broker,
+                                      const MdgSetDraw* draw) {
+  if (!sets) return set_err(MDG_E_INVALID, "null parameter sets");
+  if (!workspace) return set_err(MDG_E_INVALID, "mdg_reset_ws_sets needs a workspace");
+  const int rc = check_draw(draw);
+  if (rc) return rc;
+  return reset_ws_impl(P, S, IO, L, mask, fill_ticks, clear_nstep, workspace, workspace_bytes, sets, broker, draw);
+}
+
 extern "C" int mdg_reset_ws_sets_broker(const MdgParams* P, const MdgState* S, const MdgStepIO* IO,
                                         const MdgLaunch* L, const uint8_t* mask, int fill_ticks, int clear_nstep,
                                         void* workspace, int64_t workspace_bytes, const MdgParamSets* sets,
                                         const double* broker) {
-  if (!sets) return set_err(MDG_E_INVALID, "null parameter sets");
-  if (!workspace) return set_err(MDG_E_INVALID, "mdg_reset_ws_sets needs a workspace");
-  return reset_ws_impl(P, S, IO, L, mask, fill_ticks, clear_nstep, workspace, workspace_bytes, sets, broker);
+  return mdg_reset_ws_sets_draw(P, S, IO, L, mask, fill_ticks, clear_nstep, workspace, workspace_bytes, sets, broker,
+                                nullptr);
 }
 
 extern "C" int mdg_reset_ws_sets(const MdgParams* P, const MdgState* S, const MdgStepIO* IO, const MdgLaunch* L,
@@ -847,7 +937,8 @@ extern "C" int mdg_reset_ws_sets(const MdgParams* P, const MdgState* S, const Md
 
 static int step_autoreset_impl(const MdgParams* P, const MdgReward* R, const MdgState* S, const MdgStepIO* IO,
                                const MdgLaunch* L, int fill_ticks, int clear_nstep, void* workspace,
-                               int64_t workspace_bytes, const MdgParamSets* sets, const double* broker = nullptr) {
+                               int64_t workspace_bytes, const MdgParamSets* sets, const double* broker = nullptr,
+                               const MdgSetDraw* draw = nullptr) {
   int rc = check_common(P, L);
   if (rc) return rc;
   if (sets && (rc = check_sets(P, sets))) return rc;
@@ -857,7 +948,7 @@ static int step_autoreset_impl(const MdgParams* P, const MdgReward* R, const Mdg
   if (fill_ticks < 1) fill_ticks = 1;
   if (fill_ticks > L->window) return set_err(MDG_E_INVALID, "fill_ticks > window");
   if (L->n_envs == 0) return MDG_OK;
-  ResetWsBrokerArgs a;
+  ResetWsDrawArgs a;
   MdgStepIO io = *IO;  // the reset draws from Philox (no injected stream) and takes no units
   io.units = nullptr; io.normals = nullptr; io.uniforms = nullptr; io.actions = nullptr; io.weights = nullptr;
   rc = fill_ws_args(a, P, S, &io, L, fill_ticks, clear_nstep, workspace, workspace_bytes);
@@ -867,8 +958,7 @@ static int step_autoreset_impl(const MdgParams* P, const MdgReward* R, const Mdg
   if (!sets) return launch_fill(static_cast<const ResetWsArgs&>(a), L->n_envs);
   a.ps = *sets;
   a.broker = broker;
-  if (!broker) return launch_fill<true>(static_cast<const ResetWsSetsArgs&>(a), L->n_envs);
-  return launch_fill<true, true>(a, L->n_envs);
+  return launch_fill_sets(a, L->n_envs, draw);
 }
 
 extern "C" int mdg_step_autoreset(const MdgParams* P, const MdgReward* R, const MdgState* S, const MdgStepIO* IO,
@@ -877,12 +967,22 @@ extern "C" int mdg_step_autoreset(const MdgParams* P, const MdgReward* R, const 
   return step_autoreset_impl(P, R, S, IO, L, fill_ticks, clear_nstep, workspace, workspace_bytes, nullptr);
 }
 
+extern "C" int mdg_step_autoreset_sets_draw(const MdgParams* P, const MdgReward* R, const MdgState* S,
+                                            const MdgStepIO* IO, const MdgLaunch* L, int fill_ticks, int clear_nstep,
+                                            void* workspace, int64_t workspace_bytes, const MdgParamSets* sets,
+                                            const double* broker, const MdgSetDraw* draw) {
+  if (!sets) return set_err(MDG_E_INVALID, "null parameter sets");
+  const int rc = check_draw(draw);
+  if (rc) return rc;
+  return step_autoreset_impl(P, R, S, IO, L, fill_ticks, clear_nstep, workspace, workspace_bytes, sets, broker, draw);
+}
+
 extern "C" int mdg_step_autoreset_sets_broker(const MdgParams* P, const MdgReward* R, const MdgState* S,
                                               const MdgStepIO* IO, const MdgLaunch* L, int fill_ticks, int clear_nstep,
                                               void* workspace, int64_t workspace_bytes, const MdgParamSets* sets,
                                               const double* broker) {
-  if (!sets) return set_err(MDG_E_INVALID, "null parameter sets");
-  return step_autoreset_impl(P, R, S, IO, L, fill_ticks, clear_nstep, workspace, workspace_bytes, sets, broker);
+  return mdg_step_autoreset_sets_draw(P, R, S, IO, L, fill_ticks, clear_nstep, workspace, workspace_bytes, sets,
+                                      broker, nullptr);
 }
 
 extern "C" int mdg_step_autoreset_sets(const MdgParams* P, const MdgReward* R, const MdgState* S, const MdgStepIO* IO,
@@ -893,21 +993,27 @@ extern "C" int mdg_step_autoreset_sets(const MdgParams* P, const MdgReward* R, c
 }
 
 static int init_state_impl(const MdgParams* P, const MdgReward* R, const MdgState* S, const MdgLaunch* L,
-                           const MdgParamSets* sets, const double* broker = nullptr) {
+                           const MdgParamSets* sets, const double* broker = nullptr, const MdgSetDraw* draw = nullptr) {
   int rc = check_common(P, L);
   if (rc) return rc;
   if (sets && (rc = check_sets(P, sets))) return rc;
   if (!S) return set_err(MDG_E_INVALID, "null state");
   if (L->n_envs == 0) return MDG_OK;
-  InitBrokerArgs a;
+  InitDrawArgs a;
   a.P = *P;
   if (R) a.R = *R; else { memset(&a.R, 0, sizeof(a.R)); a.R.nstep = 1; }
   a.S = *S; a.L = *L;
   const unsigned grid = (unsigned)((L->n_envs + 128 - 1) / 128);
-  if (sets && broker) {
+  if (sets && draw) {
     a.ps = *sets;
     a.broker = broker;
-    init_sets_broker_kernel<<<grid, 128, 0, (cudaStream_t)L->stream>>>(a);
+    a.draw = *draw;
+    if (broker) init_sets_broker_draw_kernel<<<grid, 128, 0, (cudaStream_t)L->stream>>>(a);
+    else init_sets_draw_kernel<<<grid, 128, 0, (cudaStream_t)L->stream>>>(a);
+  } else if (sets && broker) {
+    a.ps = *sets;
+    a.broker = broker;
+    init_sets_broker_kernel<<<grid, 128, 0, (cudaStream_t)L->stream>>>(static_cast<const InitBrokerArgs&>(a));
   } else if (sets) {
     a.ps = *sets;
     init_sets_kernel<<<grid, 128, 0, (cudaStream_t)L->stream>>>(static_cast<const InitSetsArgs&>(a));
@@ -921,10 +1027,17 @@ extern "C" int mdg_init_state(const MdgParams* P, const MdgReward* R, const MdgS
   return init_state_impl(P, R, S, L, nullptr);
 }
 
+extern "C" int mdg_init_state_sets_draw(const MdgParams* P, const MdgReward* R, const MdgState* S, const MdgLaunch* L,
+                                        const MdgParamSets* sets, const double* broker, const MdgSetDraw* draw) {
+  if (!sets) return set_err(MDG_E_INVALID, "null parameter sets");
+  const int rc = check_draw(draw);
+  if (rc) return rc;
+  return init_state_impl(P, R, S, L, sets, broker, draw);
+}
+
 extern "C" int mdg_init_state_sets_broker(const MdgParams* P, const MdgReward* R, const MdgState* S,
                                           const MdgLaunch* L, const MdgParamSets* sets, const double* broker) {
-  if (!sets) return set_err(MDG_E_INVALID, "null parameter sets");
-  return init_state_impl(P, R, S, L, sets, broker);
+  return mdg_init_state_sets_draw(P, R, S, L, sets, broker, nullptr);
 }
 
 extern "C" int mdg_init_state_sets(const MdgParams* P, const MdgReward* R, const MdgState* S, const MdgLaunch* L,
@@ -973,6 +1086,7 @@ extern "C" int mdg_sizeof(int which) {
     case 12: return (int)sizeof(MdgPrioritized);
     case 13: return (int)sizeof(MdgReplayRows);
     case 14: return (int)sizeof(MdgParamSets);
+    case 15: return (int)sizeof(MdgSetDraw);
   }
   return -1;
 }

@@ -198,6 +198,26 @@ __device__ __forceinline__ int64_t env_set(const MdgParamSets& ps, int64_t e) {
 __device__ __forceinline__ double broker_value(const double* __restrict__ broker, int32_t n_sets, int64_t set, int k) {
   return __ldg(broker + (int64_t)k * n_sets + set);
 }
+// per-episode set draw (MdgSetDraw): u from Philox stream 4 of (env id, tick), then the number of cdf entries <= u,
+// an upper-bound binary search of ceil(log2 n_sets) + 1 loads (clamped: a cdf whose last entry is not 1 reads no
+// further than set n_sets - 1)
+__device__ __forceinline__ int32_t draw_set(const double* __restrict__ cdf, int32_t n_sets, uint32_t gid,
+                                            unsigned long long tick, uint32_t k0, uint32_t k1) {
+  uint64_t x0, x1;
+  philox4x32_10(gid, 4u << 16, (uint32_t)tick, (uint32_t)(tick >> 32), k0, k1, x0, x1);
+  const double u = (double)(x0 >> 11) * 0x1.0p-53;
+  int32_t lo = 0, len = n_sets;
+  while (len > 0) {
+    const int32_t half = len >> 1;
+    if (__ldg(cdf + lo + half) <= u) {
+      lo += half + 1;
+      len -= half + 1;
+    } else {
+      len = half;
+    }
+  }
+  return lo < n_sets ? lo : n_sets - 1;
+}
 
 // parameter sets (host): a table and an assignment, and only generators whose p slots are plain numbers
 static inline int check_sets(const MdgParams* P, const MdgParamSets* ps) {

@@ -15,7 +15,8 @@ def _get(cfg, key, default=None):
 def make_env(config, test=False, **batched):
     """Same keys as the reference; the batched ones (``n_envs``, ``seed``, ``device``) may be in
     ``config`` or passed as keywords, and every other keyword goes to ``Env``.  With ``broker_sets`` the config's
-    margins, costs and slippage are the base values of the broker sets, and no setter is called."""
+    margins, costs and slippage are the base values of the broker sets, and no setter is called.  ``param_set_weights``
+    (with ``param_sets`` or ``broker_sets``) turns on the per-episode set draw, as for ``Env``."""
     config = copy.deepcopy(config)
     if test and "data_source_config_test" in config.keys():
         config["data_source_config"] = config["data_source_config_test"]

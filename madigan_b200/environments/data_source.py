@@ -356,6 +356,30 @@ def make_broker_table(base, set_dicts):
     return table
 
 
+def make_set_cdf(weights, n_sets=None):
+    """Table of the per-episode set draw (``MdgSetDraw.cdf``): the float64 cumulative sums of ``weights``, left to right,
+    over their total (the last cumulative sum), with the last entry set to exactly 1.0.  A set of weight 0 repeats its
+    predecessor's entry and is never drawn.  Raises ValueError for a length other than ``n_sets`` (when given) or zero,
+    a negative, NaN or infinite weight, and a zero or non-finite total."""
+    try:
+        w = np.asarray(weights, dtype=np.float64)
+    except (TypeError, ValueError) as exc:
+        raise ValueError(f"set weights must be real numbers: {exc}") from None
+    if w.ndim != 1 or w.size == 0 or (n_sets is not None and w.size != n_sets):
+        want = "a non-empty sequence" if n_sets is None else f"{n_sets} weights"
+        raise ValueError(f"set weights: need {want}, got shape {w.shape}")
+    if not np.all(np.isfinite(w)) or np.any(w < 0):
+        raise ValueError("set weights must be finite and >= 0")
+    with np.errstate(over="ignore"):
+        cdf = np.cumsum(w)
+    total = cdf[-1]
+    if not (np.isfinite(total) and total > 0):
+        raise ValueError(f"set weights: the sum must be finite and > 0, got {total}")
+    cdf /= total
+    cdf[-1] = 1.0
+    return cdf
+
+
 def make_params(data_source_type, data_source_config=None, init_cash=1_000_000.,
                 required_margin=0., maintenance_margin=0., slippage_rel=0., slippage_abs=0.,
                 transaction_cost_rel=0., transaction_cost_abs=0.):

@@ -8,12 +8,13 @@ kernel through the C-ABI in ``include/madigan_b200.h``.  There is no CPU path.
 """
 import ctypes as C
 
+import numpy as np
 import torch
 
 from .. import _abi as A
 from .._lib import check, lib
 from ..utils.data import BrokerResponse, EnvInfo, State
-from .data_source import BROKER_SLOTS, make_broker_table, make_param_table, make_params, make_reward
+from .data_source import BROKER_SLOTS, make_broker_table, make_param_table, make_params, make_reward, make_set_cdf
 
 
 def _cfg_get(cfg, key, default=None):
@@ -100,7 +101,7 @@ def _reset_workspace(lib_, P, n_envs, fill_ticks, device, stream_ptr=None, strea
 class Env:
     def __init__(self, dataSourceType, initCash=1_000_000., config=None, *, n_envs=None, device=None,
                  window=None, seed=None, env_offset=0, reward=None, param_sets=None, param_set=None,
-                 broker_sets=None):
+                 broker_sets=None, param_set_weights=None):
         """``Env(data_source_type, init_cash, config)`` as the reference (env.cpp:843-849); the batched
         keys ``n_envs``, ``seed``, ``device``, ``window_length`` may come from ``config`` or keywords.
         ``reward``: None (env reward only) or a dict with ``reward_shaper_config``, ``nstep_return``,
@@ -117,7 +118,14 @@ class Env:
         same keys in ``config`` (0 when absent).  With ``param_sets`` its length must be S; without, the generator
         table is S copies of the base config.  One index per env selects both tables: env e then equals, bit for bit,
         env e of a plain Env of its set's config with ``setRequiredMargin / setMaintenanceMargin / setSlippage /
-        setTransactionCost`` and ``initCash`` at its broker set's values (see ``make_broker_table``)."""
+        setTransactionCost`` and ``initCash`` at its broker set's values (see ``make_broker_table``).
+        ``param_set_weights``: S weights (finite, >= 0, positive sum) of a per-episode set draw, so that every episode
+        runs in a market drawn anew (training that is robust to the market); needs ``param_sets`` or ``broker_sets``.
+        Every reset of an env -- the fused auto-reset of ``step`` / ``step_actions`` / ``step_weights``, the separate
+        one after a tearsheet or injected noise, and ``reset(mask)`` -- then draws the env's set with probability
+        ``w[s] / sum(w)`` on the device, from Philox keyed on seed, global env id and the env's timestamp (see
+        ``data_source.make_set_cdf``, ``set_param_set_weights``, ``episode_param_set``).  The first episode's set is
+        ``param_set`` when given, else the draw at tick 0."""
         self._lib = lib()
         if not torch.cuda.is_available():
             raise RuntimeError("madigan_b200.Env needs a CUDA device (sm_100a); there is no CPU fallback")
@@ -162,8 +170,13 @@ class Env:
             elif (param_sets if isinstance(param_sets, int) else len(param_sets)) != S:
                 raise ValueError(f"broker_sets has {S} sets, param_sets has "
                                  f"{param_sets if isinstance(param_sets, int) else len(param_sets)}")
+        if param_set_weights is not None and param_sets is None:
+            raise ValueError("param_set_weights needs param_sets or broker_sets")
         if param_sets is not None:
             self._init_param_sets(dataSourceType, ds_cfg, param_sets, param_set)
+        self._cdf, self._weights, self._DRAW, self._pDRAW = None, None, None, None  # per-episode set draw
+        if param_set_weights is not None:
+            self.set_param_set_weights(param_set_weights)
         if broker_sets is not None:
             self._btab = torch.from_numpy(btab).to(self.device).contiguous()
             self._bptr = self._btab.data_ptr()
@@ -180,12 +193,13 @@ class Env:
             if self._PS is None:
                 check(self._lib.mdg_init_state(C.byref(self.P), C.byref(self.R), C.byref(self._S),
                                                C.byref(self._launch())))
-            else:
-                check(self._lib.mdg_init_state_sets_broker(C.byref(self.P), C.byref(self.R), C.byref(self._S),
-                                                           C.byref(self._launch()), self._pPS, self._bptr))
+            else:  # with weights and no param_set, the first episode's set is the draw at tick 0
+                check(self._lib.mdg_init_state_sets_draw(C.byref(self.P), C.byref(self.R), C.byref(self._S),
+                                                         C.byref(self._launch()), self._pPS, self._bptr,
+                                                         self._pDRAW if param_set is None else None))
             self.launches += 1
-            # the constructor consumes one generator tick (Env.h:160)
-            self._reset_launch(None, 1, False, None, None)
+            # the constructor consumes one generator tick (Env.h:160); it is not a reset: it draws no set
+            self._reset_launch(None, 1, False, None, None, draw=False)
         self.n_valid = 1
 
     # ------------------------------------------------------------------ allocation
@@ -254,6 +268,8 @@ class Env:
             self.assign_param_sets(param_set)
         self._PS = A.MdgParamSets(p=self._ptab.data_ptr(), set_of_env=self._pset.data_ptr(), n_sets=S)
         self._pPS = C.byref(self._PS)
+        # set of the episode that each env's last drawing reset finished (-1: none yet)
+        self._epset = torch.full((self.N,), -1, dtype=torch.int32, device=self.device)
 
     def _broker_table(self, config, broker_sets):
         """(MDG_BROKER_NPARAM, S) numpy table of ``broker_sets``; resolves the base values"""
@@ -309,13 +325,50 @@ class Env:
         """``(N,)`` int32: the parameter set of every env (read it; change it with ``assign_param_sets``)."""
         return None if self._PS is None else self._pset
 
+    @property
+    def param_set_weights(self):
+        """The normalised weights ``w / sum(w)`` of the per-episode set draw (a float64 numpy array of S), or None when
+        the draw is off."""
+        return None if self._weights is None else self._weights.copy()
+
+    @property
+    def episode_param_set(self):
+        """``(N,)`` int32 device view: for the envs that reset in the last call with the set draw on, the set of the
+        episode that just finished; the other entries are unchanged, and -1 until an env's first such reset.  With
+        ``torch.bincount`` over ``episode_param_set[done]`` it attributes finished episodes to markets.  None without
+        parameter sets."""
+        return None if self._PS is None else self._epset
+
+    def set_param_set_weights(self, weights):
+        """Turn the per-episode set draw on with ``weights`` (S numbers: finite, >= 0, positive sum; see
+        ``data_source.make_set_cdf``), change its weights, or turn it off with None (the sets then stay as they are
+        through resets).  Validates on the host, then writes the draw's table on the env's stream: the change takes
+        effect at the next reset (a curriculum over markets), and episodes in progress keep their sets."""
+        if self._PS is None:
+            raise RuntimeError("this Env was built without param_sets / broker_sets")
+        if weights is None:
+            self._cdf, self._weights, self._DRAW, self._pDRAW = None, None, None, None
+            return
+        S = int(self._PS.n_sets)
+        cdf = make_set_cdf(weights, S)
+        w = np.asarray(weights, dtype=np.float64)
+        if self._stream is not None:
+            self._stream.wait_stream(torch.cuda.current_stream(self.device))
+        with self._device_ctx(), self._copy_ctx():
+            if self._cdf is None:
+                self._cdf = torch.empty((S,), dtype=torch.float64, device=self.device)
+            self._cdf.copy_(torch.from_numpy(cdf))
+        self._weights = w / w.sum()
+        self._DRAW = A.MdgSetDraw(cdf=self._cdf.data_ptr(), episode_set=self._epset.data_ptr())
+        self._pDRAW = C.byref(self._DRAW)
+
     def assign_param_sets(self, ids, mask=None):
         """Set the parameter set of every env (``mask=None``) or of the envs where ``mask`` (N,) is true to ``ids``
         (an (N,) integer tensor/array, or one int).  Checks the range with one host synchronisation (a setup call, not
         one for the hot loop), then writes on the env's stream.  The change takes effect at the next launch: an episode
-        in progress continues under the new values.  For a new market per episode, step without ``auto_reset``, then
-        ``assign_param_sets(new_ids, mask=done)`` and ``reset(mask=done, fill_history=True)``: the refill already
-        ticks the new set."""
+        in progress continues under the new values.  For a new market per episode, use ``param_set_weights`` (or
+        ``set_param_set_weights``): every reset then draws the env's set on the device, inside the fused auto-reset.
+        This method stays a manual override; with the draw on, the next reset of an env replaces what it wrote."""
         if self._PS is None and not hasattr(self, "_pset"):
             raise RuntimeError("this Env was built without param_sets")
         S = self._ptab.shape[2]
@@ -421,7 +474,7 @@ class Env:
             self._set_broker(transaction_cost_rel=float(transactionPct), transaction_cost_abs=float(transactionAbs))
 
     # ------------------------------------------------------------------ reset / step
-    def _reset_launch(self, mask, fill_ticks, clear_nstep, normals, uniforms):
+    def _reset_launch(self, mask, fill_ticks, clear_nstep, normals, uniforms, draw=True):
         io = self._IO
         if normals is None and uniforms is None:
             io.normals = io.uniforms = None
@@ -445,10 +498,10 @@ class Env:
                                          None if m is None else m.data_ptr(), int(fill_ticks), int(clear_nstep),
                                          ws.data_ptr(), ws.numel()))
         else:
-            check(self._lib.mdg_reset_ws_sets_broker(C.byref(self.P), C.byref(self._S), C.byref(io),
-                                                     C.byref(self._launch()), None if m is None else m.data_ptr(),
-                                                     int(fill_ticks), int(clear_nstep), ws.data_ptr(), ws.numel(),
-                                                     self._pPS, self._bptr))
+            check(self._lib.mdg_reset_ws_sets_draw(C.byref(self.P), C.byref(self._S), C.byref(io),
+                                                   C.byref(self._launch()), None if m is None else m.data_ptr(),
+                                                   int(fill_ticks), int(clear_nstep), ws.data_ptr(), ws.numel(),
+                                                   self._pPS, self._bptr, self._pDRAW if draw else None))
         self.launches += 2  # list scan + refill kernel
         self._version += 1
         del keep
@@ -559,8 +612,9 @@ class Env:
             check(self._lib.mdg_step_autoreset(self._pP, self._pR, self._pS, self._pIO, self._pL, self.k, 1,
                                                ws.data_ptr(), ws.numel()))
         else:
-            check(self._lib.mdg_step_autoreset_sets_broker(self._pP, self._pR, self._pS, self._pIO, self._pL, self.k,
-                                                           1, ws.data_ptr(), ws.numel(), self._pPS, self._bptr))
+            check(self._lib.mdg_step_autoreset_sets_draw(self._pP, self._pR, self._pS, self._pIO, self._pL, self.k,
+                                                         1, ws.data_ptr(), ws.numel(), self._pPS, self._bptr,
+                                                         self._pDRAW))
 
     def step_actions(self, actions, *, action_atoms, unit_size, normals=None, uniforms=None, auto_reset=False):
         """``env.step(agent.action_to_transaction(actions))`` in one launch: ``actions`` is an (N, nA) integer tensor
@@ -898,12 +952,18 @@ class Env:
             sd["param_set"] = self._pset.clone()
         if self._btab is not None:
             sd["broker_table"] = self._btab.clone()  # [MDG_BROKER_NPARAM][S] storage
+        if self._PS is not None:
+            sd["episode_param_set"] = self._epset.clone()
+        if self._cdf is not None:
+            sd["set_cdf"] = self._cdf.clone()
         sd["_meta"] = dict(head=self.head, n_valid=self.n_valid, gstep=self._gstep, seed=self.seed,
                            env_offset=self.env_offset, n_envs=self.N, n_assets=self.nA, window=self.k,
                            nstep=int(self.R.nstep), ra=self.ra, shaper=int(self.R.shaper),
                            margins=(self.P.required_margin, self.P.maintenance_margin),
                            costs=(self.P.tcost_rel, self.P.tcost_abs, self.P.slippage_rel, self.P.slippage_abs),
-                           n_sets=self.n_param_sets, broker_sets=self._btab is not None)
+                           n_sets=self.n_param_sets, broker_sets=self._btab is not None,
+                           set_draw=self._cdf is not None,
+                           set_weights=None if self._weights is None else self._weights.tolist())
         return sd
 
     def load_state_dict(self, sd):
@@ -920,9 +980,18 @@ class Env:
             has = lambda b: "with" if b else "without"
             raise ValueError(f"checkpoint was taken from an Env {has(m.get('broker_sets', False))} broker sets, this one "
                              f"is {has(self._btab is not None)}")
+        if m.get("set_draw", False) != (self._cdf is not None):
+            has = lambda b: "with" if b else "without"
+            raise ValueError(f"checkpoint was taken from an Env {has(m.get('set_draw', False))} the per-episode set "
+                             f"draw, this one is {has(self._cdf is not None)}")
         if self._PS is not None:
             self._ptab.copy_(sd["param_table"])
             self._pset.copy_(sd["param_set"])
+            if "episode_param_set" in sd:
+                self._epset.copy_(sd["episode_param_set"])
+        if self._cdf is not None:
+            self._cdf.copy_(sd["set_cdf"])
+            self._weights = np.asarray(m["set_weights"], dtype=np.float64)
         if self._btab is not None:
             self._btab.copy_(sd["broker_table"])
         for k_, v in sd.items():
