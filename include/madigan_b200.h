@@ -273,8 +273,8 @@ enum MdgNorm {
 int mdg_abi_version(void);
 /* sizeof of the ABI structs as compiled: 0 MdgAssetGen 1 MdgParams 2 MdgReward 3 MdgState 4 MdgStepIO
  * 5 MdgLaunch 6 MdgDerived 7 MdgWindow 8 MdgReplay 9 MdgReplayBatch 10 MdgRewardNorm 11 MdgTearsheet
- * 12 MdgPrioritized 13 MdgReplayRows 14 MdgParamSets 15 MdgSetDraw; -1 for an unknown index (lets a binding verify
- * its struct mirror) */
+ * 12 MdgPrioritized 13 MdgReplayRows 14 MdgParamSets 15 MdgSetDraw 16 MdgEpisodeResults; -1 for an unknown index
+ * (lets a binding verify its struct mirror) */
 int mdg_sizeof(int which);
 const char *mdg_last_error(void);
 
@@ -709,6 +709,52 @@ int mdg_tearsheet_reset(const MdgTearsheet *ts, const uint8_t *mask, void *strea
 int mdg_tearsheet_update(const MdgParams *params, const MdgState *state, const MdgStepIO *io, const MdgTearsheet *ts,
                          void *stream);
 int mdg_tearsheet_summary(const MdgTearsheet *ts, double *out, void *stream);
+
+/* ---------------------------------------------------------------------------------------------------
+ * Episode results: an exact table with one row per parameter set, filled on the device over every episode a run ends.
+ * Each recording step updates the tearsheet ts exactly as mdg_tearsheet_update does; for every env whose step reported
+ * done it then takes the env's tearsheet row exactly as mdg_tearsheet_summary would produce it, divides the four
+ * money fields (1 mean_equity, 2 final_equity, 5 mean_transaction_cost, 6 total_transaction_cost) by the episode's
+ * starting cash (the init_cash slot of its broker set, else MdgParams.init_cash), adds the row into the row of the
+ * episode's set (set_of_env[e] before the refill, clamped as the kernels clamp it; 0 without sets) and re-arms the env's
+ * recorder as mdg_tearsheet_reset does.
+ *
+ * Quantisation: a field value v is admitted when it is finite and |v| < 2^31 (NaN, +-inf and larger values are not
+ * counted: n_episodes - count says how many were left out).  X = rint(v 2^64) is an exact integer (for |v| >= 2^-11 it
+ * is v 2^64 unrounded); its five base-2^30 two's-complement digits (the top one signed) are each added with an int64
+ * atomic into a limb of their own.  v*v (one fp64 multiply) goes the same way into the sum-of-squares limbs.  min and
+ * max are order-preserving int64 images of the fp64 value (b = its bits; b < 0 ? b ^ 0x7fff...f : b) under
+ * atomicMin / atomicMax.  Integer addition is associative: the table does not depend on the order in which envs
+ * finish, the grid or the number of shards, and shards reduce with a plain SUM of acc (MIN / MAX of ext).
+ * A limb grows by less than 2^30 per episode: the owner normalises the digits (back to [0, 2^30), the top digit signed)
+ * at least every floor(2^32 / n_envs) recording steps, so that no limb overflows.
+ *
+ * Layout (int64, device):
+ *   acc [n_sets][2 + 11 n_fields]: n_episodes, n_margin_call (episodes whose last step had margin_call set), then per
+ *       field f: count, sum digits 0..4 (digit k has weight 2^(30k - 64)), sum-of-squares digits 0..4;
+ *       zero when empty.
+ *   ext [2][n_sets][n_fields]: min images, then max images; INT64_MAX / INT64_MIN when empty.
+ * n_fields == MDG_TS_NFIXED + 3 ts.n_offsets + ts.n_assets (the tearsheet fields, in mdg_tearsheet_summary's order);
+ * n_sets == the call's sets->n_sets, 1 without sets. */
+typedef struct MdgEpisodeResults {
+  MdgTearsheet ts; /* the recorder */
+  int64_t *acc;    /* [n_sets][2 + 11 n_fields] */
+  int64_t *ext;    /* [2][n_sets][n_fields] */
+  int32_t n_sets, n_fields;
+} MdgEpisodeResults;
+/* mdg_step_autoreset_sets_draw with the record + harvest kernel between the step kernel and the refill (three
+ * launches).  sets, broker and draw may each be NULL: a plain Env (then broker and draw must be NULL), no broker table,
+ * no draw.  res is required; MDG_E_INVALID for a null accumulator or table, an n_assets, n_fields or n_sets that does
+ * not match, or null done / margin_call. */
+int mdg_step_autoreset_results(const MdgParams *params, const MdgReward *reward, const MdgState *state,
+                               const MdgStepIO *io, const MdgLaunch *launch, int fill_ticks, int clear_nstep,
+                               void *workspace, int64_t workspace_bytes, const MdgParamSets *sets,
+                               const double *broker, const MdgSetDraw *draw, const MdgEpisodeResults *res);
+/* the record + harvest kernel alone, for a step whose finished envs are reset separately (injected noise): call it
+ * after the step and before the reset. */
+int mdg_episode_results_record(const MdgParams *params, const MdgState *state, const MdgStepIO *io,
+                               const MdgParamSets *sets, const double *broker, const MdgEpisodeResults *res,
+                               void *stream);
 
 #ifdef __cplusplus
 }

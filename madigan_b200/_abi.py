@@ -144,6 +144,13 @@ class MdgTearsheet(C.Structure):
                                    "sum_cost", "in_pos", "eq_ring", "ret_n", "ret_mean", "ret_m2", "ret_down")]
 
 
+class MdgEpisodeResults(C.Structure):
+    _fields_ = [("ts", MdgTearsheet), ("acc", _dp), ("ext", _dp), ("n_sets", C.c_int32), ("n_fields", C.c_int32)]
+
+
+MDG_RES_DIGITS = 5  # base-2^30 digits of a quantised value (MdgEpisodeResults)
+
+
 class MdgRewardNorm(C.Structure):
     _fields_ = [("kind", C.c_int32), ("window", C.c_int32), ("n_envs", C.c_int64), ("alpha", C.c_double)] + \
                [(n, _dp) for n in ("buffer", "size", "front", "count", "mean_est", "ssq", "ewma", "ewma_old",
@@ -216,6 +223,11 @@ SYMBOLS = {
     "mdg_tearsheet_reset": (C.c_int, [_P(MdgTearsheet), C.c_void_p, C.c_void_p]),
     "mdg_tearsheet_update": (C.c_int, [_P(MdgParams), _P(MdgState), _P(MdgStepIO), _P(MdgTearsheet), C.c_void_p]),
     "mdg_tearsheet_summary": (C.c_int, [_P(MdgTearsheet), C.c_void_p, C.c_void_p]),
+    "mdg_step_autoreset_results": (C.c_int, [_P(MdgParams), _P(MdgReward), _P(MdgState), _P(MdgStepIO),
+                                             _P(MdgLaunch), C.c_int, C.c_int, C.c_void_p, C.c_int64,
+                                             _P(MdgParamSets), C.c_void_p, _P(MdgSetDraw), _P(MdgEpisodeResults)]),
+    "mdg_episode_results_record": (C.c_int, [_P(MdgParams), _P(MdgState), _P(MdgStepIO), _P(MdgParamSets),
+                                             C.c_void_p, _P(MdgEpisodeResults), C.c_void_p]),
 }
 
 
@@ -230,4 +242,4 @@ def bind(lib):
 
 STRUCTS = (MdgAssetGen, MdgParams, MdgReward, MdgState, MdgStepIO, MdgLaunch, MdgDerived, MdgWindow, MdgReplay,
            MdgReplayBatch, MdgRewardNorm, MdgTearsheet, MdgPrioritized, MdgReplayRows, MdgParamSets,
-           MdgSetDraw)  # mdg_sizeof order
+           MdgSetDraw, MdgEpisodeResults)  # mdg_sizeof order

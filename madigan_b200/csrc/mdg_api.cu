@@ -938,7 +938,7 @@ extern "C" int mdg_reset_ws_sets(const MdgParams* P, const MdgState* S, const Md
 static int step_autoreset_impl(const MdgParams* P, const MdgReward* R, const MdgState* S, const MdgStepIO* IO,
                                const MdgLaunch* L, int fill_ticks, int clear_nstep, void* workspace,
                                int64_t workspace_bytes, const MdgParamSets* sets, const double* broker = nullptr,
-                               const MdgSetDraw* draw = nullptr) {
+                               const MdgSetDraw* draw = nullptr, const MdgEpisodeResults* res = nullptr) {
   int rc = check_common(P, L);
   if (rc) return rc;
   if (sets && (rc = check_sets(P, sets))) return rc;
@@ -947,6 +947,7 @@ static int step_autoreset_impl(const MdgParams* P, const MdgReward* R, const Mdg
   if (!S->reset_ts || !IO->pre_price) return set_err(MDG_E_INVALID, "state.reset_ts / io.pre_price is null");
   if (fill_ticks < 1) fill_ticks = 1;
   if (fill_ticks > L->window) return set_err(MDG_E_INVALID, "fill_ticks > window");
+  if (res && res->ts.n_envs != L->n_envs) return set_err(MDG_E_INVALID, "episode results: n_envs mismatch");
   if (L->n_envs == 0) return MDG_OK;
   ResetWsDrawArgs a;
   MdgStepIO io = *IO;  // the reset draws from Philox (no injected stream) and takes no units
@@ -955,6 +956,8 @@ static int step_autoreset_impl(const MdgParams* P, const MdgReward* R, const Mdg
   if (rc) return rc;
   rc = step_impl(P, R, S, IO, L, a.count, a.list, sets, broker);  // the step kernel appends the finished envs to the list
   if (rc) return rc;
+  // the finished episodes' rows, under the sets the refill is about to replace
+  if (res && (rc = launch_results_record(P, S, IO, sets, broker, res, L->stream))) return rc;
   if (!sets) return launch_fill(static_cast<const ResetWsArgs&>(a), L->n_envs);
   a.ps = *sets;
   a.broker = broker;
@@ -975,6 +978,19 @@ extern "C" int mdg_step_autoreset_sets_draw(const MdgParams* P, const MdgReward*
   const int rc = check_draw(draw);
   if (rc) return rc;
   return step_autoreset_impl(P, R, S, IO, L, fill_ticks, clear_nstep, workspace, workspace_bytes, sets, broker, draw);
+}
+
+extern "C" int mdg_step_autoreset_results(const MdgParams* P, const MdgReward* R, const MdgState* S,
+                                          const MdgStepIO* IO, const MdgLaunch* L, int fill_ticks, int clear_nstep,
+                                          void* workspace, int64_t workspace_bytes, const MdgParamSets* sets,
+                                          const double* broker, const MdgSetDraw* draw,
+                                          const MdgEpisodeResults* res) {
+  if (!sets && (broker || draw)) return set_err(MDG_E_INVALID, "a broker table or a set draw needs parameter sets");
+  int rc = check_draw(draw);
+  if (rc) return rc;
+  if ((rc = check_results(P, S, IO, sets, res))) return rc;
+  return step_autoreset_impl(P, R, S, IO, L, fill_ticks, clear_nstep, workspace, workspace_bytes, sets, broker, draw,
+                             res);
 }
 
 extern "C" int mdg_step_autoreset_sets_broker(const MdgParams* P, const MdgReward* R, const MdgState* S,
@@ -1087,6 +1103,7 @@ extern "C" int mdg_sizeof(int which) {
     case 13: return (int)sizeof(MdgReplayRows);
     case 14: return (int)sizeof(MdgParamSets);
     case 15: return (int)sizeof(MdgSetDraw);
+    case 16: return (int)sizeof(MdgEpisodeResults);
   }
   return -1;
 }

@@ -230,6 +230,13 @@ static inline int check_sets(const MdgParams* P, const MdgParamSets* ps) {
   return MDG_OK;
 }
 
+// episode results (mdg_tearsheet.cu): the argument checks and the record + harvest launch, which the fused
+// step + auto-reset (mdg_api.cu) issues between its step kernel and its refill
+int check_results(const MdgParams* P, const MdgState* S, const MdgStepIO* IO, const MdgParamSets* sets,
+                  const MdgEpisodeResults* res);
+int launch_results_record(const MdgParams* P, const MdgState* S, const MdgStepIO* IO, const MdgParamSets* sets,
+                          const double* broker, const MdgEpisodeResults* res, void* stream);
+
 // One getData() of asset i (DataSource.cpp).  `price` is the asset's current price
 // (== generator value for every synthetic source), gs points at gstate row gslot for
 // this env (stride N), pair_mean carries OUPair's shared mean from role 0 to role 1.

@@ -526,12 +526,15 @@ class Env:
             self.n_valid = fill
         return self._state()
 
-    def step(self, *args, normals=None, uniforms=None, auto_reset=False, tearsheet=None):
+    def step(self, *args, normals=None, uniforms=None, auto_reset=False, tearsheet=None, results=None):
         """``step()`` hold (Env.h:189-204); ``step(units)`` with units (N,nA) (Env.h:206-230);
         ``step(assetIdx|assetCode, units)`` with units (N,) (Env.h:232-256, env.cpp:995-1005).
         Returns ``(State, reward (N,), done (N,) bool, EnvInfo)``; the tensors are views of live
         buffers that the next call overwrites (same aliasing as the reference's Eigen maps).
-        ``tearsheet``: a ``utils.metrics.EpisodeTearsheet`` that records the step before any auto-reset."""
+        ``tearsheet``: a ``utils.metrics.EpisodeTearsheet`` that records the step before any auto-reset.
+        ``results``: a ``utils.metrics.EpisodeResults`` of this Env (needs ``auto_reset=True``, excludes ``tearsheet``)
+        that records the step and harvests every finished episode into its per-set table before the refill."""
+        self._check_results(results, auto_reset, tearsheet)
         asset_idx = 0
         if len(args) == 0:
             mode, units = A.MODE_HOLD, None
@@ -575,12 +578,13 @@ class Env:
             self.head = head0  # the ring head moves only once the launch has been accepted
             if auto_reset and keep is None and tearsheet is None:  # step + masked reset + history fill in one trip through the binding
                 ws = _reset_workspace(self._lib, self.P, self.N, self.k, self.device, self._stream_ptr, self._stream)
-                if self._PS is None:
+                if self._PS is None and results is None:
                     check(self._lib.mdg_step_autoreset(self._pP, self._pR, self._pS, self._pIO, self._pL, self.k, 1,
                                                        ws.data_ptr(), ws.numel()))
                 else:
-                    self._step_autoreset_call(ws)
-                self.launches += 2  # step kernel (appends the finished envs to the list) + refill kernel
+                    self._step_autoreset_call(ws, results)
+                # step kernel (appends the finished envs to the list) [+ results record] + refill kernel
+                self.launches += 2 if results is None else 3
                 auto_reset = False
             else:
                 if self._PS is None:
@@ -596,9 +600,30 @@ class Env:
             if tearsheet is not None:
                 tearsheet.update()
             if auto_reset:
+                self._record_results(results)
                 self._reset_launch(self.t["done"], self.k, True, None, None)
         t = self.t
         return self._state(), t["reward"], t["done"], self._info
+
+    def _check_results(self, results, auto_reset, tearsheet=None):
+        if results is None:
+            return
+        if getattr(results, "env", None) is not self:
+            raise ValueError("results were built on another Env")
+        if not auto_reset:
+            raise ValueError("results= needs auto_reset=True: an episode's row is harvested as the env resets")
+        if tearsheet is not None:
+            raise ValueError("results= and tearsheet= cannot be combined: the results own their recorder")
+
+    def _record_results(self, results):
+        """the record + harvest kernel alone, between a step and a separate reset of the finished envs"""
+        if results is None:
+            return
+        check(self._lib.mdg_episode_results_record(self._pP, self._pS, self._pIO,
+                                                   self._pPS if self._PS is not None else None, self._bptr,
+                                                   results._pR, self._sptr()))
+        results._recorded()
+        self.launches += 1
 
     def _step_call(self):
         if self._PS is None:
@@ -607,8 +632,14 @@ class Env:
             check(self._lib.mdg_step_sets_broker(self._pP, self._pR, self._pS, self._pIO, self._pL, self._pPS,
                                                  self._bptr))
 
-    def _step_autoreset_call(self, ws):
-        if self._PS is None:
+    def _step_autoreset_call(self, ws, results=None):
+        if results is not None:  # step, record + harvest, refill
+            check(self._lib.mdg_step_autoreset_results(self._pP, self._pR, self._pS, self._pIO, self._pL, self.k, 1,
+                                                       ws.data_ptr(), ws.numel(),
+                                                       self._pPS if self._PS is not None else None, self._bptr,
+                                                       self._pDRAW, results._pR))
+            results._recorded()
+        elif self._PS is None:
             check(self._lib.mdg_step_autoreset(self._pP, self._pR, self._pS, self._pIO, self._pL, self.k, 1,
                                                ws.data_ptr(), ws.numel()))
         else:
@@ -616,12 +647,13 @@ class Env:
                                                          1, ws.data_ptr(), ws.numel(), self._pPS, self._bptr,
                                                          self._pDRAW))
 
-    def step_actions(self, actions, *, action_atoms, unit_size, normals=None, uniforms=None, auto_reset=False):
+    def step_actions(self, actions, *, action_atoms, unit_size, normals=None, uniforms=None, auto_reset=False, results=None):
         """``env.step(agent.action_to_transaction(actions))`` in one launch: ``actions`` is an (N, nA) integer tensor
         of discrete actions in [0, action_atoms); the kernel converts them to transaction units exactly as
         ``DQN.action_to_transaction`` does (modelling/algorithm/dqn.py:160-179 -- ``(a - atoms//2) * unit_size *
         availableMargin / price``, action 0 closes an open position) and steps.  The action matrix is 1 byte per
-        asset instead of the 8 of a units matrix.  Returns what ``step(units)`` returns."""
+        asset instead of the 8 of a units matrix.  ``results``: as in ``step``.  Returns what ``step(units)`` returns."""
+        self._check_results(results, auto_reset)
         io = self._IO
         with self._device_ctx():
             a = actions if isinstance(actions, torch.Tensor) else torch.as_tensor(actions)
@@ -653,8 +685,8 @@ class Env:
                 L.action_atoms, L.unit_size = int(action_atoms), float(unit_size)
                 if auto_reset and keep is None:
                     ws = _reset_workspace(self._lib, self.P, self.N, self.k, self.device, self._stream_ptr, self._stream)
-                    self._step_autoreset_call(ws)
-                    self.launches += 1  # + the refill kernel
+                    self._step_autoreset_call(ws, results)
+                    self.launches += 1 if results is None else 2  # + [the results record and] the refill kernel
                     auto_reset = False
                 else:
                     self._step_call()
@@ -667,16 +699,18 @@ class Env:
                 self._gstep += 1
             self._version += 1
             if auto_reset:
+                self._record_results(results)
                 self._reset_launch(self.t["done"], self.k, True, None, None)
         t = self.t
         return self._state(), t["reward"], t["done"], self._info
 
-    def step_weights(self, weights, *, normals=None, uniforms=None, auto_reset=False):
+    def step_weights(self, weights, *, normals=None, uniforms=None, auto_reset=False, results=None):
         """``env.step(agent.action_to_transaction(weights))`` in one launch for a DDPG-style actor: ``weights`` is an
         (N, nA+1) real tensor of target portfolio weights, cash first; the kernel converts them to transaction units
         exactly as ``DDPG.action_to_transaction`` does (modelling/algorithm/ddpg.py:182-207 -- ``desired = w / w.sum()``
         in fp32, ``units = (desired - ledgerNormedFull)[1:] * equity / currentPrices``) and steps.  4 bytes per weight
-        cross to the device instead of 8 per unit.  Returns what ``step(units)`` returns."""
+        cross to the device instead of 8 per unit.  ``results``: as in ``step``.  Returns what ``step(units)`` returns."""
+        self._check_results(results, auto_reset)
         io = self._IO
         with self._device_ctx():
             w = weights if isinstance(weights, torch.Tensor) else torch.as_tensor(weights)
@@ -708,8 +742,8 @@ class Env:
                 self.head = head0
                 if auto_reset and keep is None:
                     ws = _reset_workspace(self._lib, self.P, self.N, self.k, self.device, self._stream_ptr, self._stream)
-                    self._step_autoreset_call(ws)
-                    self.launches += 1  # + the refill kernel
+                    self._step_autoreset_call(ws, results)
+                    self.launches += 1 if results is None else 2  # + [the results record and] the refill kernel
                     auto_reset = False
                 else:
                     self._step_call()
@@ -722,6 +756,7 @@ class Env:
                 self._gstep += 1
             self._version += 1
             if auto_reset:
+                self._record_results(results)
                 self._reset_launch(self.t["done"], self.k, True, None, None)
         t = self.t
         return self._state(), t["reward"], t["done"], self._info

@@ -1,7 +1,7 @@
 """Multi-GPU plumbing: one process per GPU, envs sharded as contiguous slabs, no step-path collective.
 
 Every env is independent (reference: Env::step touches only its own Broker/DataSource, Env.h:206-230),
-so the only data that crosses GPUs is the small episode-statistics vector, all-reduced with
+so the only data that crosses GPUs is the small episode-statistics vector (or an episode-results table), all-reduced with
 ``torch.distributed`` (NCCL over NVLink on GPUs; gloo in the CPU tests).
 """
 import os
@@ -48,6 +48,25 @@ def reduce_episode_stats(vec, n_assets):
         dist.all_reduce(mx, op=dist.ReduceOp.MAX)
         vec[3:4], vec[4:5] = mn, mx
     return vec
+
+
+def reduce_episode_results(results_or_tables):
+    """All-reduce an episode-results limb table over the ranks: a ``utils.metrics.EpisodeResults`` or its
+    ``limbs()`` dict (``acc``, ``ext``).  Carry pass, SUM of ``acc``, MIN / MAX of the min / max images, carry pass:
+    integer sums, so the table is identical on every rank and equals, digit for digit, the table one slab would have
+    filled.  Returns a new ``limbs`` dict (decode it with ``EpisodeResults.table(limbs)``).  Works on CUDA (NCCL) and
+    CPU (gloo) tensors."""
+    from .utils.metrics import carry_
+    t = results_or_tables.limbs() if hasattr(results_or_tables, "limbs") else results_or_tables
+    acc, ext = carry_(t["acc"].clone()), t["ext"].clone()
+    if dist.is_initialized() and dist.get_world_size() > 1:
+        mn, mx = ext[0].contiguous(), ext[1].contiguous()
+        dist.all_reduce(acc, op=dist.ReduceOp.SUM)
+        dist.all_reduce(mn, op=dist.ReduceOp.MIN)
+        dist.all_reduce(mx, op=dist.ReduceOp.MAX)
+        ext = torch.stack([mn, mx])
+        carry_(acc)
+    return dict(acc=acc, ext=ext)
 
 
 def summarize_stats(vec, n_assets):
